@@ -11,7 +11,12 @@ replayed from a CUDA graph.  The body of Llama-3-8B (3.4 GB) is 27x the 126 MB L
 streams its weights from HBM (L2 defeated by input size).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl gbxq|reference]
-                    [--model llama-3-8b] [--strategy bpw-4.0] [--batch 1]
+                    [--model llama-3-8b] [--strategy bpw-4.0] [--batch 1] [--dump-outputs DIR]
+
+Every timed loop runs exactly K steps.  --dump-outputs DIR writes what the last timed step computed, one
+`DIR/layer<i>_<proj>.npy` (float32, [rows, N]) per QuantizedLinear forward; inputs are seeded, so two builds run with the
+same arguments can be compared output for output.  When all rows would exceed 64 MB, a fixed seeded sample of the rows
+(the same for every layer) is written.
 
 N > 1 (launched by torch.distributed.run): tensor-parallel shards of the same model (strong scaling):
 column-parallel q/k/v/gate/up, row-parallel o/down followed by a sum all-reduce (SURVEY.md 8e).
@@ -34,6 +39,20 @@ sys.path.insert(0, ROOT)
 
 METRIC = "qmatmul_hbm_gbs_m1"
 UNIT = "GB/s"
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_rows(m_rows: int, row_elems: int, budget_bytes: int = DUMP_BUDGET_BYTES):
+    """Rows of the outputs --dump-outputs writes: None (all rows) when the whole step fits the budget as float32, else a
+    sorted seeded sample of rows, the same for every layer."""
+    import numpy as np
+
+    keep = budget_bytes // (4 * row_elems)
+    if keep < 1:
+        raise SystemExit(f"--dump-outputs: one row of every output ({4 * row_elems} bytes) exceeds {budget_bytes} bytes")
+    if keep >= m_rows:
+        return None
+    return np.sort(np.random.default_rng(0).choice(m_rows, keep, replace=False))
 
 
 def load_tensor_peak():
@@ -224,7 +243,7 @@ def run_gbxq(args):
     if world == 1:
         mode = "single"
 
-    def measure(tp: int, m_rows=None):
+    def measure(tp: int, m_rows=None, dump=False):
         Mr = M if m_rows is None else m_rows  # rows of x of this measurement
         plan = shard_plan(full_plan, tp) if tp > 1 else full_plan
 
@@ -268,36 +287,38 @@ def run_gbxq(args):
         # --stream 1: the calls of a step as a chain executed by ONE persistent launch (gbxq_qmm_stream), every call
         # ordered after the one before it (dep = previous: exactly the semantics of the launch-per-call step below).
         # Under TP the chain is cut at each all-reduce (after o_proj / down_proj).
-        chains = []
+        chains, stream_ys = [], []
         if args.stream:
             cur = ops.StreamChain(Mr)
             for p, ms in calls:
                 ys = cur.add(xbuf[ms[0].input_dims], ms)
+                stream_ys += ys
                 if tp > 1 and p in ("o_proj", "down_proj"):
                     chains.append((cur.finalize(), ys[0]))
                     cur = ops.StreamChain(Mr)
             if len(cur):
                 chains.append((cur.finalize(), None))
-            stream_y = ys[0]
 
+        # a step's result: the output of every forward, in plan order (all kept alive, so that --dump-outputs can read
+        # every one of them after the last timed step)
         def step():
             if args.stream:
                 for ch, ar in chains:
                     ch.run()
                     if ar is not None:
                         tpctx.all_reduce(ar)
-                outs[0] = stream_y
+                outs[0] = stream_ys
                 return
-            y = None
+            ys = []
             for p, ms in calls:
                 if len(ms) == 1:
                     if tp > 1 and p in ("o_proj", "down_proj"):
-                        y = tpctx.row_parallel(ms[0], xbuf[ms[0].input_dims])
+                        ys.append(tpctx.row_parallel(ms[0], xbuf[ms[0].input_dims]))
                     else:
-                        y = ms[0](xbuf[ms[0].input_dims])
+                        ys.append(ms[0](xbuf[ms[0].input_dims]))
                 else:
-                    y = ops.quantized_matmul_grouped(xbuf[ms[0].input_dims], ms)[0]
-            outs[0] = y
+                    ys += ops.quantized_matmul_grouped(xbuf[ms[0].input_dims], ms)
+            outs[0] = ys
 
         # ---- warm-up eagerly (also sets kernel attributes), then capture one step into a CUDA graph
         s = torch.cuda.Stream()
@@ -312,7 +333,8 @@ def run_gbxq(args):
         with torch.cuda.graph(graph):
             step()
         launches_per_step = ops.launch_count() - n0
-        y_last = outs[0]
+        assert len(outs[0]) == len(plan)
+        y_last = outs[0][-1]
 
         def barrier():
             if world > 1:
@@ -345,6 +367,14 @@ def run_gbxq(args):
         if args.stream and any(ch.timed_out() for ch, _ in chains):
             raise SystemExit("gbxq_qmm_stream: a CTA gave up waiting (grid not co-resident); the measurement is void")
 
+        # the outputs of the last timed step, copied to the host before the e2e steps below overwrite x_hidden
+        dumped = None
+        if dump:
+            rows = dump_rows(Mr, sum(y.shape[-1] for y in outs[0]))
+            sel = None if rows is None else torch.from_numpy(rows).to(dev)
+            dumped = {f"layer{i:02d}_{p}": (y if sel is None else y.index_select(0, sel)).float().cpu().numpy()
+                      for (i, p, *_), y in zip(plan, outs[0])}
+
         # ---- e2e: the same step through the public API with HOST buffers (pinned), copies inside the timed region
         def e2e_step():
             x_hidden.copy_(h_in, non_blocking=True)
@@ -371,9 +401,10 @@ def run_gbxq(args):
 
         return {"ms_step": ms_step, "e2e_ms": e2e_ms, "e2e_wall": e2e_wall, "launches_per_step": launches_per_step,
                 "calls": len(calls), "plan": plan, "layers": layers, "clocks": clocks, "chains": chains,
-                "h2d": int(h_in.numel() * 2), "d2h": int(h_out.numel() * 2)}
+                "h2d": int(h_in.numel() * 2), "d2h": int(h_out.numel() * 2), "outputs": dumped}
 
-    r = measure(world if mode == "tp" else 1)
+    r = measure(world if mode == "tp" else 1, dump=args.dump_outputs is not None and rank == 0)
+    dumped = r["outputs"]
     ms_step, e2e_ms, e2e_wall, launches_per_step, plan, layers, clocks, chains = (
         r["ms_step"], r["e2e_ms"], r["e2e_wall"], r["launches_per_step"], r["plan"], r["layers"], r["clocks"], r["chains"])
     ncalls, r_h2d, r_d2h = r["calls"], r["h2d"], r["d2h"]
@@ -392,13 +423,12 @@ def run_gbxq(args):
         del r2
 
     # N = 1, default decode run: the other two regimes of the same model, measured the same way in the same process
-    # (CUDA graph, CUDA events, inputs resident), so that one driver-run line carries them: a decode batch of 16 rows
-    # (HBM roofline) and a prefill chunk of 2048 tokens (tensor roofline, TFLOP/s against the sustained bf16 peak).
+    # (CUDA graph, CUDA events, inputs resident, --steps timed steps), so that one result line carries them: a decode
+    # batch of 16 rows (HBM roofline) and a prefill chunk of 2048 tokens (tensor roofline, TFLOP/s against the sustained
+    # bf16 peak).
     if world == 1 and not prefill and not args.stream and args.batch == 1 and not args.no_also:
         del r
         also = {}
-        saved_steps = args.steps
-        args.steps = max(3, min(args.steps, 5))
         rb = measure(1, 16)
         bb = sum(W.qmm_bytes(16, n, k, b, g) for (_, _, n, k, b, g) in full_plan)
         also["decode_batch_16"] = {"value": round(bb / (rb["ms_step"] * 1e-3) / 1e9, 2), "unit": UNIT, "ms_per_step": round(rb["ms_step"], 5),
@@ -413,7 +443,6 @@ def run_gbxq(args):
                                 "frac_of_tensor_peak": round(fl / (rp["ms_step"] * 1e-3) / 1e12 / tpk, 4), "peak": tpk, "peak_source": tsrc,
                                 "kernel": "gbxq::gemm_ts_kernel (tcgen05.mma, weights as the TMEM operand)"}
         del rp
-        args.steps = saved_steps
 
     bytes_step = sum(W.qmm_bytes(M, n, k, b, g) for (_, _, n, k, b, g) in full_plan) * replicas
     value = bytes_step / (ms_step * 1e-3) / 1e9
@@ -500,6 +529,12 @@ def run_gbxq(args):
         line["e2e"]["unit"] = "TFLOP/s"
     if world == 1 and not args.no_cpu_baseline and not prefill:
         line["cpu_baseline"] = cpu_sample(args, layers_for_cpu=[(p, m) for (p, m) in layers[:7]], M=M, budget_s=args.cpu_seconds)
+    if dumped is not None:
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     print(json.dumps(line), flush=True)
     finish()
 
@@ -612,7 +647,14 @@ def main():
     ap.add_argument("--no-also", action="store_true", help="N > 1: skip the measurement of the other parallelism mode")
     ap.add_argument("--allreduce", default="fused", choices=["fused", "oneshot", "nccl"], help="row-parallel layers under TP: all-reduce fused into the matmul kernel, stand-alone peer-memory kernel, or NCCL")
     ap.add_argument("--pdl", type=int, default=2, help="GBXQ_OPT_PDL (0 plain launches, 1 PDL, 2 PDL + early weight streaming)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs is not None and args.impl != "gbxq":
+        ap.error("--dump-outputs applies to --impl gbxq")
+    sys.dont_write_bytecode = True  # the benchmark may run from a read-only tree and writes nothing into it
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -7,6 +7,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -38,6 +40,19 @@ def test_shard_plans_of_the_configurations():
                 else:
                     assert k == k0 and n * tp == n0
             assert sum(n * k * bits // 8 + 4 * n * (k // g) for (_, _, n, k, bits, g) in sh) * tp == full_w
+
+
+def test_dump_rows_fit_the_budget_and_are_fixed():
+    """bench.py --dump-outputs: every row while a step's outputs fit the budget as float32, else the same seeded rows."""
+    b = _bench()
+    n = 43008 * 32  # outputs of one token through the 224 forwards of a Llama-3-8B step
+    assert b.dump_rows(1, n) is None
+    rows = b.dump_rows(2048, n)
+    assert len(rows) == b.DUMP_BUDGET_BYTES // (4 * n) and len(rows) * 4 * n <= b.DUMP_BUDGET_BYTES
+    assert bool((np.diff(rows) > 0).all()) and 0 <= rows[0] and rows[-1] < 2048
+    assert np.array_equal(rows, b.dump_rows(2048, n))
+    with pytest.raises(SystemExit):
+        b.dump_rows(1, b.DUMP_BUDGET_BYTES)
 
 
 def test_fast_argmax_first_occurrence():
