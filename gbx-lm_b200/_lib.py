@@ -39,6 +39,9 @@ EXPORTS = (
     "gbxq_qmm_rowpar_allreduce",
     "gbxq_rope_cache",
     "gbxq_decode_attention",
+    "gbxq_rope_cache_quantized",
+    "gbxq_decode_attention_quantized",
+    "gbxq_decode_attention_quantized_workspace_bytes",
     "gbxq_add_rmsnorm",
     "gbxq_silu_mul",
     "gbxq_head_gemv",
@@ -151,6 +154,12 @@ def get() -> ctypes.CDLL:
     lib.gbxq_rope_cache.argtypes = [vp, vp, vp, vp, vp, vp, vp, ci, ci, ci, ci, i64, vp]
     lib.gbxq_decode_attention.restype = ci
     lib.gbxq_decode_attention.argtypes = [vp, vp, vp, vp, vp, ci, ci, ci, ci, i64, i64, cf, vp]
+    lib.gbxq_rope_cache_quantized.restype = ci
+    lib.gbxq_rope_cache_quantized.argtypes = [vp] * 11 + [ci, ci, ci, ci, i64, ci, ci, vp]
+    lib.gbxq_decode_attention_quantized_workspace_bytes.restype = sz
+    lib.gbxq_decode_attention_quantized_workspace_bytes.argtypes = [ci, ci, ci, ci, i64]
+    lib.gbxq_decode_attention_quantized.restype = ci
+    lib.gbxq_decode_attention_quantized.argtypes = [vp] * 9 + [ci, ci, ci, ci, i64, i64, cf, ci, ci, vp, sz, vp]
     lib.gbxq_add_rmsnorm.restype = ci
     lib.gbxq_add_rmsnorm.argtypes = [vp, vp, vp, cf, vp, vp, i64, ci, vp]
     lib.gbxq_silu_mul.restype = ci

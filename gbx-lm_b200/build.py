@@ -28,6 +28,7 @@ SOURCES = [
     "gbxq_mmv8_grouped.cu",
     "gbxq_stream.cu",
     "gbxq_glue.cu",
+    "gbxq_qattn.cu",
     "gbxq_head.cu",
     "gbxq_gather.cu",
     "gbxq_gemm_sm100.cu",

@@ -185,8 +185,12 @@ class KVCache(_BlockStore):
 
 def maybe_quantize_kv_cache(prompt_cache: list, quantized_kv_start: int, kv_group_size: int, kv_bits: Optional[int]) -> None:
     """gbx_lm/utils.py:204-214: once the prompt is longer than `quantized_kv_start`, every dense cache of the list is
-    replaced by its quantized form (the list is edited in place; a list that already starts quantized is left alone)."""
-    if kv_bits is None or isinstance(prompt_cache[0], QuantizedKVCache) or prompt_cache[0].offset <= quantized_kv_start:
+    replaced by its quantized form (the list is edited in place; a list that already starts quantized is left alone).
+    The same rule decides for the static caches of the decode loop (qllama.KVCache -> qllama.QuantizedKVCache)."""
+    from . import qllama
+
+    quantized, dense = (QuantizedKVCache, qllama.QuantizedKVCache), (KVCache, qllama.KVCache)
+    if kv_bits is None or isinstance(prompt_cache[0], quantized) or prompt_cache[0].offset <= quantized_kv_start:
         return
-    prompt_cache[:] = [c.to_quantized(group_size=kv_group_size, bits=kv_bits) if isinstance(c, KVCache) else c
+    prompt_cache[:] = [c.to_quantized(group_size=kv_group_size, bits=kv_bits) if isinstance(c, dense) else c
                        for c in prompt_cache]

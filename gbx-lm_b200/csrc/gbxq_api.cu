@@ -311,6 +311,29 @@ int gbxq_decode_attention(const void* q, const void* k_cache, const void* v_cach
                                    (cudaStream_t)stream);
 }
 
+int gbxq_rope_cache_quantized(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev,
+                              uint32_t* k_codes, void* k_scales, void* k_biases, uint32_t* v_codes, void* v_scales,
+                              void* v_biases, int B, int Hq, int Hkv, int D, int64_t max_len, int bits, int group_size,
+                              void* stream) {
+    const QCacheWrite a{q, k, v, pos_dev, inv_freq_dev, k_codes, k_scales, k_biases, v_codes, v_scales, v_biases,
+                        B, Hq, Hkv, D, max_len, bits, group_size};
+    return launch_rope_cache_quantized(a, (cudaStream_t)stream);
+}
+
+size_t gbxq_decode_attention_quantized_workspace_bytes(int B, int Hq, int Hkv, int D, int64_t attend_len) {
+    return qattn_workspace_bytes(B, Hq, Hkv, D, attend_len);
+}
+
+int gbxq_decode_attention_quantized(const void* q, const uint32_t* k_codes, const void* k_scales, const void* k_biases,
+                                    const uint32_t* v_codes, const void* v_scales, const void* v_biases,
+                                    const int64_t* pos_dev, void* out, int B, int Hq, int Hkv, int D, int64_t max_len,
+                                    int64_t attend_len, float scale, int bits, int group_size, void* workspace,
+                                    size_t workspace_bytes, void* stream) {
+    const QAttn a{q, k_codes, k_scales, k_biases, v_codes, v_scales, v_biases, pos_dev, out, B, Hq, Hkv, D, max_len,
+                  attend_len, scale, bits, group_size, workspace, workspace_bytes};
+    return launch_decode_attention_quantized(a, (cudaStream_t)stream);
+}
+
 int gbxq_add_rmsnorm(const void* x, const void* r, const void* w, float eps, void* h_out, void* y_out, int64_t rows, int H,
                      void* stream) {
     if (!x || !w || !y_out) return GBXQ_ENULL;

@@ -217,6 +217,39 @@ int launch_rope_cache(void* q, const void* k, const void* v, const int64_t* pos,
                       int B, int Hq, int Hkv, int D, int64_t max_len, cudaStream_t st);
 int launch_decode_attention(const void* q, const void* kc, const void* vc, const int64_t* pos, void* out, int B, int Hq,
                             int Hkv, int D, int64_t max_len, int64_t attend_len, float scale, cudaStream_t st);
+// arguments of the quantized-cache decode step (gbxq_qattn.cu): one (codes, scales, biases) triple per side, bf16
+struct QCacheWrite {
+    void* q;
+    const void* k;
+    const void* v;
+    const int64_t* pos;
+    const float* inv_freq;
+    uint32_t* kq;
+    void *ks, *kb;
+    uint32_t* vq;
+    void *vs, *vb;
+    int B, Hq, Hkv, D;
+    int64_t max_len;
+    int bits, gs;
+};
+struct QAttn {
+    const void* q;
+    const uint32_t* kq;
+    const void *ks, *kb;
+    const uint32_t* vq;
+    const void *vs, *vb;
+    const int64_t* pos;
+    void* out;
+    int B, Hq, Hkv, D;
+    int64_t max_len, attend_len;
+    float scale;
+    int bits, gs;
+    void* ws;
+    size_t ws_bytes;
+};
+int launch_rope_cache_quantized(const QCacheWrite& a, cudaStream_t st);
+int launch_decode_attention_quantized(const QAttn& a, cudaStream_t st);
+size_t qattn_workspace_bytes(int B, int Hq, int Hkv, int D, int64_t attend_len);
 int launch_add_rmsnorm(const void* x, const void* r, const void* w, float eps, void* h_out, void* y_out, int64_t rows, int H,
                        cudaStream_t st);
 int launch_silu_mul(const void* g, const void* u, void* out, int64_t n, cudaStream_t st);

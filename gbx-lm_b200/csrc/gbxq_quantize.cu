@@ -5,7 +5,7 @@
 // (cache.py:251-263) converts a whole dense cache at once.
 //
 // Arithmetic (oracle/MLX_SPEC.md R6, fp32 throughout, every operation separately rounded -- no FMA can form because
-// no multiply feeds an add):
+// no multiply feeds an add), in gbxq_affine.cuh so that the fused cache write of gbxq_qattn.cu computes the same bits:
 //     w_max, w_min over the group;  mask = |w_min| > |w_max|
 //     scale = max((w_max - w_min) / (2^bits - 1), 1e-7);  scale = mask ? scale : -scale;  edge = mask ? w_min : w_max
 //     q0 = rint(edge / scale);  if (q0 != 0) { scale = edge / q0;  bias = edge; } else bias = 0
@@ -26,6 +26,7 @@
 // min / max inside the lanes of a group with xor shuffles, stages its codes in shared memory and writes them back as
 // coalesced words.  Destination rows can be remapped (gbxq_quantize_rows): the cache update writes the rows
 // of every (batch, head) at the current offset of a [.., capacity, ..] buffer without a second copy.
+#include "gbxq_affine.cuh"
 #include "gbxq_common.cuh"
 
 namespace gbxq {
@@ -100,7 +101,6 @@ __global__ void __launch_bounds__(kWarps * 32) quantize_kernel(const T* __restri
     constexpr int SEG = GS / EPL;         // lanes per group: 2..8 / 4..16
     constexpr int BPL = EPL * BITS / 8;   // bytes of codes per lane
     constexpr int WPC = EPL * BITS;       // words of codes per chunk
-    constexpr int NB = (1 << BITS) - 1;
     __shared__ __align__(16) uint8_t stage_all[kWarps][32 * BPL];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     uint8_t* stage = stage_all[warp];
@@ -108,7 +108,6 @@ __global__ void __launch_bounds__(kWarps * 32) quantize_kernel(const T* __restri
     const int64_t wpr = K * BITS / 32;  // words per row of codes
     const int64_t gpr = K / GS;         // groups per row
     const int64_t total_words = total / 32 * BITS;
-    const float nb = (float)NB;
     const bool dense = map.inner <= 0;
     const bool small = total_words < (int64_t(1) << 31) && total < (int64_t(1) << 31);
     const int64_t stride = (int64_t)gridDim.x * kWarps;
@@ -139,36 +138,15 @@ __global__ void __launch_bounds__(kWarps * 32) quantize_kernel(const T* __restri
             mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
             mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
         }
-        const bool mask = fabsf(mn) > fabsf(mx);
-        float scale = fmaxf(__fdiv_rn(__fsub_rn(mx, mn), nb), 1e-7f);
-        scale = mask ? scale : -scale;
-        const float edge = mask ? mn : mx;
-        const float q0 = rintf(__fdiv_rn(edge, scale));
-        float bias = 0.f;
-        if (q0 != 0.f) {
-            scale = __fdiv_rn(edge, q0);
-            bias = edge;
-        }
-        // (w - bias) / scale, correctly rounded, without a division per element: with r = RN(1 / scale),
-        // q1 = RN(d * r), rem = d - q1 * scale (exact in one FMA), q = RN(q1 + rem * r) is the IEEE quotient (Markstein;
-        // |scale| >= ~5e-8 keeps r and the quotients that can reach a rounding boundary of rint() in the normal range).
-        // rint() and the float -> int conversion are one add of 1.5 * 2^23 (ulp 1, ties to even; |q| < 2^22 always:
-        // every |w - bias| <= max - min <= (2^bits) * |scale|), the clamp is an integer min / max.
-        const float r = __frcp_rn(scale);
-        const float nscale = -scale;
+        // statistics and codes: the shared recipe (gbxq_affine.cuh)
+        const AffineGroup grp = affine_group<BITS>(mx, mn);
+        const float scale = grp.scale, bias = grp.bias;
 #pragma unroll
         for (int h = 0; h < EPL / 8; h++) {
-            uint64_t pack = 0;
+            uint32_t codes[8];
 #pragma unroll
-            for (int i = 0; i < 8; i++) {
-                const float d = __fsub_rn(v[h * 8 + i], bias);
-                const float q1 = __fmul_rn(d, r);
-                const float rem = __fmaf_rn(q1, nscale, d);
-                const float qq = __fmaf_rn(rem, r, q1);
-                int code = (int)__float_as_uint(__fadd_rn(qq, 12582912.0f)) - 0x4B400000;
-                code = min(max(code, 0), NB);
-                pack |= (uint64_t)(uint32_t)code << (i * BITS);
-            }
+            for (int i = 0; i < 8; i++) codes[i] = affine_code<BITS>(v[h * 8 + i], grp);
+            const uint64_t pack = pack_octet<BITS>(codes);
             // 8 codes are BITS bytes of the chunk's LSB-first stream; the lane's codes start at byte lane * BPL
             uint8_t* dst = stage + lane * BPL + h * BITS;
             if constexpr (BITS == 8) {

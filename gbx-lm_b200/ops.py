@@ -545,6 +545,101 @@ def decode_attention(q: torch.Tensor, k_cache: torch.Tensor, v_cache: torch.Tens
     return out
 
 
+def _check_qcache(q: torch.Tensor, k_cache3, v_cache3, group_size: int, bits: int):
+    """Shapes of the quantized-cache glue: q [B,Hq,D] bf16, triples (codes uint32 [B,Hkv,max_len,D*bits/32], scales /
+    biases bf16 [B,Hkv,max_len,D/group_size]), all contiguous on one CUDA device.  Returns (B, Hq, Hkv, D, max_len)."""
+    if bits not in (2, 3, 4, 6, 8):
+        raise ValueError(f"quantized cache: bits must be one of 2, 3, 4, 6, 8; got {bits}")
+    if group_size not in (32, 64, 128):
+        raise ValueError(f"quantized cache: group_size must be 32, 64 or 128; got {group_size}")
+    if len(k_cache3) != 3 or len(v_cache3) != 3:
+        raise ValueError("quantized cache: keys and values are (codes, scales, biases) triples")
+    if q.dim() != 3 or q.dtype != torch.bfloat16:
+        raise ValueError("quantized cache: q must be bf16 [B, Hq, D]")
+    b, hq, d = q.shape
+    kq = k_cache3[0]
+    if kq.dim() != 4:
+        raise ValueError("quantized cache: codes must be [B, Hkv, max_len, D*bits/32]")
+    hkv, max_len = kq.shape[1], kq.shape[2]
+    want = ((b, hkv, max_len, d * bits // 32), (b, hkv, max_len, d // group_size), (b, hkv, max_len, d // group_size))
+    for side in (k_cache3, v_cache3):
+        if side[0].dtype not in (torch.uint32, torch.int32) or side[1].dtype != torch.bfloat16 or side[2].dtype != torch.bfloat16:
+            raise ValueError("quantized cache: codes uint32, scales / biases bf16")
+        if tuple(tuple(t.shape) for t in side) != want:
+            raise ValueError(f"quantized cache: triple shapes {[tuple(t.shape) for t in side]} do not match q {tuple(q.shape)} "
+                             f"at bits={bits}, group_size={group_size} (want {list(want)})")
+    if d % 32 or d % group_size or hkv < 1 or hq % hkv:
+        raise ValueError(f"quantized cache: D={d}, group_size={group_size}, Hq={hq}, Hkv={hkv} are inconsistent")
+    ts = [q, *k_cache3, *v_cache3]
+    if not all(t.is_cuda and t.is_contiguous() for t in ts) or len({t.device for t in ts}) != 1:
+        raise ValueError("quantized cache ops take contiguous tensors on one CUDA device (there is no CPU path)")
+    return b, hq, hkv, d, max_len
+
+
+def rope_cache_quantized(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, position: torch.Tensor, inv_freq: torch.Tensor,
+                         k_cache3, v_cache3, group_size: int, bits: int) -> torch.Tensor:
+    """gbxq_rope_cache_quantized: q [B,Hq,D] rotated IN PLACE (returned); k rotated and v copied, each quantized into row
+    `position` (int64 device tensor [1]) of its (codes, scales, biases) triple -- bit-identical to `rope_cache` into a bf16
+    row followed by `quantize_into` of that row.  The quantized counterpart of `rope_cache` (RoPE +
+    QuantizedKVCache.update_and_fetch, gbx_lm/models/cache.py:172-185)."""
+    group_size, bits = int(group_size), int(bits)
+    b, hq, hkv, d, max_len = _check_qcache(q, k_cache3, v_cache3, group_size, bits)
+    _bf16c(k, v)
+    if tuple(k.shape) != (b, hkv, d) or tuple(v.shape) != (b, hkv, d):
+        raise ValueError(f"rope_cache_quantized: k / v must be [B, Hkv, D] = {(b, hkv, d)}")
+    if (position.dtype != torch.int64 or position.device != q.device or inv_freq.dtype != torch.float32
+            or inv_freq.numel() != d // 2 or inv_freq.device != q.device):
+        raise ValueError("rope_cache_quantized: position int64 [1], inv_freq float32 [D/2], on the device of q")
+    with torch.cuda.device(q.device):
+        rc = _lib.get().gbxq_rope_cache_quantized(
+            q.data_ptr(), k.data_ptr(), v.data_ptr(), position.data_ptr(), inv_freq.data_ptr(),
+            *[t.data_ptr() for t in k_cache3], *[t.data_ptr() for t in v_cache3], b, hq, hkv, d, max_len, bits, group_size,
+            _stream())
+    _lib.check(rc, "gbxq_rope_cache_quantized")
+    return q
+
+
+# partials of gbxq_decode_attention_quantized: one buffer per device (keyed by device, not stream, so that a graph
+# captured on a side stream uses the buffer its warm-up sized; the decode loop issues these calls from one stream at a
+# time), grown on demand.  Buffers that were outgrown stay alive, because a captured CUDA graph may still point at them.
+_QATTN_WS: dict = {}
+
+
+def _qattn_workspace(device: torch.device, need: int) -> torch.Tensor:
+    bufs = _QATTN_WS.setdefault(device.index, [])
+    if not bufs or bufs[-1].numel() < need:
+        if torch.cuda.is_current_stream_capturing():
+            raise RuntimeError("decode_attention_quantized: call it once eagerly with the same attend_len before capture")
+        bufs.append(torch.zeros((max(need, 1 << 20),), dtype=torch.uint8, device=device))
+    return bufs[-1]
+
+
+def decode_attention_quantized(q: torch.Tensor, k_cache3, v_cache3, position: torch.Tensor, scale: float, group_size: int,
+                               bits: int, attend_len: Optional[int] = None) -> torch.Tensor:
+    """gbxq_decode_attention_quantized: one query row per head, q [B,Hq,D], against the quantized triples, keys
+    0..position visible (and < attend_len, default the whole cache), GQA.  Returns [B,Hq,D] bf16.  The result does not
+    depend on attend_len beyond the clamp (bitwise).  Replaces quantized_scaled_dot_product_attention at decode
+    (gbx_lm/models/base.py:65-98)."""
+    group_size, bits = int(group_size), int(bits)
+    b, hq, hkv, d, max_len = _check_qcache(q, k_cache3, v_cache3, group_size, bits)
+    attend_len = int(max_len if attend_len is None else attend_len)
+    if not 1 <= attend_len <= max_len:
+        raise ValueError(f"decode_attention_quantized: attend_len {attend_len} outside [1, {max_len}]")
+    if position.dtype != torch.int64 or position.device != q.device:
+        raise ValueError("decode_attention_quantized: position must be an int64 [1] tensor on the device of q")
+    lib = _lib.get()
+    need = int(lib.gbxq_decode_attention_quantized_workspace_bytes(b, hq, hkv, d, attend_len))
+    out = torch.empty_like(q)
+    with torch.cuda.device(q.device):
+        ws = _qattn_workspace(q.device, need)
+        rc = lib.gbxq_decode_attention_quantized(
+            q.data_ptr(), *[t.data_ptr() for t in k_cache3], *[t.data_ptr() for t in v_cache3], position.data_ptr(),
+            out.data_ptr(), b, hq, hkv, d, max_len, attend_len, float(scale), bits, group_size, ws.data_ptr(), ws.numel(),
+            _stream())
+    _lib.check(rc, "gbxq_decode_attention_quantized")
+    return out
+
+
 def add_rmsnorm(x: torch.Tensor, r: Optional[torch.Tensor], w: torch.Tensor, eps: float, want_h: bool = True):
     """gbxq_add_rmsnorm: h = x + r (r None: h = x), y = RMSNorm(h) * w over the last dimension.  Returns (h, y); h is None
     when want_h is False.  Replaces the residual add + nn.RMSNorm pair (qllama.py:137-141)."""

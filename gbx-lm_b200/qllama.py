@@ -129,6 +129,55 @@ class KVCache:
         self.keys.index_copy_(2, positions, k)
         self.values.index_copy_(2, positions, v)
 
+    # the device quantiser, overridable so that the conversion can be exercised without a GPU
+    @staticmethod
+    def _quantize(x: torch.Tensor, group_size: int, bits: int):
+        return ops.quantize(x, group_size, bits)
+
+    def to_quantized(self, group_size: int = 64, bits: int = 4) -> "QuantizedKVCache":
+        """The static quantized cache holding these positions (cache.KVCache.to_quantized, gbx_lm/models/cache.py:251-263):
+        the whole buffers are quantized, unused zero rows become zero groups, `offset` carries over."""
+        q = QuantizedKVCache.__new__(QuantizedKVCache)
+        q.keys = tuple(self._quantize(self.keys, group_size, bits))
+        q.values = tuple(self._quantize(self.values, group_size, bits))
+        q.max_len, q.offset, q.group_size, q.bits = self.max_len, self.offset, group_size, bits
+        return q
+
+
+class QuantizedKVCache:
+    """Static pre-allocated group-quantized KV cache: the counterpart of `KVCache` in the layout of
+    `cache.QuantizedKVCache` (gbx_lm/models/cache.py:133-213) -- `keys` / `values` are (codes uint32 [B, n_kv, max_len,
+    D*bits/32], scales, biases [B, n_kv, max_len, D/group_size]) triples, with `offset`, `group_size` and `bits`.
+    The decode step writes and reads it with gbxq_rope_cache_quantized / gbxq_decode_attention_quantized."""
+
+    def __init__(self, batch: int, n_kv: int, max_len: int, head_dim: int, device, group_size: int = 64, bits: int = 8,
+                 dtype=torch.bfloat16):
+        if bits not in (2, 3, 4, 6, 8) or group_size not in (32, 64, 128) or head_dim % group_size or head_dim % 32:
+            raise ValueError(f"QuantizedKVCache: bits {bits} / group_size {group_size} do not fit head_dim {head_dim}")
+
+        def side():
+            lead = (batch, n_kv, max_len)
+            return (torch.zeros((*lead, head_dim * bits // 32), dtype=torch.int32, device=device).view(torch.uint32),
+                    torch.zeros((*lead, head_dim // group_size), dtype=dtype, device=device),
+                    torch.zeros((*lead, head_dim // group_size), dtype=dtype, device=device))
+
+        self.keys, self.values = side(), side()
+        self.max_len = max_len
+        self.offset = 0
+        self.group_size, self.bits = group_size, bits
+
+    def update(self, k: torch.Tensor, v: torch.Tensor, at: int):
+        """k / v [B, n_kv, L, D] quantized into positions [at, at + L) (ops.quantize_into, one launch per side)."""
+        ops.quantize_into(k, self.keys, at, self.group_size, self.bits)
+        ops.quantize_into(v, self.values, at, self.group_size, self.bits)
+
+    def prefix(self, n: int):
+        return tuple(t[:, :, :n] for t in self.keys), tuple(t[:, :, :n] for t in self.values)
+
+
+def cache_device(c) -> torch.device:
+    return (c.keys[0] if isinstance(c, QuantizedKVCache) else c.keys).device
+
 
 def make_prompt_cache(model, batch: int = 1, max_len: int = 4096) -> List[KVCache]:
     a = model.args
@@ -157,10 +206,17 @@ class Attention(nn.Module):  # gbx_lm/models/qllama.py:39-96
         self.o_proj = QuantizedLinear(self.n_heads * head_dim, dim, bias=o_bias)
         self.rope = RoPE(head_dim, args.rope_theta, args.rope_traditional, args.rope_scaling)
 
-    def forward(self, x, positions, cache: Optional[KVCache], attend_len: Optional[int]):
+    def fused_quantized_ok(self, cache: "QuantizedKVCache") -> bool:
+        """Shapes gbxq_decode_attention_quantized serves (include/gbxq.h)."""
+        return (self.head_dim in (64, 128) and cache.group_size <= self.head_dim
+                and self.n_heads % self.n_kv_heads == 0 and self.n_heads // self.n_kv_heads <= 8)
+
+    def forward(self, x, positions, cache: Optional[Union[KVCache, "QuantizedKVCache"]], attend_len: Optional[int]):
         B, L, _ = x.shape
         # one grouped launch for the three projections of x (ref qllama.py:76 calls them back to back)
         q, k, v = ops.quantized_matmul_grouped(x, (self.q_proj, self.k_proj, self.v_proj))
+        if isinstance(cache, QuantizedKVCache):
+            return self._forward_quantized(x, q, k, v, positions, cache, attend_len)
         if fused_decode_ok(x, L, cache) and self.head_dim in (64, 128) and cache.max_len <= 49152:
             # decode step: RoPE + cache write in one launch, one-query attention in another (SURVEY.md 8f rank 2)
             qh = q.view(B, self.n_heads, self.head_dim)
@@ -184,6 +240,33 @@ class Attention(nn.Module):  # gbx_lm/models/qllama.py:39-96
         mask = torch.arange(T, device=x.device)[None, :] <= positions[:, None]
         out = F.scaled_dot_product_attention(q, keys, values, attn_mask=mask[None, None], scale=self.scale,
                                              enable_gqa=self.n_heads != self.n_kv_heads)
+        out = out.transpose(1, 2).reshape(B, L, -1)
+        return self.tp.row_parallel(self.o_proj, out)
+
+    def _forward_quantized(self, x, q, k, v, positions, cache: "QuantizedKVCache", attend_len: Optional[int]):
+        B, L, _ = x.shape
+        gs, bits = cache.group_size, cache.bits
+        if fused_decode_ok(x, L, cache) and self.fused_quantized_ok(cache):
+            # decode step: RoPE + quantized cache write in one launch, split-K attention over the codes (+ its combine)
+            qh = q.view(B, self.n_heads, self.head_dim)
+            ops.rope_cache_quantized(qh, k.view(B, self.n_kv_heads, self.head_dim), v.view(B, self.n_kv_heads, self.head_dim),
+                                     positions, self.rope.inv_freq, cache.keys, cache.values, gs, bits)
+            out = ops.decode_attention_quantized(qh, cache.keys, cache.values, positions, self.scale, gs, bits, attend_len)
+            return self.tp.row_parallel(self.o_proj, out.view(B, 1, -1))
+        # prefill chunks and the unfused path: the reference's own (QuantizedKVCache.update_and_fetch +
+        # quantized_scaled_dot_product_attention, gbx_lm/models/base.py:65-98).  The rows are written at the HOST offset
+        # (Model.forward has already advanced it past these L positions), so this path is not graph-capturable.
+        from .switch_layers import quantized_scaled_dot_product_attention
+
+        q = self.rope(q.view(B, L, self.n_heads, -1).transpose(1, 2), positions)
+        k = self.rope(k.view(B, L, self.n_kv_heads, -1).transpose(1, 2), positions)
+        v = v.view(B, L, self.n_kv_heads, -1).transpose(1, 2)
+        T = cache.offset
+        cache.update(k, v, T - L)
+        keys, values = cache.prefix(T)
+        mask = torch.zeros((L, T), dtype=q.dtype, device=x.device)
+        mask.masked_fill_(torch.arange(T, device=x.device)[None, :] > positions[:, None], float("-inf"))
+        out = quantized_scaled_dot_product_attention(q, keys, values, self.scale, mask, group_size=gs, bits=bits)
         out = out.transpose(1, 2).reshape(B, L, -1)
         return self.tp.row_parallel(self.o_proj, out)
 

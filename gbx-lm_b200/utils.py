@@ -311,8 +311,14 @@ class DecodeGraph:
     7*L QuantizedLinear launches plus the glue -- replays as one submission (SURVEY.md 7.2 item 1)."""
 
     def __init__(self, model, cache, batch: int = 1):
+        if any(isinstance(c, qllama.QuantizedKVCache) for c in cache):
+            # the unfused quantized path writes at the HOST offset, which a replay cannot advance
+            attns = [layer.self_attn for layer in model.layers]
+            if not qllama.FUSED_DECODE or not all(a.fused_quantized_ok(c) for a, c in zip(attns, cache)):
+                raise ValueError("DecodeGraph: a quantized KV cache is graph-capturable only on the fused decode path "
+                                 "(GBXQ_FUSED_DECODE on, head_dim 64 / 128, group_size <= head_dim, Hq/Hkv <= 8)")
         self.model, self.cache = model, cache
-        dev = cache[0].keys.device
+        dev = qllama.cache_device(cache[0])
         self.tok = torch.zeros((batch, 1), dtype=torch.long, device=dev)
         self.pos = torch.zeros((1,), dtype=torch.long, device=dev)
         self.logits = None
@@ -355,6 +361,28 @@ class DecodeGraph:
         return self.logits[:, -1, :]
 
 
+def _kv_quantizer(cache: list, kv_bits: Optional[int], kv_group_size: int, quantized_kv_start: int) -> Callable[[], bool]:
+    """The reference's check after every model call (gbx_lm/utils.py:204-214, 268-270): maybe_quantize_kv_cache on the
+    list; returns True when this call converted it."""
+    from .cache import maybe_quantize_kv_cache
+
+    def step() -> bool:
+        before = cache[0]
+        maybe_quantize_kv_cache(cache, quantized_kv_start, kv_group_size, kv_bits)
+        return cache[0] is not before
+
+    return step
+
+
+def _decode_graph(model, cache, tok, position: int, device_loop: int = 0) -> Optional[DecodeGraph]:
+    """A captured decode step, or None where the cache cannot be captured (a quantized cache off the fused path)."""
+    try:
+        dg = DecodeGraph(model, cache)
+    except ValueError:
+        return None
+    return dg.capture(tok, position, device_loop=device_loop)
+
+
 def generate_step(
     prompt: torch.Tensor,
     model: nn.Module,
@@ -365,14 +393,22 @@ def generate_step(
     prefill_step_size: int = 2048,
     max_kv_size: Optional[int] = None,
     use_cuda_graph: bool = True,
+    kv_bits: Optional[int] = None,
+    kv_group_size: int = 64,
+    quantized_kv_start: int = 0,
 ) -> Generator[Tuple[int, torch.Tensor], None, None]:
-    """Mirror of gbx_lm/utils.py:217-338 for the plain-KV, greedy path: batch-1 prompt of token ids,
+    """Mirror of gbx_lm/utils.py:217-338 for the greedy path: batch-1 prompt of token ids,
     prefill in `prefill_step_size` chunks, then one token per step; yields (token, logprobs).
-    The default sampler is the argmax of the log-probabilities (utils.py:285,305-306)."""
+    The default sampler is the argmax of the log-probabilities (utils.py:285,305-306).
+    kv_bits / kv_group_size / quantized_kv_start: the reference's quantized KV cache -- after every model call, prefill
+    chunks included, the caches are converted to `kv_bits`-bit group-quantized ones once their offset exceeds
+    `quantized_kv_start` (maybe_quantize_kv_cache); kv_bits=None keeps the bf16 cache.  A decode graph captured before the
+    conversion is captured again once, after it."""
     y = prompt.reshape(-1).to(next(model.parameters()).device)
     sampler = sampler or (lambda lp: torch.argmax(lp, dim=-1))
     max_len = max_kv_size or (y.numel() + max_tokens + 1)
     cache = prompt_cache if prompt_cache is not None else qllama.make_prompt_cache(model, 1, max_len)
+    quantize_cache = _kv_quantizer(cache, kv_bits, kv_group_size, quantized_kv_start)
 
     def _logprobs(logits):
         logits = logits.float()
@@ -381,11 +417,14 @@ def generate_step(
     with torch.no_grad():
         while y.numel() > prefill_step_size:
             model(y[:prefill_step_size][None], cache)
+            quantize_cache()
             y = y[prefill_step_size:]
         logits = model(y[None], cache)[:, -1, :]
+        quantize_cache()
         lp = _logprobs(logits)
         tok = sampler(lp)
-        dg = DecodeGraph(model, cache).capture(tok, cache[0].offset) if (use_cuda_graph and tok.is_cuda) else None
+        use_graph = use_cuda_graph and tok.is_cuda
+        dg = _decode_graph(model, cache, tok, cache[0].offset) if use_graph else None
         n = 0
         while True:
             if n == max_tokens:
@@ -397,35 +436,66 @@ def generate_step(
                 logits = dg.step(tok, pos)
             else:
                 logits = model(tok.reshape(1, 1), cache)[:, -1, :]
+            converted = quantize_cache()
             lp = _logprobs(logits)
             tok = sampler(lp)
+            if converted and use_graph:  # the captured step wrote the bf16 buffers: capture the quantized step
+                dg = _decode_graph(model, cache, tok, cache[0].offset)
 
 
-def generate_tokens_device(model, prompt: torch.Tensor, max_tokens: int = 128, prefill_step_size: int = 2048) -> Tuple[List[int], dict]:
+def generate_tokens_device(model, prompt: torch.Tensor, max_tokens: int = 128, prefill_step_size: int = 2048,
+                           kv_bits: Optional[int] = None, kv_group_size: int = 64,
+                           quantized_kv_start: int = 0) -> Tuple[List[int], dict]:
     """Greedy generation with the sampler inside the captured decode step (DecodeGraph device_loop): the same tokens as
     `generate_tokens` (argmax of the log-probabilities = argmax of the logits), but the host only enqueues replays and
     reads the tokens once at the end -- the per-token host round trip of utils.py:299-337 (~0.3-0.6 ms on a B200 box)
-    is gone.  Same timing definitions as generate_tokens."""
+    is gone.  Same timing definitions as generate_tokens.  kv_bits / kv_group_size / quantized_kv_start as in
+    generate_step: when the conversion falls inside the decode, the graph replays up to that step, the caches are
+    converted, and a graph of the quantized step replays the rest."""
     y = prompt.reshape(-1).to(next(model.parameters()).device)
     n_prompt = y.numel()
     cache = qllama.make_prompt_cache(model, 1, n_prompt + max_tokens + 1)
+    quantize_cache = _kv_quantizer(cache, kv_bits, kv_group_size, quantized_kv_start)
     t0 = time.perf_counter()
     with torch.no_grad():
         while y.numel() > prefill_step_size:
             model(y[:prefill_step_size][None], cache)
+            quantize_cache()
             y = y[prefill_step_size:]
         tok = torch.argmax(model(y[None], cache)[:, -1, :].float(), dim=-1)
+        quantize_cache()
     pos0 = cache[0].offset
-    dg = DecodeGraph(model, cache).capture(tok, pos0, device_loop=max(max_tokens - 1, 1))
+    steps = max(max_tokens - 1, 0)
+    # replay i decodes position pos0 + i; the reference converts after the call that takes the offset past
+    # quantized_kv_start, i.e. after replay max(0, quantized_kv_start - pos0)
+    convert_at = steps
+    if kv_bits is not None and isinstance(cache[0], qllama.KVCache):
+        convert_at = min(max(quantized_kv_start - pos0, 0), steps)
+    dg = _decode_graph(model, cache, tok, pos0, device_loop=max(min(convert_at + 1, steps), 1))
+    if dg is None:
+        raise ValueError("generate_tokens_device: the quantized cache cannot be captured (unfused decode path)")
     first = int(tok.item())
     t_first = time.perf_counter()
-    for _ in range(max_tokens - 1):
+    outs = []
+    for _ in range(min(convert_at + 1, steps)):
         dg.graph.replay()
+    outs.append(dg.out[: min(convert_at + 1, steps), 0])
+    done = min(convert_at + 1, steps)
+    if done < steps:
+        for c in cache:
+            c.offset = pos0 + done
+        quantize_cache()
+        dg = _decode_graph(model, cache, dg.tok[:, 0].clone(), pos0 + done, device_loop=steps - done)
+        if dg is None:
+            raise ValueError("generate_tokens_device: the quantized cache cannot be captured (unfused decode path)")
+        for _ in range(steps - done):
+            dg.graph.replay()
+        outs.append(dg.out[: steps - done, 0])
     torch.cuda.synchronize()
     t1 = time.perf_counter()
-    toks = [first] + [int(t) for t in dg.out[: max_tokens - 1, 0].tolist()]
+    toks = [first] + [int(t) for o in outs for t in o.tolist()]
     for c in cache:
-        c.offset = pos0 + max_tokens - 1
+        c.offset = pos0 + steps
     stats = {
         "prompt_tokens": int(n_prompt), "prompt_tps": n_prompt / max(t_first - t0, 1e-9),
         "generation_tokens": len(toks), "generation_tps": max(len(toks) - 1, 1) / max(t1 - t_first, 1e-9),
@@ -435,7 +505,8 @@ def generate_tokens_device(model, prompt: torch.Tensor, max_tokens: int = 128, p
 
 def generate_tokens(model, prompt: torch.Tensor, max_tokens: int = 128, **kw) -> Tuple[List[int], dict]:
     """Greedy generation + the reference's timing definitions (utils.py:590-607):
-    prompt_tps = prompt_len / time_to_first_token, generation_tps = n / (t_now - t_first)."""
+    prompt_tps = prompt_len / time_to_first_token, generation_tps = n / (t_now - t_first).  Keyword arguments
+    (use_cuda_graph, prefill_step_size, kv_bits, kv_group_size, quantized_kv_start, ...) go to generate_step."""
     toks = []
     t0 = time.perf_counter()
     t_first = None

@@ -260,6 +260,38 @@ int gbxq_add_rmsnorm(const void* x, const void* r, const void* w, float eps, voi
 int gbxq_silu_mul(const void* gate, const void* up, void* out, int64_t n, void* stream);
 
 /*
+ * The same two steps of a decode step over a group-quantized KV cache (the reference's kv_bits path:
+ * QuantizedKVCache.update_and_fetch, gbx_lm/models/cache.py:172-185, and quantized_scaled_dot_product_attention,
+ * gbx_lm/models/base.py:65-98).  Each side of the cache is a triple in the layout of gbxq_quantize, position-major:
+ *     codes uint32 [B, Hkv, max_len, D*bits/32],  scales / biases bf16 [B, Hkv, max_len, D/group_size]
+ * bits in {2,3,4,6,8}, group_size in {32,64,128} with group_size <= D, D in {64, 128}, Hq/Hkv <= 8; other shapes return
+ * GBXQ_EUNSUPPORTED (nothing enqueued).
+ *   gbxq_rope_cache_quantized       q rotated in place as gbxq_rope_cache does; k rotated and v copied, each quantized
+ *                                   into row *pos of its triple.  Codes, scales and biases are bit-identical to
+ *                                   gbxq_rope_cache into a bf16 row followed by gbxq_quantize_rows of that row.  Nothing
+ *                                   outside row *pos is written (nothing at all if *pos is outside [0, max_len)).
+ *   gbxq_decode_attention_quantized out[B,Hq,D] = softmax(scale * q . K[0..min(*pos, attend_len-1)]) . V over the
+ *                                   triples, fp32 inside.  Keys are split into chunks of 256 positions, one CTA per
+ *                                   (chunk, kv head, batch) for all query heads of the group, and the partial results
+ *                                   are combined by a second launch in chunk order: the result does not depend on
+ *                                   attend_len or max_len (bitwise), and there is no context limit.  `workspace` holds
+ *                                   the partials: at least gbxq_decode_attention_quantized_workspace_bytes(B, Hq, Hkv, D,
+ *                                   attend_len) bytes, 16-byte aligned, no initialisation needed; a workspace serves
+ *                                   the calls of one stream one after another.  Returns 0 from the size query for
+ *                                   unsupported arguments.
+ */
+int gbxq_rope_cache_quantized(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev,
+                              uint32_t* k_codes, void* k_scales, void* k_biases, uint32_t* v_codes, void* v_scales,
+                              void* v_biases, int B, int Hq, int Hkv, int D, int64_t max_len, int bits, int group_size,
+                              void* stream);
+size_t gbxq_decode_attention_quantized_workspace_bytes(int B, int Hq, int Hkv, int D, int64_t attend_len);
+int gbxq_decode_attention_quantized(const void* q, const uint32_t* k_codes, const void* k_scales, const void* k_biases,
+                                    const uint32_t* v_codes, const void* v_scales, const void* v_biases,
+                                    const int64_t* pos_dev, void* out, int B, int Hq, int Hkv, int D, int64_t max_len,
+                                    int64_t attend_len, float scale, int bits, int group_size, void* workspace,
+                                    size_t workspace_bytes, void* stream);
+
+/*
  * Vocabulary projection of the decode step (SURVEY.md 8f rank 1): y[M,V] = x[M,K] . weight[V,K]^T with UNQUANTIZED bf16
  * weights -- `self.lm_head(out)` / `self.model.embed_tokens.as_linear(out)` (gbx_lm/models/qllama.py:183-184,194-198).
  * A streaming GEMV for M <= 8 rows (K % 256 == 0, 16-byte aligned x / weight): fp32 accumulation, one rounding to bf16.

@@ -4,7 +4,13 @@ layer-mix checkpoint in the gba2mlx layout -> load_model (quant_strategy.json, s
 tokens at batch 1 (CUDA-graph decode step: 7 L QuantizedLinear forwards through libgbxq + torch glue + bf16 head),
 timed with the reference's own definitions (gbx_lm/utils.py:590-607).  Prints one JSON line.
 
-    python tools/decode_bench.py [--model llama-3.2-1b] [--strategy bpw-4.0] [--tokens 128] [--prompt 32]"""
+    python tools/decode_bench.py [--model llama-3.2-1b] [--strategy bpw-4.0] [--tokens 128] [--prompt 32]
+                                 [--kv-bits none,8,4] [--kv-group-size 64] [--quantized-kv-start N]
+
+--kv-bits takes a comma-separated list (none = the bf16 cache); one JSON line per entry, from one model load.  With a
+width the caches are converted to the group-quantized cache after the model call that takes them past
+--quantized-kv-start (the reference's generate_step rule); a start one below the prompt length prefills on bf16 and
+converts once before the decode."""
 import argparse
 import json
 import os
@@ -28,6 +34,9 @@ def main():
     ap.add_argument("--tokens", type=int, default=128)
     ap.add_argument("--prompt", type=int, default=32)
     ap.add_argument("--repeat", type=int, default=3)
+    ap.add_argument("--kv-bits", default="none")
+    ap.add_argument("--kv-group-size", type=int, default=64)
+    ap.add_argument("--quantized-kv-start", type=int, default=0)
     args = ap.parse_args()
     dims = W.MODELS[args.model]
     strat = None if args.strategy == "uniform" else W.STRATEGIES[args.strategy](dims.layers)
@@ -43,25 +52,41 @@ def main():
     finally:
         shutil.rmtree(d, ignore_errors=True)
     prompt = torch.randint(0, dims.vocab, (args.prompt,), generator=torch.Generator().manual_seed(1))
+    for kv in args.kv_bits.split(","):
+        kv_bits = None if kv.strip().lower() == "none" else int(kv)
+        run(args, dims, strat, model, prompt, kv_bits, t_write, t_load)
+
+
+def run(args, dims, strat, model, prompt, kv_bits, t_write, t_load):
+    from gbx_lm_b200 import qllama
+    from gbx_lm_b200.cache import maybe_quantize_kv_cache
+
+    kw = dict(kv_bits=kv_bits, kv_group_size=args.kv_group_size, quantized_kv_start=args.quantized_kv_start)
     best, toks0 = None, None
     for r in range(args.repeat):
         n0 = ops.launch_count()
-        toks, stats = utils.generate_tokens(model, prompt, max_tokens=args.tokens, use_cuda_graph=True)
+        toks, stats = utils.generate_tokens(model, prompt, max_tokens=args.tokens, use_cuda_graph=True, **kw)
         stats["gbxq_launches"] = ops.launch_count() - n0
         if toks0 is None:
             toks0 = toks
         assert toks == toks0, "greedy decode is not reproducible run to run"
         if best is None or stats["generation_tps"] > best["generation_tps"]:
             best = stats
-    d_toks, d_stats = utils.generate_tokens_device(model, prompt, max_tokens=args.tokens)
-    d_toks, d_stats = utils.generate_tokens_device(model, prompt, max_tokens=args.tokens)
+    d_toks, d_stats = utils.generate_tokens_device(model, prompt, max_tokens=args.tokens, **kw)
+    d_toks, d_stats = utils.generate_tokens_device(model, prompt, max_tokens=args.tokens, **kw)
     assert d_toks == toks0, "device-side greedy sampler diverged from the host-side one"
-    # device time of the captured decode step alone (no sampling, no host sync between steps)
-    from gbx_lm_b200 import qllama
-
+    # device time of the captured decode step alone (no sampling, no host sync between steps), on the cache the decode
+    # runs on: converted after the prompt when kv_bits is set and the prompt is past quantized_kv_start
     cache = qllama.make_prompt_cache(model, 1, args.prompt + args.tokens + 1)
     with torch.no_grad():
-        model(prompt[None].cuda(), cache)
+        y = prompt.cuda()
+        while y.numel() > 2048:
+            model(y[:2048][None], cache)
+            maybe_quantize_kv_cache(cache, args.quantized_kv_start, args.kv_group_size, kv_bits)
+            y = y[2048:]
+        model(y[None], cache)
+        maybe_quantize_kv_cache(cache, args.quantized_kv_start, args.kv_group_size, kv_bits)
+    quantized = isinstance(cache[0], qllama.QuantizedKVCache)
     dg = utils.DecodeGraph(model, cache).capture(torch.tensor([1], device="cuda"), args.prompt)
     for _ in range(5):
         dg.graph.replay()
@@ -73,18 +98,28 @@ def main():
     e1.record()
     torch.cuda.synchronize()
     graph_ms = e0.elapsed_time(e1) / 50
+    del dg, cache
     plan = W.layer_plan(dims, strat, 4, 64)
     body = sum(W.qmm_bytes(1, n, k, b, g) for (_, _, n, k, b, g) in plan)
     head = dims.vocab * dims.hidden * 2
+    hd = dims.head_dim or dims.hidden // dims.heads
+    row = hd * kv_bits // 8 + 2 * 2 * (hd // args.kv_group_size) if quantized else hd * 2
+    kv_per_token = dims.layers * dims.kv_heads * 2 * row
+    ctx = args.prompt + args.tokens // 2  # mean visible keys over the decode
     print(json.dumps({
         "tool": "decode_bench", "model": args.model, "strategy": args.strategy, "batch": 1, "prompt_tokens": args.prompt,
+        "kv_bits": kv_bits, "kv_group_size": args.kv_group_size if kv_bits else None,
+        "quantized_kv_start": args.quantized_kv_start if kv_bits else None, "decode_cache": "quantized" if quantized else "bf16",
+        "kv_bytes_per_token": kv_per_token, "kv_bytes_per_step_at_mean_context": kv_per_token * ctx,
         "generation_tokens": best["generation_tokens"], "generation_tps": round(best["generation_tps"], 1),
         "prompt_tps": round(best["prompt_tps"], 1), "ms_per_token": round(1e3 / best["generation_tps"], 4),
         "generation_tps_device_sampler": round(d_stats["generation_tps"], 1), "graph_ms_per_step": round(graph_ms, 4), "gbxq_launches_per_generate": best["gbxq_launches"],
+        "device_tokens_equal_host_tokens": True,
         "qmm_bytes_per_token": body, "head_bytes_per_token": head,
         "hbm_gbs_body_plus_head": round((body + head) * best["generation_tps"] / 1e9, 1),
         "checkpoint_write_s": round(t_write, 1), "load_s": round(t_load, 1), "data": "synthetic (random-init, seed 0)",
-        "note": "whole decode step: quantized forwards + decode glue through libgbxq (GBXQ_FUSED_DECODE=0: torch glue), bf16 head via cuBLAS; generation_tps syncs with the host every token, generation_tps_device_sampler does not",
+        "gpu": torch.cuda.get_device_name(0),
+        "note": "whole decode step: quantized forwards + decode glue through libgbxq (GBXQ_FUSED_DECODE=0: torch glue), bf16 head via cuBLAS; generation_tps syncs with the host every token, generation_tps_device_sampler does not; graph_ms_per_step is the captured step at position prompt_tokens",
     }), flush=True)
 
 
