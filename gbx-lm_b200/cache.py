@@ -1,16 +1,19 @@
-"""The two KV caches either side of the quantized-KV attention path (SURVEY.md 8f rank 4), with the interface of the
-reference's `KVCache` (gbx_lm/models/cache.py:216-266) and `QuantizedKVCache` (cache.py:133-213): attributes `keys`,
-`values`, `offset`, `step`, (`group_size`, `bits`), methods `update_and_fetch`, `state`, `meta_state`, `trim`,
-`is_trimmable`, `to_quantized`, and the same growth rule, so that a caller written against the reference
-(`maybe_quantize_kv_cache`, gbx_lm/utils.py:204-214; the attention layers) runs unchanged.
+"""Every KV cache of the package, in two families.
 
-Built differently underneath.  Both caches are one block-grown store (`_BlockStore`): tuples of position-major CUDA
-buffers `[B, H, capacity, width]` that share `offset`; the dense cache holds one buffer per side, the quantized one
-three (codes, scales, biases).  What the reference does with `mx.quantize` followed by three slice assignments per
-side (cache.py:176-180) is ONE `gbxq_quantize_rows` launch per side that writes codes and statistics at the offset
+The growable caches mirror the reference's `KVCache` (gbx_lm/models/cache.py:216-266) and `QuantizedKVCache`
+(cache.py:133-213): attributes `keys`, `values`, `offset`, `step`, (`group_size`, `bits`), methods `update_and_fetch`,
+`state`, `meta_state`, `trim`, `is_trimmable`, `to_quantized`, and the same growth rule, so that a caller written
+against the reference (`maybe_quantize_kv_cache`, gbx_lm/utils.py:204-214; the attention layers) runs unchanged.
+Built differently underneath: both are one block-grown store (`_BlockStore`), tuples of position-major CUDA buffers
+`[B, H, capacity, width]` that share `offset`; the dense cache holds one buffer per side, the quantized one three
+(codes, scales, biases).  What the reference does with `mx.quantize` followed by three slice assignments per side
+(cache.py:176-180) is ONE `gbxq_quantize_rows` launch per side that writes codes and statistics at the offset
 (`ops.quantize_into`); `to_quantized` (cache.py:251-263) is `gbxq_quantize` over the buffers.  The consumer is
-`switch_layers.quantized_scaled_dot_product_attention` (gbx_lm/models/base.py:65-98).  The decode path of `qllama.py`
-keeps its own static bf16 cache.  CUDA only, like everything in this package."""
+`switch_layers.quantized_scaled_dot_product_attention` (gbx_lm/models/base.py:65-98).
+
+The static caches, `StaticKVCache` and `StaticQuantizedKVCache`, are what `qllama.Model` reads and writes: allocated
+once for `max_len` positions, so that the decode step is CUDA-graph capturable, in the same layouts.  The conversion
+rule `maybe_quantize_kv_cache` decides for both families.  CUDA only, like everything in this package."""
 from __future__ import annotations
 
 from typing import Callable, Optional, Sequence, Tuple
@@ -34,6 +37,15 @@ def _cat_positions(a: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
     if a.dtype == torch.uint32:
         return torch.cat([a.view(torch.int32), b.view(torch.int32)], dim=-2).view(torch.uint32)
     return torch.cat([a, b], dim=-2)
+
+
+def _zero_triple(lead, n: int, head_dim: int, group_size: int, bits: int, dtype: torch.dtype, device) -> QTensor:
+    """n zeroed positions of a quantized side: codes uint32 [*lead, n, D*bits/32], scales / biases [*lead, n, D/group_size].
+    D * bits / 32 words per position: the reference's D // (32 // bits) (cache.py:150,156) is the same for 2/4/8-bit and
+    mis-sized for the straddling 3-/6-bit packings (32 // 3 = 10)."""
+    return (_zeros((*lead, n, head_dim * bits // 32), torch.uint32, device),
+            _zeros((*lead, n, head_dim // group_size), dtype, device),
+            _zeros((*lead, n, head_dim // group_size), dtype, device))
 
 
 class _BlockStore:
@@ -89,20 +101,8 @@ class QuantizedKVCache(_BlockStore):
         self.group_size = group_size
         self.bits = bits
 
-    # the device operation, overridable so that growth / trim / state can be exercised without a GPU
-    @staticmethod
-    def _quantize_into(x: torch.Tensor, out: QTensor, offset: int, group_size: int, bits: int) -> None:
-        ops.quantize_into(x, out, offset, group_size, bits)
-
     def _fresh(self, lead, dims, like: torch.Tensor):
-        def alloc(n: int):
-            # D * bits / 32 words per position: the reference's D // (32 // bits) (cache.py:150,156) is the same for
-            # 2/4/8-bit and mis-sized for the straddling 3-/6-bit packings (32 // 3 = 10)
-            return [(_zeros((*lead, n, d * self.bits // 32), torch.uint32, like.device),
-                     _zeros((*lead, n, d // self.group_size), like.dtype, like.device),
-                     _zeros((*lead, n, d // self.group_size), like.dtype, like.device)) for d in dims]
-
-        return alloc
+        return lambda n: [_zero_triple(lead, n, d, self.group_size, self.bits, like.dtype, like.device) for d in dims]
 
     def update_and_fetch(self, keys: torch.Tensor, values: torch.Tensor) -> Tuple[QTensor, QTensor]:
         new = keys.shape[-2]
@@ -113,8 +113,8 @@ class QuantizedKVCache(_BlockStore):
         self.values = tuple(t if t.is_contiguous() else t.contiguous() for t in v_side)
         at = self.offset
         self.offset = at + new
-        self._quantize_into(keys, self.keys, at, self.group_size, self.bits)
-        self._quantize_into(values, self.values, at, self.group_size, self.bits)
+        ops.quantize_into(keys, self.keys, at, self.group_size, self.bits)
+        ops.quantize_into(values, self.values, at, self.group_size, self.bits)
         return self._valid(self.keys), self._valid(self.values)
 
     @property
@@ -143,10 +143,6 @@ class KVCache(_BlockStore):
         super().__init__()
         self.keys: Optional[torch.Tensor] = None
         self.values: Optional[torch.Tensor] = None
-
-    @staticmethod
-    def _quantize(x: torch.Tensor, group_size: int, bits: int) -> QTensor:
-        return ops.quantize(x, group_size, bits)
 
     def update_and_fetch(self, keys: torch.Tensor, values: torch.Tensor):
         new = keys.shape[-2]
@@ -178,19 +174,89 @@ class KVCache(_BlockStore):
         q = QuantizedKVCache(group_size=group_size, bits=bits)
         q.offset = self.offset
         if self.keys is not None:
-            q.keys = self._quantize(self.keys, group_size, bits)
-            q.values = self._quantize(self.values, group_size, bits)
+            q.keys = ops.quantize(self.keys, group_size, bits)
+            q.values = ops.quantize(self.values, group_size, bits)
         return q
+
+
+# The most keys gbxq_decode_attention attends: its kernel holds one float of shared memory per visible key
+# (gbxq_glue.cu, launch_decode_attention).  A longer bf16 cache takes the unfused decode path.
+DECODE_ATTENTION_MAX_KEYS = 49152
+
+
+class StaticKVCache:
+    """Static pre-allocated KV cache [B, n_kv, max_len, D] (the reference grows in steps of 256,
+    models/cache.py:215-277; a static buffer keeps the decode step CUDA-graph capturable).  `offset` is the host-side
+    count of valid positions (eager mode)."""
+
+    def __init__(self, batch: int, n_kv: int, max_len: int, head_dim: int, device, dtype=torch.bfloat16):
+        self.keys = torch.zeros((batch, n_kv, max_len, head_dim), device=device, dtype=dtype)
+        self.values = torch.zeros((batch, n_kv, max_len, head_dim), device=device, dtype=dtype)
+        self.max_len = max_len
+        self.offset = 0
+
+    @property
+    def device(self) -> torch.device:
+        return self.keys.device
+
+    def fused_decode_fits(self, head_dim: int, n_heads: int, n_kv_heads: int) -> bool:
+        """Shapes gbxq_rope_cache + gbxq_decode_attention serve (include/gbxq.h)."""
+        return head_dim in (64, 128) and self.max_len <= DECODE_ATTENTION_MAX_KEYS
+
+    def update(self, k: torch.Tensor, v: torch.Tensor, positions: torch.Tensor):
+        self.keys.index_copy_(2, positions, k)
+        self.values.index_copy_(2, positions, v)
+
+    def to_quantized(self, group_size: int = 64, bits: int = 4) -> "StaticQuantizedKVCache":
+        """The static quantized cache holding these positions (as `KVCache.to_quantized`): the whole buffers are
+        quantized, unused zero rows become zero groups, `offset` carries over."""
+        q = StaticQuantizedKVCache.__new__(StaticQuantizedKVCache)
+        q.keys = tuple(ops.quantize(self.keys, group_size, bits))
+        q.values = tuple(ops.quantize(self.values, group_size, bits))
+        q.max_len, q.offset, q.group_size, q.bits = self.max_len, self.offset, group_size, bits
+        return q
+
+
+class StaticQuantizedKVCache:
+    """Static pre-allocated group-quantized KV cache: the counterpart of `StaticKVCache` in the layout of
+    `QuantizedKVCache` -- `keys` / `values` are (codes uint32 [B, n_kv, max_len, D*bits/32], scales, biases
+    [B, n_kv, max_len, D/group_size]) triples, with `offset`, `group_size` and `bits`.  The decode step writes and
+    reads it with gbxq_rope_cache_quantized / gbxq_decode_attention_quantized."""
+
+    def __init__(self, batch: int, n_kv: int, max_len: int, head_dim: int, device, group_size: int = 64, bits: int = 8,
+                 dtype=torch.bfloat16):
+        if bits not in (2, 3, 4, 6, 8) or group_size not in (32, 64, 128) or head_dim % group_size or head_dim % 32:
+            raise ValueError(f"StaticQuantizedKVCache: bits {bits} / group_size {group_size} do not fit head_dim {head_dim}")
+        self.keys, self.values = (_zero_triple((batch, n_kv), max_len, head_dim, group_size, bits, dtype, device)
+                                  for _ in range(2))
+        self.max_len = max_len
+        self.offset = 0
+        self.group_size, self.bits = group_size, bits
+
+    @property
+    def device(self) -> torch.device:
+        return self.keys[0].device
+
+    def fused_decode_fits(self, head_dim: int, n_heads: int, n_kv_heads: int) -> bool:
+        """Shapes gbxq_rope_cache_quantized + gbxq_decode_attention_quantized serve (include/gbxq.h)."""
+        return (head_dim in (64, 128) and self.group_size <= head_dim
+                and n_heads % n_kv_heads == 0 and n_heads // n_kv_heads <= 8)
+
+    def update(self, k: torch.Tensor, v: torch.Tensor, at: int):
+        """k / v [B, n_kv, L, D] quantized into positions [at, at + L) (ops.quantize_into, one launch per side)."""
+        ops.quantize_into(k, self.keys, at, self.group_size, self.bits)
+        ops.quantize_into(v, self.values, at, self.group_size, self.bits)
+
+    def prefix(self, n: int):
+        return tuple(t[:, :, :n] for t in self.keys), tuple(t[:, :, :n] for t in self.values)
 
 
 def maybe_quantize_kv_cache(prompt_cache: list, quantized_kv_start: int, kv_group_size: int, kv_bits: Optional[int]) -> None:
     """gbx_lm/utils.py:204-214: once the prompt is longer than `quantized_kv_start`, every dense cache of the list is
     replaced by its quantized form (the list is edited in place; a list that already starts quantized is left alone).
-    The same rule decides for the static caches of the decode loop (qllama.KVCache -> qllama.QuantizedKVCache)."""
-    from . import qllama
-
-    quantized, dense = (QuantizedKVCache, qllama.QuantizedKVCache), (KVCache, qllama.KVCache)
-    if kv_bits is None or isinstance(prompt_cache[0], quantized) or prompt_cache[0].offset <= quantized_kv_start:
+    The same rule decides for the growable and for the static caches."""
+    if (kv_bits is None or isinstance(prompt_cache[0], (QuantizedKVCache, StaticQuantizedKVCache))
+            or prompt_cache[0].offset <= quantized_kv_start):
         return
-    prompt_cache[:] = [c.to_quantized(group_size=kv_group_size, bits=kv_bits) if isinstance(c, dense) else c
-                       for c in prompt_cache]
+    prompt_cache[:] = [c.to_quantized(group_size=kv_group_size, bits=kv_bits) if isinstance(c, (KVCache, StaticKVCache))
+                       else c for c in prompt_cache]

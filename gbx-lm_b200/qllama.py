@@ -24,7 +24,9 @@ import torch.nn.functional as F
 from torch import nn
 
 from . import ops
+from .cache import StaticKVCache, StaticQuantizedKVCache
 from .quantized_linear import QuantizedLinear
+from .switch_layers import quantized_scaled_dot_product_attention
 from .tp import TPContext
 
 
@@ -115,76 +117,12 @@ class RoPE(nn.Module):
         return out.to(x.dtype)
 
 
-class KVCache:
-    """Static pre-allocated KV cache [B, n_kv, max_len, D] (the reference grows in steps of 256,
-    models/cache.py:215-277; a static buffer keeps the decode step CUDA-graph capturable)."""
-
-    def __init__(self, batch: int, n_kv: int, max_len: int, head_dim: int, device, dtype=torch.bfloat16):
-        self.keys = torch.zeros((batch, n_kv, max_len, head_dim), device=device, dtype=dtype)
-        self.values = torch.zeros((batch, n_kv, max_len, head_dim), device=device, dtype=dtype)
-        self.max_len = max_len
-        self.offset = 0  # host-side count of valid positions (eager mode)
-
-    def update(self, k: torch.Tensor, v: torch.Tensor, positions: torch.Tensor):
-        self.keys.index_copy_(2, positions, k)
-        self.values.index_copy_(2, positions, v)
-
-    # the device quantiser, overridable so that the conversion can be exercised without a GPU
-    @staticmethod
-    def _quantize(x: torch.Tensor, group_size: int, bits: int):
-        return ops.quantize(x, group_size, bits)
-
-    def to_quantized(self, group_size: int = 64, bits: int = 4) -> "QuantizedKVCache":
-        """The static quantized cache holding these positions (cache.KVCache.to_quantized, gbx_lm/models/cache.py:251-263):
-        the whole buffers are quantized, unused zero rows become zero groups, `offset` carries over."""
-        q = QuantizedKVCache.__new__(QuantizedKVCache)
-        q.keys = tuple(self._quantize(self.keys, group_size, bits))
-        q.values = tuple(self._quantize(self.values, group_size, bits))
-        q.max_len, q.offset, q.group_size, q.bits = self.max_len, self.offset, group_size, bits
-        return q
-
-
-class QuantizedKVCache:
-    """Static pre-allocated group-quantized KV cache: the counterpart of `KVCache` in the layout of
-    `cache.QuantizedKVCache` (gbx_lm/models/cache.py:133-213) -- `keys` / `values` are (codes uint32 [B, n_kv, max_len,
-    D*bits/32], scales, biases [B, n_kv, max_len, D/group_size]) triples, with `offset`, `group_size` and `bits`.
-    The decode step writes and reads it with gbxq_rope_cache_quantized / gbxq_decode_attention_quantized."""
-
-    def __init__(self, batch: int, n_kv: int, max_len: int, head_dim: int, device, group_size: int = 64, bits: int = 8,
-                 dtype=torch.bfloat16):
-        if bits not in (2, 3, 4, 6, 8) or group_size not in (32, 64, 128) or head_dim % group_size or head_dim % 32:
-            raise ValueError(f"QuantizedKVCache: bits {bits} / group_size {group_size} do not fit head_dim {head_dim}")
-
-        def side():
-            lead = (batch, n_kv, max_len)
-            return (torch.zeros((*lead, head_dim * bits // 32), dtype=torch.int32, device=device).view(torch.uint32),
-                    torch.zeros((*lead, head_dim // group_size), dtype=dtype, device=device),
-                    torch.zeros((*lead, head_dim // group_size), dtype=dtype, device=device))
-
-        self.keys, self.values = side(), side()
-        self.max_len = max_len
-        self.offset = 0
-        self.group_size, self.bits = group_size, bits
-
-    def update(self, k: torch.Tensor, v: torch.Tensor, at: int):
-        """k / v [B, n_kv, L, D] quantized into positions [at, at + L) (ops.quantize_into, one launch per side)."""
-        ops.quantize_into(k, self.keys, at, self.group_size, self.bits)
-        ops.quantize_into(v, self.values, at, self.group_size, self.bits)
-
-    def prefix(self, n: int):
-        return tuple(t[:, :, :n] for t in self.keys), tuple(t[:, :, :n] for t in self.values)
-
-
-def cache_device(c) -> torch.device:
-    return (c.keys[0] if isinstance(c, QuantizedKVCache) else c.keys).device
-
-
-def make_prompt_cache(model, batch: int = 1, max_len: int = 4096) -> List[KVCache]:
+def make_prompt_cache(model, batch: int = 1, max_len: int = 4096) -> List[StaticKVCache]:
     a = model.args
     hd = a.head_dim or a.hidden_size // a.num_attention_heads
     dev = model.model.embed_tokens.weight.device
     n_kv = a.num_key_value_heads // model.tp.world
-    return [KVCache(batch, n_kv, max_len, hd, dev) for _ in range(a.num_hidden_layers)]
+    return [StaticKVCache(batch, n_kv, max_len, hd, dev) for _ in range(a.num_hidden_layers)]
 
 
 class Attention(nn.Module):  # gbx_lm/models/qllama.py:39-96
@@ -206,67 +144,55 @@ class Attention(nn.Module):  # gbx_lm/models/qllama.py:39-96
         self.o_proj = QuantizedLinear(self.n_heads * head_dim, dim, bias=o_bias)
         self.rope = RoPE(head_dim, args.rope_theta, args.rope_traditional, args.rope_scaling)
 
-    def fused_quantized_ok(self, cache: "QuantizedKVCache") -> bool:
-        """Shapes gbxq_decode_attention_quantized serves (include/gbxq.h)."""
-        return (self.head_dim in (64, 128) and cache.group_size <= self.head_dim
-                and self.n_heads % self.n_kv_heads == 0 and self.n_heads // self.n_kv_heads <= 8)
+    def takes_fused_decode(self, cache: Union[StaticKVCache, StaticQuantizedKVCache]) -> bool:
+        """Whether a decode step on `cache` runs the fused kernel pair of the cache's type: GBXQ_FUSED_DECODE on and
+        shapes the pair serves."""
+        return FUSED_DECODE and cache.fused_decode_fits(self.head_dim, self.n_heads, self.n_kv_heads)
 
-    def forward(self, x, positions, cache: Optional[Union[KVCache, "QuantizedKVCache"]], attend_len: Optional[int]):
+    def forward(self, x, positions, cache: Optional[Union[StaticKVCache, StaticQuantizedKVCache]],
+                attend_len: Optional[int]):
         B, L, _ = x.shape
         # one grouped launch for the three projections of x (ref qllama.py:76 calls them back to back)
         q, k, v = ops.quantized_matmul_grouped(x, (self.q_proj, self.k_proj, self.v_proj))
-        if isinstance(cache, QuantizedKVCache):
-            return self._forward_quantized(x, q, k, v, positions, cache, attend_len)
-        if fused_decode_ok(x, L, cache) and self.head_dim in (64, 128) and cache.max_len <= 49152:
-            # decode step: RoPE + cache write in one launch, one-query attention in another (SURVEY.md 8f rank 2)
+        quantized = isinstance(cache, StaticQuantizedKVCache)
+        if fused_decode_ok(x, L, cache) and self.takes_fused_decode(cache):
+            # decode step: RoPE + cache write in one launch, one-query attention in another (SURVEY.md 8f rank 2); over
+            # the quantized cache the attention is split-K on the codes (+ its combine launch)
             qh = q.view(B, self.n_heads, self.head_dim)
-            ops.rope_cache(qh, k.view(B, self.n_kv_heads, self.head_dim), v.view(B, self.n_kv_heads, self.head_dim),
-                           positions, self.rope.inv_freq, cache.keys, cache.values)
-            out = ops.decode_attention(qh, cache.keys, cache.values, positions, self.scale, attend_len)
+            kh, vh = k.view(B, self.n_kv_heads, self.head_dim), v.view(B, self.n_kv_heads, self.head_dim)
+            if quantized:
+                gs, bits = cache.group_size, cache.bits
+                ops.rope_cache_quantized(qh, kh, vh, positions, self.rope.inv_freq, cache.keys, cache.values, gs, bits)
+                out = ops.decode_attention_quantized(qh, cache.keys, cache.values, positions, self.scale, gs, bits,
+                                                     attend_len)
+            else:
+                ops.rope_cache(qh, kh, vh, positions, self.rope.inv_freq, cache.keys, cache.values)
+                out = ops.decode_attention(qh, cache.keys, cache.values, positions, self.scale, attend_len)
             return self.tp.row_parallel(self.o_proj, out.view(B, 1, -1))
-        q = q.view(B, L, self.n_heads, -1).transpose(1, 2)
-        k = k.view(B, L, self.n_kv_heads, -1).transpose(1, 2)
-        v = v.view(B, L, self.n_kv_heads, -1).transpose(1, 2)
-        q = self.rope(q, positions)
-        k = self.rope(k, positions)
-        if cache is not None:
-            cache.update(k, v, positions)
-            T = attend_len if attend_len is not None else cache.max_len
-            keys, values = cache.keys[:, :, :T], cache.values[:, :, :T]
-        else:
-            T = L
-            keys, values = k, v
-        # causal over absolute positions: key j visible to query at position p iff j <= p
-        mask = torch.arange(T, device=x.device)[None, :] <= positions[:, None]
-        out = F.scaled_dot_product_attention(q, keys, values, attn_mask=mask[None, None], scale=self.scale,
-                                             enable_gqa=self.n_heads != self.n_kv_heads)
-        out = out.transpose(1, 2).reshape(B, L, -1)
-        return self.tp.row_parallel(self.o_proj, out)
-
-    def _forward_quantized(self, x, q, k, v, positions, cache: "QuantizedKVCache", attend_len: Optional[int]):
-        B, L, _ = x.shape
-        gs, bits = cache.group_size, cache.bits
-        if fused_decode_ok(x, L, cache) and self.fused_quantized_ok(cache):
-            # decode step: RoPE + quantized cache write in one launch, split-K attention over the codes (+ its combine)
-            qh = q.view(B, self.n_heads, self.head_dim)
-            ops.rope_cache_quantized(qh, k.view(B, self.n_kv_heads, self.head_dim), v.view(B, self.n_kv_heads, self.head_dim),
-                                     positions, self.rope.inv_freq, cache.keys, cache.values, gs, bits)
-            out = ops.decode_attention_quantized(qh, cache.keys, cache.values, positions, self.scale, gs, bits, attend_len)
-            return self.tp.row_parallel(self.o_proj, out.view(B, 1, -1))
-        # prefill chunks and the unfused path: the reference's own (QuantizedKVCache.update_and_fetch +
-        # quantized_scaled_dot_product_attention, gbx_lm/models/base.py:65-98).  The rows are written at the HOST offset
-        # (Model.forward has already advanced it past these L positions), so this path is not graph-capturable.
-        from .switch_layers import quantized_scaled_dot_product_attention
-
         q = self.rope(q.view(B, L, self.n_heads, -1).transpose(1, 2), positions)
         k = self.rope(k.view(B, L, self.n_kv_heads, -1).transpose(1, 2), positions)
         v = v.view(B, L, self.n_kv_heads, -1).transpose(1, 2)
-        T = cache.offset
-        cache.update(k, v, T - L)
-        keys, values = cache.prefix(T)
-        mask = torch.zeros((L, T), dtype=q.dtype, device=x.device)
-        mask.masked_fill_(torch.arange(T, device=x.device)[None, :] > positions[:, None], float("-inf"))
-        out = quantized_scaled_dot_product_attention(q, keys, values, self.scale, mask, group_size=gs, bits=bits)
+        if cache is None:
+            T, keys, values = L, k, v
+        elif quantized:
+            # the rows are written at the HOST offset (Model.forward has already advanced it past these L positions), so
+            # this path is not graph-capturable
+            T = cache.offset
+            cache.update(k, v, T - L)
+            keys, values = cache.prefix(T)
+        else:
+            cache.update(k, v, positions)
+            T = attend_len if attend_len is not None else cache.max_len
+            keys, values = cache.keys[:, :, :T], cache.values[:, :, :T]
+        # causal over absolute positions: key j visible to query at position p iff j <= p
+        visible = torch.arange(T, device=x.device)[None, :] <= positions[:, None]
+        if quantized:
+            # the reference's attention on the codes (gbx_lm/models/base.py:65-98), with its additive mask
+            mask = torch.zeros((L, T), dtype=q.dtype, device=x.device).masked_fill_(~visible, float("-inf"))
+            out = quantized_scaled_dot_product_attention(q, keys, values, self.scale, mask, cache.group_size, cache.bits)
+        else:
+            out = F.scaled_dot_product_attention(q, keys, values, attn_mask=visible[None, None], scale=self.scale,
+                                                 enable_gqa=self.n_heads != self.n_kv_heads)
         out = out.transpose(1, 2).reshape(B, L, -1)
         return self.tp.row_parallel(self.o_proj, out)
 
@@ -343,7 +269,7 @@ class Model(nn.Module):  # gbx_lm/models/qllama.py:177-209
         if not args.tie_word_embeddings:
             self.lm_head = nn.Linear(args.hidden_size, args.vocab_size, bias=False)
 
-    def forward(self, inputs: torch.Tensor, cache: Optional[List[KVCache]] = None,
+    def forward(self, inputs: torch.Tensor, cache: Optional[List[Union[StaticKVCache, StaticQuantizedKVCache]]] = None,
                 positions: Optional[torch.Tensor] = None, attend_len: Optional[int] = None, hidden_states: bool = False):
         """inputs int64 [B, L].  positions int64 [L] (absolute); default = cache offset .. offset+L.
         attend_len: number of cache positions attended (None = whole static cache, for graph replay)."""

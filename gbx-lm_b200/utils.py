@@ -24,6 +24,7 @@ import torch
 from torch import nn
 
 from . import qllama, qqwen2
+from .cache import StaticKVCache, StaticQuantizedKVCache, maybe_quantize_kv_cache
 from .quantized_linear import QuantizedLinear
 from .tp import TPContext, proj_kind, shard_tensor
 
@@ -311,14 +312,12 @@ class DecodeGraph:
     7*L QuantizedLinear launches plus the glue -- replays as one submission (SURVEY.md 7.2 item 1)."""
 
     def __init__(self, model, cache, batch: int = 1):
-        if any(isinstance(c, qllama.QuantizedKVCache) for c in cache):
-            # the unfused quantized path writes at the HOST offset, which a replay cannot advance
-            attns = [layer.self_attn for layer in model.layers]
-            if not qllama.FUSED_DECODE or not all(a.fused_quantized_ok(c) for a, c in zip(attns, cache)):
-                raise ValueError("DecodeGraph: a quantized KV cache is graph-capturable only on the fused decode path "
-                                 "(GBXQ_FUSED_DECODE on, head_dim 64 / 128, group_size <= head_dim, Hq/Hkv <= 8)")
+        # the unfused quantized path writes at the HOST offset, which a replay cannot advance
+        if any(isinstance(c, StaticQuantizedKVCache) and not layer.self_attn.takes_fused_decode(c)
+               for layer, c in zip(model.layers, cache)):
+            raise ValueError("DecodeGraph: a quantized KV cache is graph-capturable only on the fused decode path")
         self.model, self.cache = model, cache
-        dev = qllama.cache_device(cache[0])
+        dev = cache[0].device
         self.tok = torch.zeros((batch, 1), dtype=torch.long, device=dev)
         self.pos = torch.zeros((1,), dtype=torch.long, device=dev)
         self.logits = None
@@ -364,8 +363,6 @@ class DecodeGraph:
 def _kv_quantizer(cache: list, kv_bits: Optional[int], kv_group_size: int, quantized_kv_start: int) -> Callable[[], bool]:
     """The reference's check after every model call (gbx_lm/utils.py:204-214, 268-270): maybe_quantize_kv_cache on the
     list; returns True when this call converted it."""
-    from .cache import maybe_quantize_kv_cache
-
     def step() -> bool:
         before = cache[0]
         maybe_quantize_kv_cache(cache, quantized_kv_start, kv_group_size, kv_bits)
@@ -381,6 +378,22 @@ def _decode_graph(model, cache, tok, position: int, device_loop: int = 0) -> Opt
     except ValueError:
         return None
     return dg.capture(tok, position, device_loop=device_loop)
+
+
+def prefill(model, prompt: torch.Tensor, cache: list, prefill_step_size: int = 2048, kv_bits: Optional[int] = None,
+            kv_group_size: int = 64, quantized_kv_start: int = 0) -> torch.Tensor:
+    """The prompt (token ids [n], on the model's device) through the model in `prefill_step_size` chunks, with the
+    conversion rule of `generate_step` applied after every model call; returns the logits of the last position [1, V]."""
+    quantize_cache = _kv_quantizer(cache, kv_bits, kv_group_size, quantized_kv_start)
+    y = prompt.reshape(-1)
+    with torch.no_grad():
+        while y.numel() > prefill_step_size:
+            model(y[:prefill_step_size][None], cache)
+            quantize_cache()
+            y = y[prefill_step_size:]
+        logits = model(y[None], cache)[:, -1, :]
+        quantize_cache()
+    return logits
 
 
 def generate_step(
@@ -408,20 +421,15 @@ def generate_step(
     sampler = sampler or (lambda lp: torch.argmax(lp, dim=-1))
     max_len = max_kv_size or (y.numel() + max_tokens + 1)
     cache = prompt_cache if prompt_cache is not None else qllama.make_prompt_cache(model, 1, max_len)
-    quantize_cache = _kv_quantizer(cache, kv_bits, kv_group_size, quantized_kv_start)
+    kv = dict(kv_bits=kv_bits, kv_group_size=kv_group_size, quantized_kv_start=quantized_kv_start)
+    quantize_cache = _kv_quantizer(cache, **kv)
 
     def _logprobs(logits):
         logits = logits.float()
         return logits - torch.logsumexp(logits, dim=-1, keepdim=True)
 
     with torch.no_grad():
-        while y.numel() > prefill_step_size:
-            model(y[:prefill_step_size][None], cache)
-            quantize_cache()
-            y = y[prefill_step_size:]
-        logits = model(y[None], cache)[:, -1, :]
-        quantize_cache()
-        lp = _logprobs(logits)
+        lp = _logprobs(prefill(model, y, cache, prefill_step_size, **kv))
         tok = sampler(lp)
         use_graph = use_cuda_graph and tok.is_cuda
         dg = _decode_graph(model, cache, tok, cache[0].offset) if use_graph else None
@@ -455,47 +463,41 @@ def generate_tokens_device(model, prompt: torch.Tensor, max_tokens: int = 128, p
     y = prompt.reshape(-1).to(next(model.parameters()).device)
     n_prompt = y.numel()
     cache = qllama.make_prompt_cache(model, 1, n_prompt + max_tokens + 1)
-    quantize_cache = _kv_quantizer(cache, kv_bits, kv_group_size, quantized_kv_start)
+    kv = dict(kv_bits=kv_bits, kv_group_size=kv_group_size, quantized_kv_start=quantized_kv_start)
     t0 = time.perf_counter()
-    with torch.no_grad():
-        while y.numel() > prefill_step_size:
-            model(y[:prefill_step_size][None], cache)
-            quantize_cache()
-            y = y[prefill_step_size:]
-        tok = torch.argmax(model(y[None], cache)[:, -1, :].float(), dim=-1)
-        quantize_cache()
+    tok = torch.argmax(prefill(model, y, cache, prefill_step_size, **kv).float(), dim=-1)
     pos0 = cache[0].offset
     steps = max(max_tokens - 1, 0)
     # replay i decodes position pos0 + i; the reference converts after the call that takes the offset past
-    # quantized_kv_start, i.e. after replay max(0, quantized_kv_start - pos0)
-    convert_at = steps
-    if kv_bits is not None and isinstance(cache[0], qllama.KVCache):
-        convert_at = min(max(quantized_kv_start - pos0, 0), steps)
-    dg = _decode_graph(model, cache, tok, pos0, device_loop=max(min(convert_at + 1, steps), 1))
-    if dg is None:
-        raise ValueError("generate_tokens_device: the quantized cache cannot be captured (unfused decode path)")
-    first = int(tok.item())
-    t_first = time.perf_counter()
-    outs = []
-    for _ in range(min(convert_at + 1, steps)):
-        dg.graph.replay()
-    outs.append(dg.out[: min(convert_at + 1, steps), 0])
-    done = min(convert_at + 1, steps)
-    if done < steps:
-        for c in cache:
-            c.offset = pos0 + done
-        quantize_cache()
-        dg = _decode_graph(model, cache, dg.tok[:, 0].clone(), pos0 + done, device_loop=steps - done)
+    # quantized_kv_start, i.e. after replay max(0, quantized_kv_start - pos0): the replays up to there are one segment,
+    # the rest a second one on a graph of the quantized step
+    head = steps
+    if kv_bits is not None and isinstance(cache[0], StaticKVCache):
+        head = min(max(quantized_kv_start - pos0, 0) + 1, steps)
+    segments = [head] + ([steps - head] if head < steps else [])
+    outs, pos = [], pos0
+    for i, n in enumerate(segments):
+        if i:  # at the conversion: convert the caches, continue from the last token on a graph of the quantized step
+            for c in cache:
+                c.offset = pos
+            maybe_quantize_kv_cache(cache, quantized_kv_start, kv_group_size, kv_bits)
+            tok = dg.tok[:, 0].clone()
+        # captured even for zero replays (max_tokens 1): the cache is checked for capturability all the same
+        dg = _decode_graph(model, cache, tok, pos, device_loop=max(n, 1))
         if dg is None:
             raise ValueError("generate_tokens_device: the quantized cache cannot be captured (unfused decode path)")
-        for _ in range(steps - done):
+        if i == 0:  # the capture of the first graph counts as prompt time
+            first = int(tok.item())
+            t_first = time.perf_counter()
+        for _ in range(n):
             dg.graph.replay()
-        outs.append(dg.out[: steps - done, 0])
+        outs.append(dg.out[:n, 0])
+        pos += n
     torch.cuda.synchronize()
     t1 = time.perf_counter()
     toks = [first] + [int(t) for o in outs for t in o.tolist()]
     for c in cache:
-        c.offset = pos0 + steps
+        c.offset = pos
     stats = {
         "prompt_tokens": int(n_prompt), "prompt_tps": n_prompt / max(t_first - t0, 1e-9),
         "generation_tokens": len(toks), "generation_tps": max(len(toks) - 1, 1) / max(t1 - t_first, 1e-9),

@@ -8,6 +8,7 @@ import pytest
 import torch
 
 from gbx_lm_b200 import ops, qllama, switch_layers, utils, workloads as W
+from gbx_lm_b200.cache import DECODE_ATTENTION_MAX_KEYS, StaticQuantizedKVCache
 from oracle import mlx_affine as A
 from tests import ref_model
 
@@ -117,7 +118,7 @@ def test_decode_attention_quantized_long_context(cuda_device, bits):
     g = torch.Generator(device=cuda_device).manual_seed(6)
     q = torch.randn((B, Hq, D), generator=g, device=cuda_device).to(torch.bfloat16)
     kd, vd = _oracle_deq(k3, gs, bits).to(cuda_device), _oracle_deq(v3, gs, bits).to(cuda_device)
-    for pos in (n - 1, 49152, 1000):
+    for pos in (n - 1, DECODE_ATTENTION_MAX_KEYS, 1000):
         p = torch.tensor([pos], device=cuda_device)
         got = ops.decode_attention_quantized(q, k3, v3, p, D ** -0.5, gs, bits)
         _close(got, _ref_attention(q, kd, vd, pos, D ** -0.5))
@@ -157,7 +158,7 @@ def _model(tmp_path, name, cuda_device, seed=5):
 
 @pytest.mark.parametrize("kv_bits", (4, 8))
 @pytest.mark.parametrize("name", ("tiny-llama", "tiny-qwen2"))
-def test_fused_quantized_decode_matches_unfused(cuda_device, tmp_path, monkeypatch, name, kv_bits):
+def test_fused_decode_on_static_quantized_cache_matches_unfused(cuda_device, tmp_path, monkeypatch, name, kv_bits):
     dims, _, model = _model(tmp_path, name, cuda_device)
     toks = torch.randint(0, dims.vocab, (1, 40), generator=torch.Generator().manual_seed(4)).to(cuda_device)
 
@@ -170,7 +171,7 @@ def test_fused_quantized_decode_matches_unfused(cuda_device, tmp_path, monkeypat
             cache[:] = [c.to_quantized(64, kv_bits) for c in cache]
             for i in range(8, 40):
                 outs.append(model(toks[:, i:i + 1], cache).float())
-        assert isinstance(cache[0], qllama.QuantizedKVCache) and cache[0].offset == 40
+        assert isinstance(cache[0], StaticQuantizedKVCache) and cache[0].offset == 40
         return torch.cat(outs, 1)
 
     a, b = run(True), run(False)
@@ -180,18 +181,21 @@ def test_fused_quantized_decode_matches_unfused(cuda_device, tmp_path, monkeypat
     assert clear.sum() >= 10 and (a.argmax(-1)[clear] == b.argmax(-1)[clear]).all()
 
 
-@pytest.mark.parametrize("kv_bits,start", [(4, 0), (8, 0), (4, 20), (8, 20)])
+@pytest.mark.parametrize("kv_bits,start,max_tokens",
+                         [(4, 0, 40), (8, 0, 40), (4, 20, 40), (8, 20, 40), (4, 11, 40), (8, 100, 40), (4, 12, 1), (8, 0, 1)],
+                         ids=["4-0", "8-0", "4-20", "8-20", "4-11", "8-100", "4-12-max1", "8-0-max1"])
 @pytest.mark.parametrize("name", ("tiny-llama", "tiny-qwen2"))
-def test_generate_with_quantized_cache_graph_eager_device(cuda_device, tmp_path, name, kv_bits, start):
-    """start 0: converted after the first prefill call; start 20 with a 12-token prompt: converted mid-decode (the graph
-    is captured again, the device loop replays up to the conversion and continues on a new graph)."""
+def test_generate_with_quantized_cache_graph_eager_device(cuda_device, tmp_path, name, kv_bits, start, max_tokens):
+    """With a 12-token prompt: start 0 converts after the first prefill call, start 11 right after the prompt, start 20
+    mid-decode (the graph is captured again, the device loop replays up to the conversion and continues on a new graph),
+    start 100 never; max_tokens 1 yields the prefill's token alone."""
     dims, _, model = _model(tmp_path, name, cuda_device, seed=11)
     prompt = torch.randint(0, dims.vocab, (12,), generator=torch.Generator().manual_seed(3))
     kw = dict(kv_bits=kv_bits, kv_group_size=64, quantized_kv_start=start)
-    g_toks, _ = utils.generate_tokens(model, prompt, max_tokens=40, use_cuda_graph=True, **kw)
-    e_toks, _ = utils.generate_tokens(model, prompt, max_tokens=40, use_cuda_graph=False, **kw)
-    d_toks, stats = utils.generate_tokens_device(model, prompt, max_tokens=40, **kw)
-    assert len(g_toks) == 40 and g_toks == e_toks and d_toks == g_toks and stats["generation_tps"] > 0
+    g_toks, _ = utils.generate_tokens(model, prompt, max_tokens=max_tokens, use_cuda_graph=True, **kw)
+    e_toks, _ = utils.generate_tokens(model, prompt, max_tokens=max_tokens, use_cuda_graph=False, **kw)
+    d_toks, stats = utils.generate_tokens_device(model, prompt, max_tokens=max_tokens, **kw)
+    assert len(g_toks) == max_tokens and g_toks == e_toks and d_toks == g_toks and stats["generation_tps"] > 0
     c_toks, _ = utils.generate_tokens(model, prompt, max_tokens=16, prefill_step_size=5, **kw)  # conversion mid-prefill
     assert len(c_toks) == 16
 

@@ -1,7 +1,7 @@
 """CPU tests of the quantized-KV decode path: the C-level argument validation of gbxq_rope_cache_quantized /
 gbxq_decode_attention_quantized and the workspace query (no GPU needed: validation fails before any CUDA call), the
-argument checks of the Python ops, the static quantized cache of qllama and its conversion rule, with the device
-quantiser stubbed by the oracle."""
+argument checks of the Python ops, the static caches of cache.py and their conversion rule, with the device quantiser
+stubbed by the oracle."""
 import ctypes
 
 import numpy as np
@@ -91,21 +91,21 @@ def test_quantized_ops_refuse_cpu_tensors_and_bad_triples():
         chk(q, k3[:2], v3, 64, 4)                                         # not a triple
 
 
-def test_static_quantized_cache_shapes():
-    from gbx_lm_b200 import qllama
+def test_static_quantized_kv_cache_shapes():
+    from gbx_lm_b200.cache import StaticQuantizedKVCache
 
     for bits in (2, 3, 4, 6, 8):
         for d, gss in ((64, (32, 64)), (128, (32, 64, 128))):
             for gs in gss:
-                c = qllama.QuantizedKVCache(2, 3, 40, d, "cpu", group_size=gs, bits=bits)
+                c = StaticQuantizedKVCache(2, 3, 40, d, "cpu", group_size=gs, bits=bits)
                 for side in (c.keys, c.values):
                     assert side[0].shape == (2, 3, 40, d * bits // 32) and side[0].dtype == torch.uint32
                     assert side[1].shape == side[2].shape == (2, 3, 40, d // gs) and side[1].dtype == torch.bfloat16
                 assert (c.offset, c.group_size, c.bits, c.max_len) == (0, gs, bits, 40)
-    assert qllama.QuantizedKVCache(1, 1, 8, 128, "cpu", 64, 3).keys[0].shape[-1] == 12   # 3-bit: 128 * 3 / 32 words
-    assert qllama.QuantizedKVCache(1, 1, 8, 64, "cpu", 32, 6).keys[0].shape[-1] == 12    # 6-bit: 64 * 6 / 32 words
+    assert StaticQuantizedKVCache(1, 1, 8, 128, "cpu", 64, 3).keys[0].shape[-1] == 12   # 3-bit: 128 * 3 / 32 words
+    assert StaticQuantizedKVCache(1, 1, 8, 64, "cpu", 32, 6).keys[0].shape[-1] == 12    # 6-bit: 64 * 6 / 32 words
     with pytest.raises(ValueError):
-        qllama.QuantizedKVCache(1, 1, 8, 64, "cpu", group_size=128, bits=4)
+        StaticQuantizedKVCache(1, 1, 8, 64, "cpu", group_size=128, bits=4)
 
 
 def _oracle_quantize(x, group_size, bits):
@@ -118,15 +118,14 @@ def _i32(t):
     return t.view(torch.int32) if t.dtype == torch.uint32 else t
 
 
-def test_static_to_quantized_and_conversion_rule(monkeypatch):
-    from gbx_lm_b200 import cache, qllama
+def test_static_kv_cache_to_quantized_and_conversion_rule(monkeypatch):
+    from gbx_lm_b200 import cache, ops
 
-    monkeypatch.setattr(qllama.KVCache, "_quantize", staticmethod(_oracle_quantize))
-    monkeypatch.setattr(cache.KVCache, "_quantize", staticmethod(_oracle_quantize))
+    monkeypatch.setattr(ops, "quantize", _oracle_quantize)
     gen = torch.Generator().manual_seed(3)
 
     def filled(n):
-        cs = [qllama.KVCache(1, 2, 32, 64, "cpu") for _ in range(3)]
+        cs = [cache.StaticKVCache(1, 2, 32, 64, "cpu") for _ in range(3)]
         for c in cs:
             c.keys[:, :, :n] = torch.randn((1, 2, n, 64), generator=gen).to(torch.bfloat16)
             c.values[:, :, :n] = torch.randn((1, 2, n, 64), generator=gen).to(torch.bfloat16)
@@ -135,7 +134,7 @@ def test_static_to_quantized_and_conversion_rule(monkeypatch):
 
     cs = filled(10)
     q = cs[0].to_quantized(group_size=32, bits=4)
-    assert isinstance(q, qllama.QuantizedKVCache) and (q.offset, q.max_len, q.group_size, q.bits) == (10, 32, 32, 4)
+    assert isinstance(q, cache.StaticQuantizedKVCache) and (q.offset, q.max_len, q.group_size, q.bits) == (10, 32, 32, 4)
     for got, want in zip(q.keys + q.values, _oracle_quantize(cs[0].keys, 32, 4) + _oracle_quantize(cs[0].values, 32, 4)):
         assert got.shape == want.shape and torch.equal(_i32(got), _i32(want))
     assert (_i32(q.keys[0])[:, :, 10:] == 0).all() and (q.keys[2][:, :, 10:] == 0).all()  # unused rows: zero groups
@@ -145,7 +144,7 @@ def test_static_to_quantized_and_conversion_rule(monkeypatch):
         cs = filled(10)
         cache.maybe_quantize_kv_cache(cs, quantized_kv_start=start, kv_group_size=64, kv_bits=kv_bits)
         kinds = {type(c) for c in cs}
-        assert kinds == ({qllama.QuantizedKVCache} if converts else {qllama.KVCache}), (start, kv_bits)
+        assert kinds == ({cache.StaticQuantizedKVCache} if converts else {cache.StaticKVCache}), (start, kv_bits)
         if converts:
             assert all(c.bits == kv_bits and c.group_size == 64 and c.offset == 10 for c in cs)
     # a list that is already quantized is left alone

@@ -178,11 +178,11 @@ def _oracle_quantize_into(x, out, offset, group_size, bits):
 
 
 @pytest.fixture()
-def stubbed_caches(monkeypatch):
-    from gbx_lm_b200 import cache
+def cache_on_oracle_ops(monkeypatch):
+    from gbx_lm_b200 import cache, ops
 
-    monkeypatch.setattr(cache.QuantizedKVCache, "_quantize_into", staticmethod(_oracle_quantize_into))
-    monkeypatch.setattr(cache.KVCache, "_quantize", staticmethod(_oracle_quantize))
+    monkeypatch.setattr(ops, "quantize_into", _oracle_quantize_into)
+    monkeypatch.setattr(ops, "quantize", _oracle_quantize)
     return cache
 
 
@@ -190,8 +190,8 @@ def _i32(t):
     return t.view(torch.int32) if t.dtype == torch.uint32 else t
 
 
-def test_quantized_kv_cache_growth_trim_and_state(stubbed_caches):
-    cache = stubbed_caches
+def test_quantized_kv_cache_growth_trim_and_state_with_oracle_ops(cache_on_oracle_ops):
+    cache = cache_on_oracle_ops
     B, H, D, gs, bits = 1, 2, 64, 32, 4
     gen = torch.Generator().manual_seed(0)
     c = cache.QuantizedKVCache(group_size=gs, bits=bits)
@@ -234,8 +234,8 @@ def test_quantized_kv_cache_growth_trim_and_state(stubbed_caches):
     assert torch.equal(_i32(qk2[0])[..., :255, :], _i32(k_state[0]))
 
 
-def test_quantized_kv_cache_straddling_widths_allocate_the_stream_length(stubbed_caches):
-    cache = stubbed_caches
+def test_quantized_kv_cache_straddling_widths_allocate_the_stream_length_with_oracle_ops(cache_on_oracle_ops):
+    cache = cache_on_oracle_ops
     for bits in (3, 6):
         c = cache.QuantizedKVCache(group_size=64, bits=bits)
         k = torch.randn((1, 1, 2, 128)).to(torch.bfloat16)
@@ -245,8 +245,8 @@ def test_quantized_kv_cache_straddling_widths_allocate_the_stream_length(stubbed
         assert torch.equal(_i32(qk[0]), _i32(want[0]))
 
 
-def test_kv_cache_to_quantized_and_maybe_quantize(stubbed_caches):
-    cache = stubbed_caches
+def test_kv_cache_to_quantized_and_maybe_quantize_with_oracle_ops(cache_on_oracle_ops):
+    cache = cache_on_oracle_ops
     gen = torch.Generator().manual_seed(1)
     caches = [cache.KVCache() for _ in range(2)]
     k = torch.randn((1, 2, 10, 64), generator=gen).to(torch.bfloat16)

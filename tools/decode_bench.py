@@ -59,7 +59,7 @@ def main():
 
 def run(args, dims, strat, model, prompt, kv_bits, t_write, t_load):
     from gbx_lm_b200 import qllama
-    from gbx_lm_b200.cache import maybe_quantize_kv_cache
+    from gbx_lm_b200.cache import StaticQuantizedKVCache
 
     kw = dict(kv_bits=kv_bits, kv_group_size=args.kv_group_size, quantized_kv_start=args.quantized_kv_start)
     best, toks0 = None, None
@@ -78,15 +78,8 @@ def run(args, dims, strat, model, prompt, kv_bits, t_write, t_load):
     # device time of the captured decode step alone (no sampling, no host sync between steps), on the cache the decode
     # runs on: converted after the prompt when kv_bits is set and the prompt is past quantized_kv_start
     cache = qllama.make_prompt_cache(model, 1, args.prompt + args.tokens + 1)
-    with torch.no_grad():
-        y = prompt.cuda()
-        while y.numel() > 2048:
-            model(y[:2048][None], cache)
-            maybe_quantize_kv_cache(cache, args.quantized_kv_start, args.kv_group_size, kv_bits)
-            y = y[2048:]
-        model(y[None], cache)
-        maybe_quantize_kv_cache(cache, args.quantized_kv_start, args.kv_group_size, kv_bits)
-    quantized = isinstance(cache[0], qllama.QuantizedKVCache)
+    utils.prefill(model, prompt.cuda(), cache, **kw)
+    quantized = isinstance(cache[0], StaticQuantizedKVCache)
     dg = utils.DecodeGraph(model, cache).capture(torch.tensor([1], device="cuda"), args.prompt)
     for _ in range(5):
         dg.graph.replay()

@@ -26,9 +26,9 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from gbx_lm_b200 import ops, switch_layers  # noqa: E402
+from gbx_lm_b200.cache import DECODE_ATTENTION_MAX_KEYS  # noqa: E402
 
 SHAPES = [("llama-3-8b", 32, 8, 128), ("llama-3.2-3b", 24, 8, 128), ("llama-3.2-1b", 32, 8, 64)]
-BF16_MAX_KEYS = 49152
 
 
 def hbm_peak():
@@ -102,7 +102,7 @@ def main():
             pos = torch.tensor([n - 1], device=dev)
             scale = d ** -0.5
             for kind in ("bf16", "q8", "q4", "qsdpa4"):
-                if kind == "bf16" and n > BF16_MAX_KEYS:
+                if kind == "bf16" and n > DECODE_ATTENTION_MAX_KEYS:
                     rows.append({"model": model, "keys": n, "cache": kind, "us": None, "note": "above the kernel's 49 152-key cap"})
                     print(f"{model:13s} keys {n:7d} {kind:7s}  -- above the bf16 kernel's 49 152-key cap")
                     continue
