@@ -40,6 +40,8 @@ EXPORTS = (
     "gbxq_rope_cache",
     "gbxq_decode_attention",
     "gbxq_rope_cache_quantized",
+    "gbxq_rope_cache_ring",
+    "gbxq_rope_cache_quantized_ring",
     "gbxq_decode_attention_quantized",
     "gbxq_decode_attention_quantized_workspace_bytes",
     "gbxq_add_rmsnorm",
@@ -156,6 +158,10 @@ def get() -> ctypes.CDLL:
     lib.gbxq_decode_attention.argtypes = [vp, vp, vp, vp, vp, ci, ci, ci, ci, i64, i64, cf, vp]
     lib.gbxq_rope_cache_quantized.restype = ci
     lib.gbxq_rope_cache_quantized.argtypes = [vp] * 11 + [ci, ci, ci, ci, i64, ci, ci, vp]
+    lib.gbxq_rope_cache_ring.restype = ci
+    lib.gbxq_rope_cache_ring.argtypes = [vp, vp, vp, vp, vp, vp, vp, ci, ci, ci, ci, i64, i64, vp]
+    lib.gbxq_rope_cache_quantized_ring.restype = ci
+    lib.gbxq_rope_cache_quantized_ring.argtypes = [vp] * 11 + [ci, ci, ci, ci, i64, i64, ci, ci, vp]
     lib.gbxq_decode_attention_quantized_workspace_bytes.restype = sz
     lib.gbxq_decode_attention_quantized_workspace_bytes.argtypes = [ci, ci, ci, ci, i64]
     lib.gbxq_decode_attention_quantized.restype = ci

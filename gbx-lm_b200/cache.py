@@ -12,11 +12,13 @@ Built differently underneath: both are one block-grown store (`_BlockStore`), tu
 `switch_layers.quantized_scaled_dot_product_attention` (gbx_lm/models/base.py:65-98).
 
 The static caches, `StaticKVCache` and `StaticQuantizedKVCache`, are what `qllama.Model` reads and writes: allocated
-once for `max_len` positions, so that the decode step is CUDA-graph capturable, in the same layouts.  The conversion
+once for `max_len` positions, so that the decode step is CUDA-graph capturable, in the same layouts.
+`StaticRotatingKVCache` and `StaticRotatingQuantizedKVCache` are their rotating forms (the reference's RotatingKVCache,
+`max_kv_size`): a window of `max_len` rows with `keep` sinks, written as a ring (`ring_slot`, `_Ring`).  The conversion
 rule `maybe_quantize_kv_cache` decides for both families.  CUDA only, like everything in this package."""
 from __future__ import annotations
 
-from typing import Callable, Optional, Sequence, Tuple
+from typing import Callable, List, Optional, Sequence, Tuple
 
 import torch
 
@@ -189,6 +191,8 @@ class StaticKVCache:
     models/cache.py:215-277; a static buffer keeps the decode step CUDA-graph capturable).  `offset` is the host-side
     count of valid positions (eager mode)."""
 
+    keep: Optional[int] = None  # sink rows of a rotating cache; None: a flat cache, position p in row p
+
     def __init__(self, batch: int, n_kv: int, max_len: int, head_dim: int, device, dtype=torch.bfloat16):
         self.keys = torch.zeros((batch, n_kv, max_len, head_dim), device=device, dtype=dtype)
         self.values = torch.zeros((batch, n_kv, max_len, head_dim), device=device, dtype=dtype)
@@ -198,6 +202,11 @@ class StaticKVCache:
     @property
     def device(self) -> torch.device:
         return self.keys.device
+
+    @property
+    def attend_len(self) -> int:
+        """Rows a model call attends once `offset` counts its positions."""
+        return self.offset
 
     def fused_decode_fits(self, head_dim: int, n_heads: int, n_kv_heads: int) -> bool:
         """Shapes gbxq_rope_cache + gbxq_decode_attention serve (include/gbxq.h)."""
@@ -223,6 +232,8 @@ class StaticQuantizedKVCache:
     [B, n_kv, max_len, D/group_size]) triples, with `offset`, `group_size` and `bits`.  The decode step writes and
     reads it with gbxq_rope_cache_quantized / gbxq_decode_attention_quantized."""
 
+    keep: Optional[int] = None  # as StaticKVCache.keep
+
     def __init__(self, batch: int, n_kv: int, max_len: int, head_dim: int, device, group_size: int = 64, bits: int = 8,
                  dtype=torch.bfloat16):
         if bits not in (2, 3, 4, 6, 8) or group_size not in (32, 64, 128) or head_dim % group_size or head_dim % 32:
@@ -237,6 +248,11 @@ class StaticQuantizedKVCache:
     def device(self) -> torch.device:
         return self.keys[0].device
 
+    @property
+    def attend_len(self) -> int:
+        """Rows a model call attends once `offset` counts its positions."""
+        return self.offset
+
     def fused_decode_fits(self, head_dim: int, n_heads: int, n_kv_heads: int) -> bool:
         """Shapes gbxq_rope_cache_quantized + gbxq_decode_attention_quantized serve (include/gbxq.h)."""
         return (head_dim in (64, 128) and self.group_size <= head_dim
@@ -249,6 +265,156 @@ class StaticQuantizedKVCache:
 
     def prefix(self, n: int):
         return tuple(t[:, :, :n] for t in self.keys), tuple(t[:, :, :n] for t in self.values)
+
+
+# The sink count of the reference's rotating caches: generate_step builds them through make_prompt_cache, which passes
+# keep=4 (gbx_lm/models/cache.py:280-420, RotatingKVCache; SURVEY.md section 2 row 5).
+DEFAULT_KV_KEEP = 4
+
+
+def ring_slot(p, window: int, keep: int):
+    """Row of a rotating cache (`window` rows, the first `keep` of them sinks) that holds absolute position p (an int or
+    an int64 tensor of positions):
+
+        ring_slot(p) = p                                       if p < window
+                     = keep + (p - keep) mod (window - keep)   otherwise
+
+    -- where the reference's in-place update puts a token (RotatingKVCache._update_in_place: the write index wraps to
+    `keep` at `max_size`).  The device computes the same rule (kv_cache_row, gbxq_common.cuh)."""
+    if isinstance(p, torch.Tensor):
+        return torch.where(p < window, p, keep + (p - keep) % (window - keep))
+    return p if p < window else keep + (p - keep) % (window - keep)
+
+
+class _Ring:
+    """What the two rotating caches add to their flat bases.  The buffers hold `window` = `max_len` rows for good;
+    `offset` counts every position processed (absolute, as the reference's `offset`).  Position p lives in row
+    ring_slot(p), and a query at position p sees key position j iff
+
+        j <= p  and  (j < keep  or  j > p - (window - keep))
+
+    -- the sinks and the last window - keep positions: min(p + 1, window) keys, the set a reference decode step sees.
+
+    A decode step writes its row on the device (gbxq_rope_cache_ring) and attends the first `attend_len` rows, which are
+    exactly the ring's contents in some order.  A call of L positions at off .. off + L - 1 that takes the ring past its
+    window (`wraps`) attends `window_with` (the valid rows plus its own keys) under `visible`, then `store`s the
+    positions that survive it."""
+
+    def _set_ring(self, window: int, keep: int):
+        if isinstance(window, bool) or not isinstance(window, int) or window < 1:
+            raise ValueError(f"rotating KV cache: window must be an int >= 1, got {window!r}")
+        if isinstance(keep, bool) or not isinstance(keep, int) or not 0 <= keep < window:
+            raise ValueError(f"rotating KV cache: keep must be an int in [0, window = {window}), got {keep!r}")
+        self.keep = keep
+
+    @property
+    def window(self) -> int:
+        return self.max_len
+
+    @property
+    def attend_len(self) -> int:
+        return min(self.offset, self.max_len)
+
+    def ring_slot(self, p):
+        return ring_slot(p, self.max_len, self.keep)
+
+    def held_positions(self, offset: Optional[int] = None) -> torch.Tensor:
+        """int64 [min(offset, window)] on the cache's device: the absolute position in each valid row after `offset`
+        positions (default: the cache's).  Row s >= keep of a wrapped ring holds last - ((last - s) mod (window - keep)),
+        last = offset - 1."""
+        offset = self.offset if offset is None else offset
+        s = torch.arange(min(offset, self.max_len), device=self.device)
+        if offset <= self.max_len:
+            return s
+        last = offset - 1
+        return torch.where(s < self.keep, s, last - (last - s) % (self.max_len - self.keep))
+
+    def visible(self, key_positions: torch.Tensor, positions: torch.Tensor) -> torch.Tensor:
+        """bool [L, T]: whether the query at positions[i] sees the key at key_positions[j]."""
+        j, p = key_positions[None, :], positions[:, None]
+        return (j <= p) & ((j < self.keep) | (j > p - (self.max_len - self.keep)))
+
+    def wraps(self) -> bool:
+        """Whether the model call that has just advanced `offset` past its positions reaches beyond the window."""
+        return self.offset > self.max_len
+
+    def store_runs(self, off: int, L: int) -> List[Tuple[int, int, int]]:
+        """(first chunk index, count, first row) of each contiguous run of the chunk at off .. off + L - 1 that survives
+        it: the positions p < keep and p >= off + L - (window - keep), each to ring_slot(p).  At most three runs (the
+        sinks, then the ring part, split where it wraps); no row is written twice."""
+        end, runs = off + L, []
+        if off < self.keep:
+            runs.append((0, min(end, self.keep) - off, off))
+        p = max(off, self.keep, end - (self.max_len - self.keep))
+        while p < end:
+            row = self.ring_slot(p)
+            n = min(end - p, self.max_len - row)
+            runs.append((p - off, n, row))
+            p += n
+        return runs
+
+
+class StaticRotatingKVCache(_Ring, StaticKVCache):
+    """`StaticKVCache` as a rotating window of `window` positions with `keep` sinks (the reference's RotatingKVCache,
+    gbx_lm/models/cache.py:280-420, as a static buffer; the rule is `_Ring`'s)."""
+
+    def __init__(self, batch: int, n_kv: int, window: int, head_dim: int, device, keep: int = DEFAULT_KV_KEEP,
+                 dtype=torch.bfloat16):
+        self._set_ring(window, keep)
+        super().__init__(batch, n_kv, window, head_dim, device, dtype)
+
+    def window_with(self, k: torch.Tensor, v: torch.Tensor, off: int):
+        """(keys, values, key positions): the valid rows before the chunk k / v [B, n_kv, L, D] at `off`, then the chunk."""
+        n = min(off, self.max_len)
+        pos = torch.arange(off, off + k.shape[-2], device=self.device)
+        return (torch.cat([self.keys[:, :, :n], k], 2), torch.cat([self.values[:, :, :n], v], 2),
+                torch.cat([self.held_positions(off), pos]))
+
+    def store(self, keys: torch.Tensor, values: torch.Tensor, off: int, L: int):
+        """The surviving positions of the chunk (the last L rows of `keys` / `values`) into their rows."""
+        base = keys.shape[-2] - L
+        for i, n, row in self.store_runs(off, L):
+            self.keys[:, :, row:row + n] = keys[:, :, base + i:base + i + n]
+            self.values[:, :, row:row + n] = values[:, :, base + i:base + i + n]
+
+    def to_quantized(self, group_size: int = 64, bits: int = 4) -> "StaticRotatingQuantizedKVCache":
+        """As `StaticKVCache.to_quantized`; rows, `keep` and `offset` carry over."""
+        q = StaticRotatingQuantizedKVCache.__new__(StaticRotatingQuantizedKVCache)
+        q.keys = tuple(ops.quantize(self.keys, group_size, bits))
+        q.values = tuple(ops.quantize(self.values, group_size, bits))
+        q.max_len, q.offset, q.group_size, q.bits, q.keep = self.max_len, self.offset, group_size, bits, self.keep
+        return q
+
+
+class StaticRotatingQuantizedKVCache(_Ring, StaticQuantizedKVCache):
+    """`StaticQuantizedKVCache` as a rotating window (the rule is `_Ring`'s).  The reference raises NotImplementedError
+    for a quantized rotating cache; here `kv_bits` and `max_kv_size` compose (DESIGN.md section 7)."""
+
+    def __init__(self, batch: int, n_kv: int, window: int, head_dim: int, device, keep: int = DEFAULT_KV_KEEP,
+                 group_size: int = 64, bits: int = 8, dtype=torch.bfloat16):
+        self._set_ring(window, keep)
+        super().__init__(batch, n_kv, window, head_dim, device, group_size, bits, dtype)
+
+    def window_with(self, k: torch.Tensor, v: torch.Tensor, off: int):
+        """As `StaticRotatingKVCache.window_with` on triples: the chunk is quantized first (ops.quantize)."""
+        n = min(off, self.max_len)
+        pos = torch.arange(off, off + k.shape[-2], device=self.device)
+        kq, vq = ops.quantize(k, self.group_size, self.bits), ops.quantize(v, self.group_size, self.bits)
+        return (tuple(_cat_positions(t[:, :, :n], c) for t, c in zip(self.keys, kq)),
+                tuple(_cat_positions(t[:, :, :n], c) for t, c in zip(self.values, vq)),
+                torch.cat([self.held_positions(off), pos]))
+
+    def store(self, keys, values, off: int, L: int):
+        """The surviving rows of the already quantized chunk (the last L rows of each triple) copied into their rows."""
+        base = keys[0].shape[-2] - L
+        for i, n, row in self.store_runs(off, L):
+            for dst, src in zip(self.keys + self.values, tuple(keys) + tuple(values)):
+                _rows(dst)[:, :, row:row + n] = _rows(src)[:, :, base + i:base + i + n]
+
+
+def _rows(t: torch.Tensor) -> torch.Tensor:
+    # uint32 codes have no copy kernel of their own: copied as int32
+    return t.view(torch.int32) if t.dtype == torch.uint32 else t
 
 
 def maybe_quantize_kv_cache(prompt_cache: list, quantized_kv_start: int, kv_group_size: int, kv_bits: Optional[int]) -> None:

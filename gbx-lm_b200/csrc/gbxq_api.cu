@@ -301,7 +301,17 @@ int gbxq_dequantize(const uint32_t* qweight, const void* scales, const void* bia
 int gbxq_rope_cache(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev, void* k_cache,
                     void* v_cache, int B, int Hq, int Hkv, int D, int64_t max_len, void* stream) {
     if (!q || !k || !v || !pos_dev || !inv_freq_dev || !k_cache || !v_cache) return GBXQ_ENULL;
-    return launch_rope_cache(q, k, v, pos_dev, inv_freq_dev, k_cache, v_cache, B, Hq, Hkv, D, max_len, (cudaStream_t)stream);
+    return launch_rope_cache(q, k, v, pos_dev, inv_freq_dev, k_cache, v_cache, B, Hq, Hkv, D, max_len, -1,
+                             (cudaStream_t)stream);
+}
+
+int gbxq_rope_cache_ring(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev,
+                         void* k_cache, void* v_cache, int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep,
+                         void* stream) {
+    if (!q || !k || !v || !pos_dev || !inv_freq_dev || !k_cache || !v_cache) return GBXQ_ENULL;
+    if (keep < 0 || keep >= max_len) return GBXQ_ESHAPE;
+    return launch_rope_cache(q, k, v, pos_dev, inv_freq_dev, k_cache, v_cache, B, Hq, Hkv, D, max_len, keep,
+                             (cudaStream_t)stream);
 }
 
 int gbxq_decode_attention(const void* q, const void* k_cache, const void* v_cache, const int64_t* pos_dev, void* out, int B,
@@ -316,7 +326,17 @@ int gbxq_rope_cache_quantized(void* q, const void* k, const void* v, const int64
                               void* v_biases, int B, int Hq, int Hkv, int D, int64_t max_len, int bits, int group_size,
                               void* stream) {
     const QCacheWrite a{q, k, v, pos_dev, inv_freq_dev, k_codes, k_scales, k_biases, v_codes, v_scales, v_biases,
-                        B, Hq, Hkv, D, max_len, bits, group_size};
+                        B, Hq, Hkv, D, max_len, bits, group_size, -1};
+    return launch_rope_cache_quantized(a, (cudaStream_t)stream);
+}
+
+int gbxq_rope_cache_quantized_ring(void* q, const void* k, const void* v, const int64_t* pos_dev,
+                                   const float* inv_freq_dev, uint32_t* k_codes, void* k_scales, void* k_biases,
+                                   uint32_t* v_codes, void* v_scales, void* v_biases, int B, int Hq, int Hkv, int D,
+                                   int64_t max_len, int64_t keep, int bits, int group_size, void* stream) {
+    if (keep < 0 || keep >= max_len) return GBXQ_ESHAPE;
+    const QCacheWrite a{q, k, v, pos_dev, inv_freq_dev, k_codes, k_scales, k_biases, v_codes, v_scales, v_biases,
+                        B, Hq, Hkv, D, max_len, bits, group_size, keep};
     return launch_rope_cache_quantized(a, (cudaStream_t)stream);
 }
 

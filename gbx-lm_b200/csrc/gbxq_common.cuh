@@ -90,6 +90,16 @@ __device__ __forceinline__ void extract_octet(const uint32_t* __restrict__ row, 
     for (int i = 0; i < 8; i++) q[i] = (uint32_t)((win >> (i * BITS)) & ((1u << BITS) - 1u));
 }
 
+// Row of a static KV cache of max_len rows that receives absolute position pos, or -1 for none (the decode-step cache
+// writes of gbxq_glue.cu / gbxq_qattn.cu).  keep < 0: a flat cache, row = pos, nothing outside [0, max_len).
+// keep in [0, max_len): a rotating cache of window max_len whose first keep rows are attention sinks; the rule of
+// cache.py's ring_slot: pos below max_len, keep + (pos - keep) mod (max_len - keep) from there.
+__device__ __forceinline__ int64_t kv_cache_row(int64_t pos, int64_t max_len, int64_t keep) {
+    if (pos < 0) return -1;
+    if (pos < max_len) return pos;
+    return keep < 0 ? -1 : keep + (pos - keep) % (max_len - keep);
+}
+
 // ------------------------------------------------------------------ small PTX wrappers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -213,8 +223,9 @@ int stream_plan(const gbxq_stream_call* calls, int ncalls, int64_t M, int dtype,
                 gbxq_stream_info* info);
 void stream_debug_patch(void* host_blob, int ncalls, unsigned long long* dbg_dev);
 int launch_stream(const gbxq_stream_info* info, const void* blob, void* counters, cudaStream_t st);
+// keep < 0: a flat cache; keep in [0, max_len): a rotating cache with keep sink rows (kv_cache_row)
 int launch_rope_cache(void* q, const void* k, const void* v, const int64_t* pos, const float* inv_freq, void* kc, void* vc,
-                      int B, int Hq, int Hkv, int D, int64_t max_len, cudaStream_t st);
+                      int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep, cudaStream_t st);
 int launch_decode_attention(const void* q, const void* kc, const void* vc, const int64_t* pos, void* out, int B, int Hq,
                             int Hkv, int D, int64_t max_len, int64_t attend_len, float scale, cudaStream_t st);
 // arguments of the quantized-cache decode step (gbxq_qattn.cu): one (codes, scales, biases) triple per side, bf16
@@ -231,6 +242,7 @@ struct QCacheWrite {
     int B, Hq, Hkv, D;
     int64_t max_len;
     int bits, gs;
+    int64_t keep;  // < 0: a flat cache; else the sink rows of a rotating cache (kv_cache_row)
 };
 struct QAttn {
     const void* q;

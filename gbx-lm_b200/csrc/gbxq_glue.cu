@@ -2,7 +2,8 @@
 // QuantizedLinear forwards of a block in the reference's callers (gbx_lm/models/qllama.py:76-141) as four small kernels
 // instead of ~45 framework launches per block:
 //   rope_cache        q, k <- RoPE(q, k) (mx.fast.rope, traditional=False; qllama.py:83-88), k / v written into the static
-//                     KV cache at the step's position (cache.update_and_fetch, qllama.py:85)
+//                     KV cache at the step's position (cache.update_and_fetch, qllama.py:85), or, on a rotating cache, at
+//                     the ring slot of that position (RotatingKVCache, gbx_lm/models/cache.py:280-420; kv_cache_row)
 //   decode_attention  one query row per head against the cache, causal over absolute positions, GQA
 //                     (scaled_dot_product_attention, qllama.py:90-93)
 //   add_rmsnorm       h = x + r (residual, qllama.py:137-141) and y = RMSNorm(h) * w (nn.RMSNorm) in one pass
@@ -34,15 +35,16 @@ __device__ __forceinline__ __nv_bfloat16 tobf(float v) { return __float2bfloat16
 __global__ void rope_cache_kernel(__nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ k,
                                   const __nv_bfloat16* __restrict__ v, const int64_t* __restrict__ pos_p,
                                   const float* __restrict__ inv_freq, __nv_bfloat16* __restrict__ kc,
-                                  __nv_bfloat16* __restrict__ vc, int Hq, int Hkv, int D, int64_t max_len) {
+                                  __nv_bfloat16* __restrict__ vc, int Hq, int Hkv, int D, int64_t max_len, int64_t keep) {
     const int h = blockIdx.x, b = blockIdx.y, i = threadIdx.x, half = D / 2;
     pdl_wait_then_trigger();
-    const int64_t pos = *pos_p;
-    if (pos < 0 || pos >= max_len) return;  // never write outside the cache
+    const int64_t pos = *pos_p;  // the RoPE angle is the absolute position's; k / v go to its cache row
+    const int64_t row = kv_cache_row(pos, max_len, keep);
+    if (row < 0) return;  // never write outside the cache
     if (h < Hq + Hkv) {
         const bool isq = h < Hq;
         const __nv_bfloat16* src = isq ? q + ((size_t)b * Hq + h) * D : k + ((size_t)b * Hkv + (h - Hq)) * D;
-        __nv_bfloat16* dst = isq ? q + ((size_t)b * Hq + h) * D : kc + (((size_t)b * Hkv + (h - Hq)) * max_len + pos) * D;
+        __nv_bfloat16* dst = isq ? q + ((size_t)b * Hq + h) * D : kc + (((size_t)b * Hkv + (h - Hq)) * max_len + row) * D;
         const float ang = __fmul_rn((float)pos, inv_freq[i]);
         const float c = cosf(ang), s = sinf(ang);
         const float x1 = bf(src[i]), x2 = bf(src[i + half]);
@@ -54,7 +56,7 @@ __global__ void rope_cache_kernel(__nv_bfloat16* __restrict__ q, const __nv_bflo
     } else {
         const int hv = h - Hq - Hkv;
         const __nv_bfloat16* src = v + ((size_t)b * Hkv + hv) * D;
-        __nv_bfloat16* dst = vc + (((size_t)b * Hkv + hv) * max_len + pos) * D;
+        __nv_bfloat16* dst = vc + (((size_t)b * Hkv + hv) * max_len + row) * D;
         dst[i] = src[i];
         dst[i + half] = src[i + half];
     }
@@ -217,11 +219,11 @@ cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, cudaStream
 }  // namespace
 
 int launch_rope_cache(void* q, const void* k, const void* v, const int64_t* pos, const float* inv_freq, void* kc, void* vc,
-                      int B, int Hq, int Hkv, int D, int64_t max_len, cudaStream_t st) {
-    if (B < 1 || Hq < 1 || Hkv < 1 || D < 2 || (D & 1) || D / 2 > 1024 || max_len < 1) return GBXQ_ESHAPE;
+                      int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep, cudaStream_t st) {
+    if (B < 1 || Hq < 1 || Hkv < 1 || D < 2 || (D & 1) || D / 2 > 1024 || max_len < 1 || keep >= max_len) return GBXQ_ESHAPE;
     const cudaError_t e = launch_pdl(rope_cache_kernel, dim3(Hq + 2 * Hkv, B), dim3(D / 2), st,
         reinterpret_cast<__nv_bfloat16*>(q), reinterpret_cast<const __nv_bfloat16*>(k), reinterpret_cast<const __nv_bfloat16*>(v),
-        pos, inv_freq, reinterpret_cast<__nv_bfloat16*>(kc), reinterpret_cast<__nv_bfloat16*>(vc), Hq, Hkv, D, max_len);
+        pos, inv_freq, reinterpret_cast<__nv_bfloat16*>(kc), reinterpret_cast<__nv_bfloat16*>(vc), Hq, Hkv, D, max_len, keep);
     count_launch();
     return check_cuda(e);
 }

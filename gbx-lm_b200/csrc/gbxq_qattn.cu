@@ -6,6 +6,7 @@
 //                          triple at row *pos -- the quantized counterpart of gbxq_rope_cache.  The rotated k is rounded
 //                          to bf16 first and the groups go through the recipe of gbxq_quantize (gbxq_affine.cuh), so the
 //                          triples are bit-identical to gbxq_rope_cache into a bf16 row followed by gbxq_quantize_rows.
+//                          On a rotating cache the row is the ring slot of the position (kv_cache_row).
 //   qattn_partial          flash-decoding over the codes: one CTA per (key chunk of 256, kv head, batch) serves all
 //                          Hq/Hkv query heads of the group, so K and V are read from HBM once.  The chunk's K and V codes
 //                          (contiguous: the cache is position-major) are brought in with cp.async; scores use the
@@ -65,7 +66,8 @@ __device__ __forceinline__ void copy_async(void* dst, const void* src, uint32_t 
 
 // ------------------------------------------------------------------------------------------ RoPE + quantized cache write
 // grid (Hq + 2 Hkv, B), one warp per row of D; lane owns the D/32 consecutive elements lane*EPL ...  Head h < Hq: q
-// rotated in place; Hq <= h < Hq+Hkv: k rotated, rounded to bf16 and quantized into row *pos; else v quantized.
+// rotated in place; Hq <= h < Hq+Hkv: k rotated, rounded to bf16 and quantized into row kv_cache_row(*pos); else v
+// quantized.
 template <int D, int BITS>
 __global__ void __launch_bounds__(32) rope_cache_q_kernel(__nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ k,
                                                           const __nv_bfloat16* __restrict__ v, const int64_t* __restrict__ pos_p,
@@ -73,14 +75,15 @@ __global__ void __launch_bounds__(32) rope_cache_q_kernel(__nv_bfloat16* __restr
                                                           __nv_bfloat16* __restrict__ ks, __nv_bfloat16* __restrict__ kb,
                                                           uint32_t* __restrict__ vq, __nv_bfloat16* __restrict__ vs,
                                                           __nv_bfloat16* __restrict__ vb, int Hq, int Hkv, int64_t max_len,
-                                                          int gs) {
+                                                          int64_t keep, int gs) {
     constexpr int EPL = D / 32, HALF = D / 2, W = D * BITS / 32;
     __shared__ uint32_t codes_s[D];
     __shared__ __align__(8) uint8_t bytes_s[D * BITS / 8 + 8];
     const int h = blockIdx.x, b = blockIdx.y, lane = threadIdx.x;
     pdl_wait_then_trigger();
-    const int64_t pos = *pos_p;
-    if (pos < 0 || pos >= max_len) return;  // never write outside the cache
+    const int64_t pos = *pos_p;  // the RoPE angle is the absolute position's; k / v go to its cache row
+    const int64_t slot = kv_cache_row(pos, max_len, keep);
+    if (slot < 0) return;  // never write outside the cache
     float val[EPL];
     int hh;  // kv head of a k / v row
     if (h < Hq + Hkv) {
@@ -127,7 +130,7 @@ __global__ void __launch_bounds__(32) rope_cache_q_kernel(__nv_bfloat16* __restr
     const AffineGroup grp = affine_group<BITS>(mx, mn);
 #pragma unroll
     for (int e = 0; e < EPL; e++) codes_s[lane * EPL + e] = affine_code<BITS>(val[e], grp);
-    const size_t row = ((size_t)b * Hkv + hh) * (size_t)max_len + (size_t)pos;
+    const size_t row = ((size_t)b * Hkv + hh) * (size_t)max_len + (size_t)slot;
     const int ng = D / gs;
     if (lane % seg == 0) {
         cs[row * ng + lane / seg] = tobf(grp.scale);
@@ -442,7 +445,7 @@ int launch_rope_q(const QCacheWrite& a, cudaStream_t st) {
         reinterpret_cast<__nv_bfloat16*>(a.q), reinterpret_cast<const __nv_bfloat16*>(a.k),
         reinterpret_cast<const __nv_bfloat16*>(a.v), a.pos, a.inv_freq, a.kq, reinterpret_cast<__nv_bfloat16*>(a.ks),
         reinterpret_cast<__nv_bfloat16*>(a.kb), a.vq, reinterpret_cast<__nv_bfloat16*>(a.vs),
-        reinterpret_cast<__nv_bfloat16*>(a.vb), a.Hq, a.Hkv, a.max_len, a.gs);
+        reinterpret_cast<__nv_bfloat16*>(a.vb), a.Hq, a.Hkv, a.max_len, a.keep, a.gs);
     count_launch();
     return check_cuda(e);
 }
@@ -504,6 +507,7 @@ int qattn_bits(const QAttn& a, cudaStream_t st) {
 int launch_rope_cache_quantized(const QCacheWrite& a, cudaStream_t st) {
     const int rc = check_common(a.B, a.Hq, a.Hkv, a.D, a.max_len, a.bits, a.gs);
     if (rc != GBXQ_OK) return rc;
+    if (a.keep >= a.max_len) return GBXQ_ESHAPE;
     if (!a.q || !a.k || !a.v || !a.pos || !a.inv_freq || !a.kq || !a.ks || !a.kb || !a.vq || !a.vs || !a.vb) return GBXQ_ENULL;
     if (((uintptr_t)a.kq | (uintptr_t)a.vq) & 3) return GBXQ_EALIGN;
     return a.D == 64 ? rope_q_bits<64>(a, st) : rope_q_bits<128>(a, st);

@@ -513,19 +513,36 @@ def _bf16c(*ts):
             raise ValueError("decode glue ops take contiguous CUDA bf16 tensors")
 
 
+def _check_keep(keep: Optional[int], max_len: int, where: str) -> Optional[int]:
+    """The sink count of a rotating cache of window max_len: None (a flat cache) or an int in [0, max_len)."""
+    if keep is None:
+        return None
+    if isinstance(keep, bool) or not isinstance(keep, int) or not 0 <= keep < max_len:
+        raise ValueError(f"{where}: keep must be an int in [0, {max_len}) (the cache's window), got {keep!r}")
+    return keep
+
+
 def rope_cache(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, position: torch.Tensor, inv_freq: torch.Tensor,
-               k_cache: torch.Tensor, v_cache: torch.Tensor) -> torch.Tensor:
+               k_cache: torch.Tensor, v_cache: torch.Tensor, keep: Optional[int] = None) -> torch.Tensor:
     """gbxq_rope_cache: q [B,Hq,D] rotated IN PLACE (returned), k rotated and v copied into the caches [B,Hkv,max_len,D] at
-    `position` (int64 device tensor [1]).  Replaces RoPE + cache.update of a decode step (gbx_lm/models/qllama.py:83-88)."""
+    `position` (int64 device tensor [1]).  Replaces RoPE + cache.update of a decode step (gbx_lm/models/qllama.py:83-88).
+    keep = an int: the caches are a rotating window of max_len rows with `keep` sinks, and k / v go to row
+    ring_slot(position) (gbxq_rope_cache_ring; cache.ring_slot)."""
     _bf16c(q, k, v, k_cache, v_cache)
     b, hq, d = q.shape
     hkv, max_len = k_cache.shape[1], k_cache.shape[2]
     if position.dtype != torch.int64 or inv_freq.dtype != torch.float32 or inv_freq.numel() != d // 2:
         raise ValueError("rope_cache: position int64 [1], inv_freq float32 [D/2]")
+    keep = _check_keep(keep, max_len, "rope_cache")
+    args = (q.data_ptr(), k.data_ptr(), v.data_ptr(), position.data_ptr(), inv_freq.data_ptr(), k_cache.data_ptr(),
+            v_cache.data_ptr(), b, hq, hkv, d, max_len)
+    lib = _lib.get()
     with torch.cuda.device(q.device):
-        rc = _lib.get().gbxq_rope_cache(q.data_ptr(), k.data_ptr(), v.data_ptr(), position.data_ptr(), inv_freq.data_ptr(),
-                                        k_cache.data_ptr(), v_cache.data_ptr(), b, hq, hkv, d, max_len, _stream())
-    _lib.check(rc, "gbxq_rope_cache")
+        if keep is None:
+            rc, name = lib.gbxq_rope_cache(*args, _stream()), "gbxq_rope_cache"
+        else:
+            rc, name = lib.gbxq_rope_cache_ring(*args, keep, _stream()), "gbxq_rope_cache_ring"
+    _lib.check(rc, name)
     return q
 
 
@@ -577,11 +594,12 @@ def _check_qcache(q: torch.Tensor, k_cache3, v_cache3, group_size: int, bits: in
 
 
 def rope_cache_quantized(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, position: torch.Tensor, inv_freq: torch.Tensor,
-                         k_cache3, v_cache3, group_size: int, bits: int) -> torch.Tensor:
+                         k_cache3, v_cache3, group_size: int, bits: int, keep: Optional[int] = None) -> torch.Tensor:
     """gbxq_rope_cache_quantized: q [B,Hq,D] rotated IN PLACE (returned); k rotated and v copied, each quantized into row
     `position` (int64 device tensor [1]) of its (codes, scales, biases) triple -- bit-identical to `rope_cache` into a bf16
     row followed by `quantize_into` of that row.  The quantized counterpart of `rope_cache` (RoPE +
-    QuantizedKVCache.update_and_fetch, gbx_lm/models/cache.py:172-185)."""
+    QuantizedKVCache.update_and_fetch, gbx_lm/models/cache.py:172-185).  keep = an int: row ring_slot(position) of a
+    rotating cache, as `rope_cache` (gbxq_rope_cache_quantized_ring)."""
     group_size, bits = int(group_size), int(bits)
     b, hq, hkv, d, max_len = _check_qcache(q, k_cache3, v_cache3, group_size, bits)
     _bf16c(k, v)
@@ -590,12 +608,17 @@ def rope_cache_quantized(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, posi
     if (position.dtype != torch.int64 or position.device != q.device or inv_freq.dtype != torch.float32
             or inv_freq.numel() != d // 2 or inv_freq.device != q.device):
         raise ValueError("rope_cache_quantized: position int64 [1], inv_freq float32 [D/2], on the device of q")
+    keep = _check_keep(keep, max_len, "rope_cache_quantized")
+    args = (q.data_ptr(), k.data_ptr(), v.data_ptr(), position.data_ptr(), inv_freq.data_ptr(),
+            *[t.data_ptr() for t in k_cache3], *[t.data_ptr() for t in v_cache3], b, hq, hkv, d, max_len)
+    lib = _lib.get()
     with torch.cuda.device(q.device):
-        rc = _lib.get().gbxq_rope_cache_quantized(
-            q.data_ptr(), k.data_ptr(), v.data_ptr(), position.data_ptr(), inv_freq.data_ptr(),
-            *[t.data_ptr() for t in k_cache3], *[t.data_ptr() for t in v_cache3], b, hq, hkv, d, max_len, bits, group_size,
-            _stream())
-    _lib.check(rc, "gbxq_rope_cache_quantized")
+        if keep is None:
+            rc, name = lib.gbxq_rope_cache_quantized(*args, bits, group_size, _stream()), "gbxq_rope_cache_quantized"
+        else:
+            rc = lib.gbxq_rope_cache_quantized_ring(*args, keep, bits, group_size, _stream())
+            name = "gbxq_rope_cache_quantized_ring"
+    _lib.check(rc, name)
     return q
 
 

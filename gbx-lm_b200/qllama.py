@@ -24,7 +24,7 @@ import torch.nn.functional as F
 from torch import nn
 
 from . import ops
-from .cache import StaticKVCache, StaticQuantizedKVCache
+from .cache import StaticKVCache, StaticQuantizedKVCache, StaticRotatingKVCache
 from .quantized_linear import QuantizedLinear
 from .switch_layers import quantized_scaled_dot_product_attention
 from .tp import TPContext
@@ -117,11 +117,15 @@ class RoPE(nn.Module):
         return out.to(x.dtype)
 
 
-def make_prompt_cache(model, batch: int = 1, max_len: int = 4096) -> List[StaticKVCache]:
+def make_prompt_cache(model, batch: int = 1, max_len: int = 4096, keep: Optional[int] = None) -> List[StaticKVCache]:
+    """One static bf16 cache per layer: flat caches of max_len positions, or with `keep` an int, rotating caches of
+    window max_len with `keep` sinks (the reference's RotatingKVCache)."""
     a = model.args
     hd = a.head_dim or a.hidden_size // a.num_attention_heads
     dev = model.model.embed_tokens.weight.device
     n_kv = a.num_key_value_heads // model.tp.world
+    if keep is not None:
+        return [StaticRotatingKVCache(batch, n_kv, max_len, hd, dev, keep) for _ in range(a.num_hidden_layers)]
     return [StaticKVCache(batch, n_kv, max_len, hd, dev) for _ in range(a.num_hidden_layers)]
 
 
@@ -160,20 +164,29 @@ class Attention(nn.Module):  # gbx_lm/models/qllama.py:39-96
             # the quantized cache the attention is split-K on the codes (+ its combine launch)
             qh = q.view(B, self.n_heads, self.head_dim)
             kh, vh = k.view(B, self.n_kv_heads, self.head_dim), v.view(B, self.n_kv_heads, self.head_dim)
+            # (a rotating cache: the row is the position's ring slot, and the attention reads the whole window)
             if quantized:
                 gs, bits = cache.group_size, cache.bits
-                ops.rope_cache_quantized(qh, kh, vh, positions, self.rope.inv_freq, cache.keys, cache.values, gs, bits)
+                ops.rope_cache_quantized(qh, kh, vh, positions, self.rope.inv_freq, cache.keys, cache.values, gs, bits,
+                                         keep=cache.keep)
                 out = ops.decode_attention_quantized(qh, cache.keys, cache.values, positions, self.scale, gs, bits,
                                                      attend_len)
             else:
-                ops.rope_cache(qh, kh, vh, positions, self.rope.inv_freq, cache.keys, cache.values)
+                ops.rope_cache(qh, kh, vh, positions, self.rope.inv_freq, cache.keys, cache.values, keep=cache.keep)
                 out = ops.decode_attention(qh, cache.keys, cache.values, positions, self.scale, attend_len)
             return self.tp.row_parallel(self.o_proj, out.view(B, 1, -1))
         q = self.rope(q.view(B, L, self.n_heads, -1).transpose(1, 2), positions)
         k = self.rope(k.view(B, L, self.n_kv_heads, -1).transpose(1, 2), positions)
         v = v.view(B, L, self.n_kv_heads, -1).transpose(1, 2)
+        # a rotating cache that this call takes past its window: the positions attend the ring's rows and the call's own
+        # keys under the window rule, and only then are the positions that survive the call stored (prefill glue, host
+        # offsets: not graph-capturable).  Until then a rotating cache is written and read as the flat cache is.
+        ring = cache is not None and cache.keep is not None and cache.wraps()
         if cache is None:
             T, keys, values = L, k, v
+        elif ring:
+            keys, values, key_positions = cache.window_with(k, v, cache.offset - L)
+            T = key_positions.numel()
         elif quantized:
             # the rows are written at the HOST offset (Model.forward has already advanced it past these L positions), so
             # this path is not graph-capturable
@@ -184,8 +197,10 @@ class Attention(nn.Module):  # gbx_lm/models/qllama.py:39-96
             cache.update(k, v, positions)
             T = attend_len if attend_len is not None else cache.max_len
             keys, values = cache.keys[:, :, :T], cache.values[:, :, :T]
-        # causal over absolute positions: key j visible to query at position p iff j <= p
-        visible = torch.arange(T, device=x.device)[None, :] <= positions[:, None]
+        if ring:
+            visible = cache.visible(key_positions, positions)
+        else:  # causal over absolute positions: key j visible to query at position p iff j <= p
+            visible = torch.arange(T, device=x.device)[None, :] <= positions[:, None]
         if quantized:
             # the reference's attention on the codes (gbx_lm/models/base.py:65-98), with its additive mask
             mask = torch.zeros((L, T), dtype=q.dtype, device=x.device).masked_fill_(~visible, float("-inf"))
@@ -193,6 +208,8 @@ class Attention(nn.Module):  # gbx_lm/models/qllama.py:39-96
         else:
             out = F.scaled_dot_product_attention(q, keys, values, attn_mask=visible[None, None], scale=self.scale,
                                                  enable_gqa=self.n_heads != self.n_kv_heads)
+        if ring:
+            cache.store(keys, values, cache.offset - L, L)
         out = out.transpose(1, 2).reshape(B, L, -1)
         return self.tp.row_parallel(self.o_proj, out)
 
@@ -278,9 +295,9 @@ class Model(nn.Module):  # gbx_lm/models/qllama.py:177-209
             off = cache[0].offset if cache is not None else 0
             positions = torch.arange(off, off + L, device=inputs.device)
             if cache is not None:
-                attend_len = off + L
                 for c in cache:
                     c.offset = off + L
+                attend_len = cache[0].attend_len  # off + L; at most the window on a rotating cache
         out = self.model(inputs, positions, cache, attend_len)
         # vocabulary projection (qllama.py:194-198): decode-sized inputs go through the streaming bf16 GEMV
         # (gbxq_head_gemv), prefill through the dense matmul

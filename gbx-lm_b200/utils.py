@@ -24,7 +24,7 @@ import torch
 from torch import nn
 
 from . import qllama, qqwen2
-from .cache import StaticKVCache, StaticQuantizedKVCache, maybe_quantize_kv_cache
+from .cache import DEFAULT_KV_KEEP, StaticKVCache, StaticQuantizedKVCache, maybe_quantize_kv_cache
 from .quantized_linear import QuantizedLinear
 from .tp import TPContext, proj_kind, shard_tensor
 
@@ -312,10 +312,11 @@ class DecodeGraph:
     7*L QuantizedLinear launches plus the glue -- replays as one submission (SURVEY.md 7.2 item 1)."""
 
     def __init__(self, model, cache, batch: int = 1):
-        # the unfused quantized path writes at the HOST offset, which a replay cannot advance
-        if any(isinstance(c, StaticQuantizedKVCache) and not layer.self_attn.takes_fused_decode(c)
+        # the unfused quantized and rotating paths write at the HOST offset, which a replay cannot advance
+        if any((isinstance(c, StaticQuantizedKVCache) or c.keep is not None) and not layer.self_attn.takes_fused_decode(c)
                for layer, c in zip(model.layers, cache)):
-            raise ValueError("DecodeGraph: a quantized KV cache is graph-capturable only on the fused decode path")
+            raise ValueError("DecodeGraph: a quantized or rotating KV cache is graph-capturable only on the fused decode "
+                             "path")
         self.model, self.cache = model, cache
         dev = cache[0].device
         self.tok = torch.zeros((batch, 1), dtype=torch.long, device=dev)
@@ -372,12 +373,20 @@ def _kv_quantizer(cache: list, kv_bits: Optional[int], kv_group_size: int, quant
 
 
 def _decode_graph(model, cache, tok, position: int, device_loop: int = 0) -> Optional[DecodeGraph]:
-    """A captured decode step, or None where the cache cannot be captured (a quantized cache off the fused path)."""
+    """A captured decode step, or None where the cache cannot be captured (a quantized or rotating cache off the fused
+    path)."""
     try:
         dg = DecodeGraph(model, cache)
     except ValueError:
         return None
     return dg.capture(tok, position, device_loop=device_loop)
+
+
+def _prompt_cache(model, run_len: int, max_kv_size: Optional[int]) -> list:
+    """Flat caches for a run of `run_len` positions, or rotating caches of window max_kv_size."""
+    if max_kv_size is None:
+        return qllama.make_prompt_cache(model, 1, run_len)
+    return qllama.make_prompt_cache(model, 1, max_kv_size, keep=DEFAULT_KV_KEEP)
 
 
 def prefill(model, prompt: torch.Tensor, cache: list, prefill_step_size: int = 2048, kv_bits: Optional[int] = None,
@@ -416,11 +425,12 @@ def generate_step(
     kv_bits / kv_group_size / quantized_kv_start: the reference's quantized KV cache -- after every model call, prefill
     chunks included, the caches are converted to `kv_bits`-bit group-quantized ones once their offset exceeds
     `quantized_kv_start` (maybe_quantize_kv_cache); kv_bits=None keeps the bf16 cache.  A decode graph captured before the
-    conversion is captured again once, after it."""
+    conversion is captured again once, after it.
+    max_kv_size = W: rotating caches of W positions with DEFAULT_KV_KEEP sinks (the reference's RotatingKVCache), so the
+    memory and the attention of every step stay bounded however long the run; they compose with kv_bits."""
     y = prompt.reshape(-1).to(next(model.parameters()).device)
     sampler = sampler or (lambda lp: torch.argmax(lp, dim=-1))
-    max_len = max_kv_size or (y.numel() + max_tokens + 1)
-    cache = prompt_cache if prompt_cache is not None else qllama.make_prompt_cache(model, 1, max_len)
+    cache = prompt_cache if prompt_cache is not None else _prompt_cache(model, y.numel() + max_tokens + 1, max_kv_size)
     kv = dict(kv_bits=kv_bits, kv_group_size=kv_group_size, quantized_kv_start=quantized_kv_start)
     quantize_cache = _kv_quantizer(cache, **kv)
 
@@ -452,17 +462,18 @@ def generate_step(
 
 
 def generate_tokens_device(model, prompt: torch.Tensor, max_tokens: int = 128, prefill_step_size: int = 2048,
-                           kv_bits: Optional[int] = None, kv_group_size: int = 64,
-                           quantized_kv_start: int = 0) -> Tuple[List[int], dict]:
+                           kv_bits: Optional[int] = None, kv_group_size: int = 64, quantized_kv_start: int = 0,
+                           max_kv_size: Optional[int] = None) -> Tuple[List[int], dict]:
     """Greedy generation with the sampler inside the captured decode step (DecodeGraph device_loop): the same tokens as
     `generate_tokens` (argmax of the log-probabilities = argmax of the logits), but the host only enqueues replays and
     reads the tokens once at the end -- the per-token host round trip of utils.py:299-337 (~0.3-0.6 ms on a B200 box)
     is gone.  Same timing definitions as generate_tokens.  kv_bits / kv_group_size / quantized_kv_start as in
     generate_step: when the conversion falls inside the decode, the graph replays up to that step, the caches are
-    converted, and a graph of the quantized step replays the rest."""
+    converted, and a graph of the quantized step replays the rest.  max_kv_size as in generate_step: the captured step
+    writes the ring slot of its device-side position, so the replays wrap without the host."""
     y = prompt.reshape(-1).to(next(model.parameters()).device)
     n_prompt = y.numel()
-    cache = qllama.make_prompt_cache(model, 1, n_prompt + max_tokens + 1)
+    cache = _prompt_cache(model, n_prompt + max_tokens + 1, max_kv_size)
     kv = dict(kv_bits=kv_bits, kv_group_size=kv_group_size, quantized_kv_start=quantized_kv_start)
     t0 = time.perf_counter()
     tok = torch.argmax(prefill(model, y, cache, prefill_step_size, **kv).float(), dim=-1)

@@ -257,6 +257,25 @@ int gbxq_decode_attention(const void* q, const void* k_cache, const void* v_cach
                           int B, int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale, void* stream);
 int gbxq_add_rmsnorm(const void* x, const void* r, const void* w, float eps, void* h_out, void* y_out, int64_t rows,
                      int H, void* stream);
+
+/*
+ * The cache writes of a ROTATING KV cache (the reference's RotatingKVCache, gbx_lm/models/cache.py:280-420): window W =
+ * max_len rows, of which the first `keep` are attention sinks, 0 <= keep < max_len (else GBXQ_ESHAPE).  Absolute
+ * position p is stored in row
+ *     ring_slot(p) = p                                   if p < W
+ *                  = keep + (p - keep) mod (W - keep)    otherwise
+ * gbxq_rope_cache_ring / gbxq_rope_cache_quantized_ring are gbxq_rope_cache / gbxq_rope_cache_quantized with k and v
+ * written to row ring_slot(*pos) instead of row *pos: the RoPE angle is the absolute *pos, q is rotated in place, and
+ * nothing else is written.  For *pos < max_len they are bitwise the flat entry points.  The slot is computed on the
+ * device, so a captured decode step wraps without the host.
+ * No attention entry point of its own: gbxq_decode_attention and gbxq_decode_attention_quantized attend rows
+ * [0, min(*pos, attend_len-1)], and with max_len = W and attend_len = min(tokens so far, W) (a replayed graph: W) those
+ * rows are exactly the ring's contents -- the sinks and the last W - keep positions.  Softmax does not depend on the
+ * order of the rows, so the result is the windowed attention up to the order of summation.
+ */
+int gbxq_rope_cache_ring(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev,
+                         void* k_cache, void* v_cache, int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep,
+                         void* stream);
 int gbxq_silu_mul(const void* gate, const void* up, void* out, int64_t n, void* stream);
 
 /*
@@ -284,6 +303,11 @@ int gbxq_rope_cache_quantized(void* q, const void* k, const void* v, const int64
                               uint32_t* k_codes, void* k_scales, void* k_biases, uint32_t* v_codes, void* v_scales,
                               void* v_biases, int B, int Hq, int Hkv, int D, int64_t max_len, int bits, int group_size,
                               void* stream);
+/* gbxq_rope_cache_quantized writing row ring_slot(*pos) of a rotating cache (see gbxq_rope_cache_ring). */
+int gbxq_rope_cache_quantized_ring(void* q, const void* k, const void* v, const int64_t* pos_dev,
+                                   const float* inv_freq_dev, uint32_t* k_codes, void* k_scales, void* k_biases,
+                                   uint32_t* v_codes, void* v_scales, void* v_biases, int B, int Hq, int Hkv, int D,
+                                   int64_t max_len, int64_t keep, int bits, int group_size, void* stream);
 size_t gbxq_decode_attention_quantized_workspace_bytes(int B, int Hq, int Hkv, int D, int64_t attend_len);
 int gbxq_decode_attention_quantized(const void* q, const uint32_t* k_codes, const void* k_scales, const void* k_biases,
                                     const uint32_t* v_codes, const void* v_scales, const void* v_biases,

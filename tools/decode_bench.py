@@ -6,11 +6,17 @@ timed with the reference's own definitions (gbx_lm/utils.py:590-607).  Prints on
 
     python tools/decode_bench.py [--model llama-3.2-1b] [--strategy bpw-4.0] [--tokens 128] [--prompt 32]
                                  [--kv-bits none,8,4] [--kv-group-size 64] [--quantized-kv-start N]
+                                 [--max-kv-size none,W] [--graph-positions P1,P2,...]
 
 --kv-bits takes a comma-separated list (none = the bf16 cache); one JSON line per entry, from one model load.  With a
 width the caches are converted to the group-quantized cache after the model call that takes them past
 --quantized-kv-start (the reference's generate_step rule); a start one below the prompt length prefills on bf16 and
-converts once before the decode."""
+converts once before the decode.
+
+--max-kv-size takes a comma-separated list too (none = the flat cache, W = rotating caches of W positions with 4 sinks,
+`generate_step(max_kv_size=W)`); every (kv-bits, max-kv-size) pair is one JSON line.  --graph-positions times the
+captured step at each listed position as well (default: the prompt length); on a rotating cache every position past
+the window attends the same W keys."""
 import argparse
 import json
 import os
@@ -24,6 +30,7 @@ import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from gbx_lm_b200 import ops, utils  # noqa: E402
+from gbx_lm_b200.cache import DEFAULT_KV_KEEP  # noqa: E402
 from gbx_lm_b200 import workloads as W  # noqa: E402
 
 
@@ -37,6 +44,8 @@ def main():
     ap.add_argument("--kv-bits", default="none")
     ap.add_argument("--kv-group-size", type=int, default=64)
     ap.add_argument("--quantized-kv-start", type=int, default=0)
+    ap.add_argument("--max-kv-size", default="none")
+    ap.add_argument("--graph-positions", default="")
     args = ap.parse_args()
     dims = W.MODELS[args.model]
     strat = None if args.strategy == "uniform" else W.STRATEGIES[args.strategy](dims.layers)
@@ -52,16 +61,17 @@ def main():
     finally:
         shutil.rmtree(d, ignore_errors=True)
     prompt = torch.randint(0, dims.vocab, (args.prompt,), generator=torch.Generator().manual_seed(1))
-    for kv in args.kv_bits.split(","):
-        kv_bits = None if kv.strip().lower() == "none" else int(kv)
-        run(args, dims, strat, model, prompt, kv_bits, t_write, t_load)
+    none_or_int = lambda s: None if s.strip().lower() == "none" else int(s)
+    for size in args.max_kv_size.split(","):
+        for kv in args.kv_bits.split(","):
+            run(args, dims, strat, model, prompt, none_or_int(kv), none_or_int(size), t_write, t_load)
 
 
-def run(args, dims, strat, model, prompt, kv_bits, t_write, t_load):
-    from gbx_lm_b200 import qllama
+def run(args, dims, strat, model, prompt, kv_bits, max_kv_size, t_write, t_load):
     from gbx_lm_b200.cache import StaticQuantizedKVCache
 
-    kw = dict(kv_bits=kv_bits, kv_group_size=args.kv_group_size, quantized_kv_start=args.quantized_kv_start)
+    kw = dict(kv_bits=kv_bits, kv_group_size=args.kv_group_size, quantized_kv_start=args.quantized_kv_start,
+              max_kv_size=max_kv_size)
     best, toks0 = None, None
     for r in range(args.repeat):
         n0 = ops.launch_count()
@@ -77,21 +87,31 @@ def run(args, dims, strat, model, prompt, kv_bits, t_write, t_load):
     assert d_toks == toks0, "device-side greedy sampler diverged from the host-side one"
     # device time of the captured decode step alone (no sampling, no host sync between steps), on the cache the decode
     # runs on: converted after the prompt when kv_bits is set and the prompt is past quantized_kv_start
-    cache = qllama.make_prompt_cache(model, 1, args.prompt + args.tokens + 1)
-    utils.prefill(model, prompt.cuda(), cache, **kw)
+    # (and the prefill alone, device-synchronised, on that cache)
+    cache = utils._prompt_cache(model, args.prompt + args.tokens + 1, max_kv_size)
+    kv = {k: v for k, v in kw.items() if k != "max_kv_size"}
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    utils.prefill(model, prompt.cuda(), cache, **kv)
+    torch.cuda.synchronize()
+    prefill_ms = (time.perf_counter() - t0) * 1e3
     quantized = isinstance(cache[0], StaticQuantizedKVCache)
-    dg = utils.DecodeGraph(model, cache).capture(torch.tensor([1], device="cuda"), args.prompt)
-    for _ in range(5):
-        dg.graph.replay()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    torch.cuda.synchronize()
-    e0.record()
-    for _ in range(50):
-        dg.graph.replay()
-    e1.record()
-    torch.cuda.synchronize()
-    graph_ms = e0.elapsed_time(e1) / 50
-    del dg, cache
+    graph_ms = {}
+    for pos in [args.prompt] + [int(p) for p in args.graph_positions.split(",") if p]:
+        # the step's cost depends on the position (the keys it attends), not on the cache's contents
+        dg = utils.DecodeGraph(model, cache).capture(torch.tensor([1], device="cuda"), pos)
+        for _ in range(5):
+            dg.graph.replay()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        torch.cuda.synchronize()
+        e0.record()
+        for _ in range(50):
+            dg.graph.replay()
+        e1.record()
+        torch.cuda.synchronize()
+        graph_ms[pos] = round(e0.elapsed_time(e1) / 50, 4)
+        del dg
+    del cache
     plan = W.layer_plan(dims, strat, 4, 64)
     body = sum(W.qmm_bytes(1, n, k, b, g) for (_, _, n, k, b, g) in plan)
     head = dims.vocab * dims.hidden * 2
@@ -99,20 +119,24 @@ def run(args, dims, strat, model, prompt, kv_bits, t_write, t_load):
     row = hd * kv_bits // 8 + 2 * 2 * (hd // args.kv_group_size) if quantized else hd * 2
     kv_per_token = dims.layers * dims.kv_heads * 2 * row
     ctx = args.prompt + args.tokens // 2  # mean visible keys over the decode
+    if max_kv_size is not None:
+        ctx = min(ctx, max_kv_size)
     print(json.dumps({
         "tool": "decode_bench", "model": args.model, "strategy": args.strategy, "batch": 1, "prompt_tokens": args.prompt,
         "kv_bits": kv_bits, "kv_group_size": args.kv_group_size if kv_bits else None,
         "quantized_kv_start": args.quantized_kv_start if kv_bits else None, "decode_cache": "quantized" if quantized else "bf16",
+        "max_kv_size": max_kv_size, "kv_keep": DEFAULT_KV_KEEP if max_kv_size else None,
         "kv_bytes_per_token": kv_per_token, "kv_bytes_per_step_at_mean_context": kv_per_token * ctx,
         "generation_tokens": best["generation_tokens"], "generation_tps": round(best["generation_tps"], 1),
         "prompt_tps": round(best["prompt_tps"], 1), "ms_per_token": round(1e3 / best["generation_tps"], 4),
-        "generation_tps_device_sampler": round(d_stats["generation_tps"], 1), "graph_ms_per_step": round(graph_ms, 4), "gbxq_launches_per_generate": best["gbxq_launches"],
+        "generation_tps_device_sampler": round(d_stats["generation_tps"], 1), "graph_ms_per_step": graph_ms[args.prompt],
+        "graph_ms_at_position": graph_ms, "prefill_ms": round(prefill_ms, 2), "gbxq_launches_per_generate": best["gbxq_launches"],
         "device_tokens_equal_host_tokens": True,
         "qmm_bytes_per_token": body, "head_bytes_per_token": head,
         "hbm_gbs_body_plus_head": round((body + head) * best["generation_tps"] / 1e9, 1),
         "checkpoint_write_s": round(t_write, 1), "load_s": round(t_load, 1), "data": "synthetic (random-init, seed 0)",
         "gpu": torch.cuda.get_device_name(0),
-        "note": "whole decode step: quantized forwards + decode glue through libgbxq (GBXQ_FUSED_DECODE=0: torch glue), bf16 head via cuBLAS; generation_tps syncs with the host every token, generation_tps_device_sampler does not; graph_ms_per_step is the captured step at position prompt_tokens",
+        "note": "whole decode step: quantized forwards + decode glue through libgbxq (GBXQ_FUSED_DECODE=0: torch glue), bf16 head via cuBLAS; generation_tps syncs with the host every token, generation_tps_device_sampler does not; graph_ms_per_step is the captured step at position prompt_tokens; prefill_ms is utils.prefill of the prompt alone",
     }), flush=True)
 
 
