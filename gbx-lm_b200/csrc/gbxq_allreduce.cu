@@ -46,8 +46,8 @@ __global__ void __launch_bounds__(256) allreduce_oneshot_kernel(const T* in, T* 
     // the CTAs that are done), so that a CUDA graph can replay the call: every CTA reads it at entry, the last CTA to
     // finish advances it.  The launch is plain stream-ordered, so the next call sees the advanced value.
     uint32_t* local = peer_flags[rank] + world * GBXQ_AR_MAX_CTAS;
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    asm volatile("griddepcontrol.wait;" ::: "memory");  // `in` (and the device-resident sequence number) belong to earlier kernels
+    griddep_launch_dependents();
+    griddep_wait();  // `in` (and the device-resident sequence number) belong to earlier kernels
     const bool dev_seq = seq == 0u;
     if (dev_seq) seq = *reinterpret_cast<volatile uint32_t*>(local) + 1u;
     const int64_t half = (int64_t)(seq & 1u) * half_elems;
@@ -112,20 +112,8 @@ int launch_t(const void* in, void* out, int64_t count, void* const* peer_bufs, u
     int ctas = (int)((nvec + 255) / 256);
     if (ctas < 1) ctas = 1;
     if (ctas > GBXQ_AR_MAX_CTAS) ctas = GBXQ_AR_MAX_CTAS;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)ctas);
-    cfg.blockDim = dim3(256);
-    cfg.dynamicSmemBytes = 0;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = mmv_get_pdl_mode() > 0 ? 1 : 0;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, allreduce_oneshot_kernel<T, 8>, (const T*)in, (T*)out, count, peer_bufs,
-                                             peer_flags, capacity / 2, rank, world, seq);
-    count_launch();
-    return check_cuda(e);
+    return launch(allreduce_oneshot_kernel<T, 8>, dim3((unsigned)ctas), dim3(256), 0, st, true, (const T*)in, (T*)out, count,
+                  peer_bufs, peer_flags, capacity / 2, rank, world, seq);
 }
 
 }  // namespace

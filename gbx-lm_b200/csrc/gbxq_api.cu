@@ -3,7 +3,6 @@
 // gbx_lm/models/quantized_linear_gba.py:195-205 (quantized_matmul + bias) and
 // gbx_lm/tuner/lora.py:62-68 (dequantize).
 #include <atomic>
-#include <cstdlib>
 
 #include "gbxq_common.cuh"
 
@@ -12,6 +11,10 @@ namespace gbxq {
 thread_local cudaError_t g_last_cuda_error = cudaSuccess;
 static std::atomic<uint64_t> g_launches{0};
 void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
+
+// GBXQ_OPT_PDL: written by gbxq_set_option, read by every launching thread
+static std::atomic<int> g_pdl{2};
+int pdl_mode() { return g_pdl.load(std::memory_order_relaxed); }
 
 int device_sm_count() {
     // per-device cache (the library may be used from several devices of one process)
@@ -35,10 +38,7 @@ static constexpr int64_t kSkinnyMaxM = 16;  // 2 passes of 8 tokens; above that 
 // Measured on the 8B decode step (profiles/r02y_*): 8 rows 2.09 ms on the skinny kernel against 3.22 ms, 16 rows 3.9
 // against 3.28 ms, 32 rows 5.9 (shared-memory-operand GEMM) against 3.76 ms -> from 9 rows.
 static int ts_min_m() {
-    static const int v = [] {
-        const char* e = getenv("GBXQ_TS_MIN_M");
-        return e ? atoi(e) : 9;
-    }();
+    static const int v = env_int("GBXQ_TS_MIN_M", 9);
     return v;
 }
 
@@ -108,13 +108,13 @@ void gbxq_debug_stream_timeline(void* host_blob, int ncalls, unsigned long long*
 
 int gbxq_set_option(int key, int value) {
     if (key == GBXQ_OPT_PDL) {
-        mmv_set_pdl_mode(value);
+        g_pdl.store(value < 0 ? 0 : (value > 2 ? 2 : value), std::memory_order_relaxed);
         return GBXQ_OK;
     }
     return GBXQ_EUNSUPPORTED;
 }
 int gbxq_get_option(int key) {
-    if (key == GBXQ_OPT_PDL) return mmv_get_pdl_mode();
+    if (key == GBXQ_OPT_PDL) return pdl_mode();
     return GBXQ_EUNSUPPORTED;
 }
 

@@ -9,6 +9,7 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <stdlib.h>
 
 #include <atomic>
 
@@ -32,6 +33,17 @@ inline int check_cuda(cudaError_t e) {
     return GBXQ_OK;
 }
 
+// GBXQ_OPT_PDL (include/gbxq.h), set by gbxq_set_option: 0 plain launches; 1 PDL, every global read after
+// griddepcontrol.wait; 2 (default) PDL, frozen weights streamed before the wait.
+int pdl_mode();
+inline int pdl_early_weights() { return pdl_mode() >= 2 ? 1 : 0; }
+
+// an integer tuning knob from the environment, `dflt` when unset
+inline int env_int(const char* name, int dflt) {
+    const char* v = getenv(name);
+    return v ? atoi(v) : dflt;
+}
+
 // Per-DEVICE one-time configuration of a kernel (cudaFuncSetAttribute is a per-device property: a process that drives
 // several GPUs must set it on each).  `need()` is true until `done()` was called on the current device.
 struct DeviceOnce {
@@ -49,6 +61,40 @@ struct DeviceOnce {
         if (d >= 0) mask.fetch_or(uint64_t(1) << d, std::memory_order_relaxed);
     }
 };
+
+// Lets kernel Kern take up to `bytes` of dynamic shared memory, once per device.  The state is keyed on the kernel
+// itself: every instantiation of a kernel template is configured on its own.
+template <auto Kern>
+int allow_dynamic_smem(int bytes) {
+    static DeviceOnce configured;
+    if (configured.need()) {
+        const cudaError_t e = cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+        if (e != cudaSuccess) return check_cuda(e);
+        configured.done();
+    }
+    return GBXQ_OK;
+}
+
+// Every kernel launch of the library: enqueues kern(args...) on st with `smem` bytes of dynamic shared memory, counts
+// it and returns its status.  pdl: the launch carries the programmatic-stream-serialization attribute while
+// pdl_mode() > 0, so the kernel may start before the previous kernel of the stream has ended.  Such a kernel must
+// execute griddep_wait() before it reads what an earlier kernel wrote (or writes what one may still read).
+template <typename... KArgs, typename... Args>
+int launch(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, bool pdl, const Args&... args) {
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = pdl && pdl_mode() > 0 ? 1 : 0;
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
+    count_launch();
+    return check_cuda(e);
+}
 
 // ------------------------------------------------------------------ element types
 template <int DT> struct TypeOf;
@@ -102,6 +148,20 @@ __device__ __forceinline__ int64_t kv_cache_row(int64_t pos, int64_t max_len, in
 
 // ------------------------------------------------------------------ small PTX wrappers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+
+// Programmatic dependent launch (both are no-ops in a launch without the attribute): wait until the kernels before this
+// one in the stream have completed and their writes are visible; let the next kernel of the stream start launching.
+__device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void griddep_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+// The small decode-step kernels (gbxq_glue.cu, gbxq_qattn.cu): wait for the producers of the inputs FIRST, then let the
+// next kernel of the stream (a QuantizedLinear forward) become resident and stream its frozen weights while this one
+// runs.  The order matters: triggering before the wait would let the next matmul's CTAs fill the SMs while this grid is
+// not yet scheduled, and they would wait for it forever.
+__device__ __forceinline__ void pdl_wait_then_trigger() {
+    griddep_wait();
+    griddep_launch_dependents();
+}
 
 // d = a(bf16) * b(bf16) + c(f32): one FHFMA.BF16 on sm_100 (PTX ISA 8.6 mixed-precision fma).
 __device__ __forceinline__ float fma_bf16_f32(uint16_t a, uint16_t b, float c) {
@@ -269,8 +329,6 @@ int launch_head_gemv(const void* x, const void* w, void* y, int64_t M, int64_t V
 int launch_gather_qmm(const void* x, const uint32_t* w, const void* s, const void* b, const void* bias, const int32_t* lhs,
                       const int32_t* rhs, void* y, int64_t R, int64_t XB, int64_t E, int64_t M, int64_t N, int64_t K,
                       int transpose, int bits, int gs, int dtype, cudaStream_t st);
-void mmv_set_pdl_mode(int mode);
-int mmv_get_pdl_mode();
 bool gemm_supported(int64_t M, int64_t N, int64_t K, int bits, int gs, int dtype, const void* x, const void* w,
                     const void* y);
 int launch_gemm(const void* x, const uint32_t* w, const void* s, const void* b, const void* bias, void* y, int64_t M,

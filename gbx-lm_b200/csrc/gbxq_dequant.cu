@@ -51,9 +51,8 @@ static int launch_t(const uint32_t* w, const void* s, const void* b, void* out, 
     int64_t blocks = (total + threads - 1) / threads;
     const int64_t cap = (int64_t)device_sm_count() * 16;
     if (blocks > cap) blocks = cap;
-    dequant_kernel<BITS, T><<<(unsigned)blocks, threads, 0, st>>>(w, (const T*)s, (const T*)b, (T*)out, N, K, gs);
-    count_launch();
-    return check_cuda(cudaGetLastError());
+    return launch(dequant_kernel<BITS, T>, dim3((unsigned)blocks), dim3(threads), 0, st, false, w, (const T*)s, (const T*)b,
+                  (T*)out, N, K, gs);
 }
 
 template <int BITS>

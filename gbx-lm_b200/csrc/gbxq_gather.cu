@@ -156,18 +156,16 @@ int launch_t(const void* x, const uint32_t* w, const void* s, const void* b, con
         const int64_t cap = (int64_t)device_sm_count() * 8;
         if (blocks > cap) blocks = cap;
         dim3 grid((unsigned)blocks, (unsigned)mtiles, (unsigned)R);
-        gather_t_kernel<BITS, T, MT><<<grid, 256, 0, st>>>((const T*)x, w, (const T*)s, (const T*)b, (const T*)bias, lhs, rhs,
-                                                           (T*)y, XB, E, M, N, K, gs);
+        return launch(gather_t_kernel<BITS, T, MT>, grid, dim3(256), 0, st, false, (const T*)x, w, (const T*)s, (const T*)b,
+                      (const T*)bias, lhs, rhs, (T*)y, XB, E, M, N, K, gs);
     } else {
         const int64_t octs = (N + 7) / 8;
         int oct = 32;
         while (oct > 1 && oct / 2 >= octs) oct /= 2;  // narrow N (head_dim 64 / 128): more k slices per block
         dim3 grid((unsigned)((octs + oct - 1) / oct), (unsigned)mtiles, (unsigned)R);
-        gather_n_kernel<BITS, T, MT><<<grid, 256, 0, st>>>((const T*)x, w, (const T*)s, (const T*)b, lhs, rhs, (T*)y, XB, E, M,
-                                                           N, K, gs, oct);
+        return launch(gather_n_kernel<BITS, T, MT>, grid, dim3(256), 0, st, false, (const T*)x, w, (const T*)s, (const T*)b, lhs,
+                      rhs, (T*)y, XB, E, M, N, K, gs, oct);
     }
-    count_launch();
-    return check_cuda(cudaGetLastError());
 }
 
 template <int BITS>

@@ -490,10 +490,8 @@ bool encode_2d(CUtensorMap* tm, CUtensorMapDataType dt, const void* base, uint64
     const cuuint64_t gstride[1] = {pitch_bytes};
     const cuuint32_t box[2] = {box_inner, box_outer};
     const cuuint32_t estr[2] = {1, 1};
-    static const int promo = [] {  // GBXQ_TMA_L2PROMO = 0 / 64 / 128 / 256 (development switch; default 256 bytes)
-        const char* e = getenv("GBXQ_TMA_L2PROMO");
-        return e ? atoi(e) : 256;
-    }();
+    // GBXQ_TMA_L2PROMO = 0 / 64 / 128 / 256 (development switch; default 256 bytes)
+    static const int promo = env_int("GBXQ_TMA_L2PROMO", 256);
     const CUtensorMapL2promotion pr = promo == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE
                                       : (promo == 64 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
                                                      : (promo == 128 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B));
@@ -509,16 +507,10 @@ template <int BITS, int BN>
 int launch_inst(const Maps& mp, const GemmParams& p, cudaStream_t st) {
     constexpr size_t smem = Cfg<BITS, BN>::SMEM;
     static_assert(smem <= 227 * 1024, "shared memory budget");
-    static DeviceOnce configured;  // per device: the attribute is a per-device property
-    if (configured.need()) {
-        cudaError_t e = cudaFuncSetAttribute(gemm_kernel<BITS, BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return check_cuda(e);
-        configured.done();
-    }
+    const int rc = allow_dynamic_smem<gemm_kernel<BITS, BN>>((int)smem);
+    if (rc != GBXQ_OK) return rc;
     dim3 grid((unsigned)((p.N + kTileN - 1) / kTileN), (unsigned)((p.M + BN - 1) / BN), (unsigned)(p.splits > 1 ? p.splits : 1));
-    gemm_kernel<BITS, BN><<<grid, kThreads, smem, st>>>(mp.x, mp.w, mp.s, mp.b, p);
-    count_launch();
-    return check_cuda(cudaGetLastError());
+    return launch(gemm_kernel<BITS, BN>, grid, dim3(kThreads), smem, st, false, mp.x, mp.w, mp.s, mp.b, p);
 }
 
 template <int BITS>

@@ -149,9 +149,6 @@ template <int BITS, int BN> struct Cfg {
     static constexpr size_t SMEM = (size_t)XS * B_BYTES + (size_t)WS * W_SLOT + (size_t)SS * S_SLOT + NBAR * 8 + 16 + 1024;
 };
 
-__device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void griddep_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
 __device__ __forceinline__ unsigned long long gtime() {
     unsigned long long t;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
@@ -304,7 +301,7 @@ TS_KERNEL(TS_SIG) {
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    if (threadIdx.x == 0) griddep_launch();  // the next kernel of the stream may start its prologue when SMs free up
+    if (threadIdx.x == 0) griddep_launch_dependents();  // the next kernel of the stream may start its prologue when SMs free up
     if (threadIdx.x == 0) TS_STAMP(1);
 
     // The three single-issuer roles below run their loops with the WHOLE warp (uniform control flow, every lane polls
@@ -579,26 +576,11 @@ template <int BITS, int BN>
 int launch_inst(const Maps& mp, const TsParams& p, cudaStream_t st) {
     constexpr size_t smem = Cfg<BITS, BN>::SMEM;
     static_assert(smem <= 227 * 1024, "shared memory budget");
-    auto kern = TS_KERNEL<BITS, BN>;
-    static DeviceOnce configured;
-    if (configured.need()) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return check_cuda(e);
-        configured.done();
-    }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)((p.N + kTileN - 1) / kTileN), (unsigned)((p.M + BN - 1) / BN), (unsigned)(p.splits > 1 ? p.splits : 1));
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = mmv_get_pdl_mode() > 0 ? 1 : 0;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, mp.x, mp.w, mp.s, mp.b, p);
-    count_launch();
-    return check_cuda(e);
+    constexpr auto kern = TS_KERNEL<BITS, BN>;
+    const int rc = allow_dynamic_smem<kern>((int)smem);
+    if (rc != GBXQ_OK) return rc;
+    const dim3 grid((unsigned)((p.N + kTileN - 1) / kTileN), (unsigned)((p.M + BN - 1) / BN), (unsigned)(p.splits > 1 ? p.splits : 1));
+    return launch(kern, grid, dim3(kThreads), smem, st, true, mp.x, mp.w, mp.s, mp.b, p);
 }
 
 template <int BITS>
@@ -666,13 +648,10 @@ int TS_LAUNCH(const void* x, const uint32_t* w, const void* s, const void* b, co
     p.K = K;
     p.gs_shift = gs == 32 ? 5 : (gs == 64 ? 6 : 7);
     p.splits = 1;
-    p.early_w = mmv_get_pdl_mode() >= 2 ? 1 : 0;
+    p.early_w = pdl_early_weights();
     p.w_raw = reinterpret_cast<const uint8_t*>(w);
     p.row_bytes = K * bits / 8;
-    static const int rotate = [] {
-        const char* e = getenv("GBXQ_TS_ROTATE");
-        return e ? atoi(e) : 0;
-    }();
+    static const int rotate = env_int("GBXQ_TS_ROTATE", 0);
     p.rotate = rotate;
 #ifdef GBXQ_TS_DIRECT
     p.s_raw = reinterpret_cast<const uint16_t*>(s);
@@ -707,26 +686,11 @@ int TS_LAUNCH(const void* x, const uint32_t* w, const void* s, const void* b, co
 template <int BITS, int BN>
 int launch_inst(const TsMaps& mp, const TsParams& p, int tiles, cudaStream_t st) {
     constexpr size_t smem = Cfg<BITS, BN>::SMEM;
-    auto kern = TS_KERNEL<BITS, BN>;
-    static DeviceOnce configured;
-    if (configured.need()) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return check_cuda(e);
-        configured.done();
-    }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)tiles, (unsigned)((p.M + BN - 1) / BN), (unsigned)(p.splits > 1 ? p.splits : 1));
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = mmv_get_pdl_mode() > 0 ? 1 : 0;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, mp, p);
-    count_launch();
-    return check_cuda(e);
+    constexpr auto kern = TS_KERNEL<BITS, BN>;
+    const int rc = allow_dynamic_smem<kern>((int)smem);
+    if (rc != GBXQ_OK) return rc;
+    const dim3 grid((unsigned)tiles, (unsigned)((p.M + BN - 1) / BN), (unsigned)(p.splits > 1 ? p.splits : 1));
+    return launch(kern, grid, dim3(kThreads), smem, st, true, mp, p);
 }
 
 template <int BITS>
@@ -791,7 +755,7 @@ int launch_gemm_ts_grouped(const gbxq_segment* segs, int nseg, const void* x, in
     p.K = K;
     p.gs_shift = gs == 32 ? 5 : (gs == 64 ? 6 : 7);
     p.splits = 1;
-    p.early_w = mmv_get_pdl_mode() >= 2 ? 1 : 0;
+    p.early_w = pdl_early_weights();
     p.rotate = 0;
     p.dbg = nullptr;
     {

@@ -411,16 +411,10 @@ __global__ void __launch_bounds__(kThreads, 1) gemv_kernel(const GemvParams p) {
 
 template <int BITS, int NSB, int MT, int CPW, bool SB_TMA>
 int launch_inst(const GemvParams& p, size_t smem_bytes, int grid, cudaStream_t st) {
-    static DeviceOnce configured;  // per device: the attribute is a per-device property
-    if (configured.need()) {
-        cudaError_t e = cudaFuncSetAttribute(gemv_kernel<BITS, NSB, MT, CPW, SB_TMA>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        if (e != cudaSuccess) return check_cuda(e);
-        configured.done();
-    }
-    gemv_kernel<BITS, NSB, MT, CPW, SB_TMA><<<grid, kThreads, smem_bytes, st>>>(p);
-    count_launch();
-    return check_cuda(cudaGetLastError());
+    constexpr auto kern = gemv_kernel<BITS, NSB, MT, CPW, SB_TMA>;
+    const int rc = allow_dynamic_smem<kern>(227 * 1024);
+    if (rc != GBXQ_OK) return rc;
+    return launch(kern, dim3(grid), dim3(kThreads), smem_bytes, st, false, p);
 }
 
 template <int BITS> constexpr int nsb_for(int gs) { return Fmt<BITS>::CPU > gs ? Fmt<BITS>::CPU / gs : 1; }

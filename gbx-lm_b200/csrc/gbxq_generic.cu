@@ -73,10 +73,8 @@ static int launch_t(const void* x, const uint32_t* w, const void* s, const void*
     const int64_t mtiles = (M + MT - 1) / MT;
     if (mtiles > 65535) return GBXQ_EUNSUPPORTED;
     dim3 grid((unsigned)blocks, (unsigned)mtiles);
-    generic_kernel<BITS, T, MT><<<grid, threads, 0, st>>>((const T*)x, w, (const T*)s, (const T*)b, (const T*)bias,
-                                                          (T*)y, M, N, K, gs);
-    count_launch();
-    return check_cuda(cudaGetLastError());
+    return launch(generic_kernel<BITS, T, MT>, grid, dim3(threads), 0, st, false, (const T*)x, w, (const T*)s, (const T*)b,
+                  (const T*)bias, (T*)y, M, N, K, gs);
 }
 
 template <int BITS>

@@ -18,15 +18,6 @@ namespace gbxq {
 
 namespace {
 
-// Programmatic dependent launch, glue side: wait for the producers of the inputs FIRST, then let the next kernel of the
-// stream (a QuantizedLinear forward) become resident and stream its frozen weights while this small kernel runs.
-// The order matters: triggering before the wait would let the next matmul's CTAs fill the SMs while this grid is not
-// yet scheduled, and they would wait for it forever.
-__device__ __forceinline__ void pdl_wait_then_trigger() {
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-}
-
 __device__ __forceinline__ float bf(const __nv_bfloat16 v) { return __bfloat162float(v); }
 __device__ __forceinline__ __nv_bfloat16 tobf(float v) { return __float2bfloat16_rn(v); }
 
@@ -201,31 +192,14 @@ __global__ void __launch_bounds__(256) silu_mul_kernel(const __nv_bfloat16* __re
     reinterpret_cast<uint4*>(out)[i] = a;
 }
 
-template <typename... KArgs, typename... Args>
-cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, cudaStream_t st, Args... args) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = 0;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = mmv_get_pdl_mode() > 0 ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
-}
-
 }  // namespace
 
 int launch_rope_cache(void* q, const void* k, const void* v, const int64_t* pos, const float* inv_freq, void* kc, void* vc,
                       int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep, cudaStream_t st) {
     if (B < 1 || Hq < 1 || Hkv < 1 || D < 2 || (D & 1) || D / 2 > 1024 || max_len < 1 || keep >= max_len) return GBXQ_ESHAPE;
-    const cudaError_t e = launch_pdl(rope_cache_kernel, dim3(Hq + 2 * Hkv, B), dim3(D / 2), st,
+    return launch(rope_cache_kernel, dim3(Hq + 2 * Hkv, B), dim3(D / 2), 0, st, true,
         reinterpret_cast<__nv_bfloat16*>(q), reinterpret_cast<const __nv_bfloat16*>(k), reinterpret_cast<const __nv_bfloat16*>(v),
         pos, inv_freq, reinterpret_cast<__nv_bfloat16*>(kc), reinterpret_cast<__nv_bfloat16*>(vc), Hq, Hkv, D, max_len, keep);
-    count_launch();
-    return check_cuda(e);
 }
 
 int launch_decode_attention(const void* q, const void* kc, const void* vc, const int64_t* pos, void* out, int B, int Hq,
@@ -238,53 +212,31 @@ int launch_decode_attention(const void* q, const void* kc, const void* vc, const
     auto O = reinterpret_cast<__nv_bfloat16*>(out);
     if (attend_len > 49152) return GBXQ_EUNSUPPORTED;  // one float of shared memory per visible key
     const size_t smem = (size_t)attend_len * sizeof(float);
-    static DeviceOnce configured;  // per device: the attribute is a per-device property
-    if (configured.need()) {
-        cudaError_t ea = cudaFuncSetAttribute(decode_attention_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 49152 * 4);
-        if (ea == cudaSuccess)
-            ea = cudaFuncSetAttribute(decode_attention_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, 49152 * 4);
-        if (ea != cudaSuccess) return check_cuda(ea);
-        configured.done();
-    }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid;
-    cfg.blockDim = dim3(256);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = mmv_get_pdl_mode() > 0 ? 1 : 0;
-    cudaError_t e;
+    int rc = allow_dynamic_smem<decode_attention_kernel<64>>(49152 * 4);
+    if (rc == GBXQ_OK) rc = allow_dynamic_smem<decode_attention_kernel<128>>(49152 * 4);
+    if (rc != GBXQ_OK) return rc;
     switch (D) {
-        case 64: e = cudaLaunchKernelEx(&cfg, decode_attention_kernel<64>, Q, K, V, pos, O, Hq, Hkv, max_len, attend_len, scale); break;
-        case 128: e = cudaLaunchKernelEx(&cfg, decode_attention_kernel<128>, Q, K, V, pos, O, Hq, Hkv, max_len, attend_len, scale); break;
-        default: return GBXQ_EUNSUPPORTED;
+        case 64: return launch(decode_attention_kernel<64>, grid, dim3(256), smem, st, true, Q, K, V, pos, O, Hq, Hkv, max_len, attend_len, scale);
+        case 128: return launch(decode_attention_kernel<128>, grid, dim3(256), smem, st, true, Q, K, V, pos, O, Hq, Hkv, max_len, attend_len, scale);
     }
-    count_launch();
-    return check_cuda(e);
+    return GBXQ_EUNSUPPORTED;
 }
 
 int launch_add_rmsnorm(const void* x, const void* r, const void* w, float eps, void* h_out, void* y_out, int64_t rows, int H,
                        cudaStream_t st) {
     if (rows < 1 || H < 8 || H % 8) return GBXQ_ESHAPE;
-    const cudaError_t e = launch_pdl(add_rmsnorm_kernel, dim3((unsigned)rows), dim3(256), st,
+    return launch(add_rmsnorm_kernel, dim3((unsigned)rows), dim3(256), 0, st, true,
         reinterpret_cast<const __nv_bfloat16*>(x), reinterpret_cast<const __nv_bfloat16*>(r),
         reinterpret_cast<const __nv_bfloat16*>(w), eps, reinterpret_cast<__nv_bfloat16*>(h_out),
         reinterpret_cast<__nv_bfloat16*>(y_out), H);
-    count_launch();
-    return check_cuda(e);
 }
 
 int launch_silu_mul(const void* g, const void* u, void* out, int64_t n, cudaStream_t st) {
     if (n < 8 || n % 8) return GBXQ_ESHAPE;
     const int64_t nvec = n / 8;
-    const cudaError_t e = launch_pdl(silu_mul_kernel, dim3((unsigned)((nvec + 255) / 256)), dim3(256), st,
-                                     reinterpret_cast<const __nv_bfloat16*>(g), reinterpret_cast<const __nv_bfloat16*>(u),
-                                     reinterpret_cast<__nv_bfloat16*>(out), nvec);
-    count_launch();
-    return check_cuda(e);
+    return launch(silu_mul_kernel, dim3((unsigned)((nvec + 255) / 256)), dim3(256), 0, st, true,
+                  reinterpret_cast<const __nv_bfloat16*>(g), reinterpret_cast<const __nv_bfloat16*>(u),
+                  reinterpret_cast<__nv_bfloat16*>(out), nvec);
 }
 
 }  // namespace gbxq

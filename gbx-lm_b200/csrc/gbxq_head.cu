@@ -38,7 +38,7 @@ head_gemv_kernel(const __nv_bfloat16* __restrict__ x, const uint4* __restrict__ 
     // contiguous row ranges per warp (a warp streams one long contiguous piece of W)
     const int64_t r0 = gw * V / nwarps, r1 = (gw + 1) * V / nwarps;
 
-    if (threadIdx.x == 0) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    if (threadIdx.x == 0) griddep_launch_dependents();
     // first vectors of the first row: requested before the dependency wait (frozen parameters)
     uint4 wv[kInFlight];
     const uint4* row = w + (size_t)r0 * nvec;
@@ -47,7 +47,7 @@ head_gemv_kernel(const __nv_bfloat16* __restrict__ x, const uint4* __restrict__ 
         for (int u = 0; u < kInFlight; u++)
             if (u < per_lane) wv[u] = ldg_stream(row + lane + 32 * u);
     }
-    asm volatile("griddepcontrol.wait;" ::: "memory");
+    griddep_wait();
     for (int i = threadIdx.x; i < MT * nvec; i += kHeadThreads) {
         const int m = i / nvec;
         xs[i] = m < M ? reinterpret_cast<const uint4*>(x)[i] : make_uint4(0u, 0u, 0u, 0u);
@@ -99,29 +99,14 @@ head_gemv_kernel(const __nv_bfloat16* __restrict__ x, const uint4* __restrict__ 
 }
 
 template <int MT> int launch_mt(const void* x, const void* w, void* y, int M, int64_t V, int K, cudaStream_t st) {
-    auto kern = head_gemv_kernel<MT>;
+    constexpr auto kern = head_gemv_kernel<MT>;
     const size_t smem = (size_t)MT * K * 2;
-    static DeviceOnce configured;
-    if (configured.need()) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
-        if (e != cudaSuccess) return check_cuda(e);
-        configured.done();
-    }
+    const int rc = allow_dynamic_smem<kern>(100 * 1024);
+    if (rc != GBXQ_OK) return rc;
     if (smem > 100 * 1024) return GBXQ_EUNSUPPORTED;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)(2 * device_sm_count()));
-    cfg.blockDim = dim3(kHeadThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = mmv_get_pdl_mode() > 0 ? 1 : 0;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, reinterpret_cast<const __nv_bfloat16*>(x), reinterpret_cast<const uint4*>(w),
-                                             reinterpret_cast<__nv_bfloat16*>(y), M, V, K);
-    count_launch();
-    return check_cuda(e);
+    return launch(kern, dim3((unsigned)(2 * device_sm_count())), dim3(kHeadThreads), smem, st, true,
+                  reinterpret_cast<const __nv_bfloat16*>(x), reinterpret_cast<const uint4*>(w),
+                  reinterpret_cast<__nv_bfloat16*>(y), M, V, K);
 }
 
 }  // namespace

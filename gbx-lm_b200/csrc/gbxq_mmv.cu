@@ -60,8 +60,6 @@ __device__ __forceinline__ uint32_t hmul2_bf16(uint32_t a, uint32_t b) {
     asm("mul.rn.bf16x2 %0, %1, %2;" : "=r"(d) : "r"(a), "r"(b));
     return d;
 }
-__device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void griddep_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
 // ---- packing geometry.  A thread chunk = TB bytes = CQ codes = NP pairs; pair p = codes (pa, pb) that one LOP3
 //      extracts together (same position in the low / high half of a 32-bit word).
@@ -175,7 +173,7 @@ __global__ void __launch_bounds__(kThreads, kMinCtasPerSm) mmv_kernel(const MmvP
         fence_mbar_init();
     }
     __syncthreads();
-    if (threadIdx.x == 0) griddep_launch();  // the next kernel of the stream may become resident now
+    if (threadIdx.x == 0) griddep_launch_dependents();  // the next kernel of the stream may become resident now
 
     if (warp == kCW) {
         // ===================== producer warp: one elected lane drives the TMA engine =====================
@@ -464,11 +462,6 @@ struct Plan {
     size_t smem;
 };
 
-int env_int(const char* name, int dflt) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : dflt;
-}
-
 Plan make_plan(int64_t M, int64_t N, int64_t K, int bits, int gs) {
     Plan pl{};
     if (!(bits == 2 || bits == 4 || bits == 8) || M < 1 || M > 4 || N < 1) return pl;
@@ -515,30 +508,12 @@ Plan make_plan(int64_t M, int64_t N, int64_t K, int bits, int gs) {
     return pl;
 }
 
-int g_pdl_mode = 2;  // 0: plain launches; 1: PDL, wait before any global read; 2: PDL, weights streamed before the wait
-
 template <int BITS, int TB, int MP, int CPW, int R>
 int launch_inst(const MmvParams& p, const Plan& pl, cudaStream_t st) {
-    auto kern = mmv_kernel<BITS, TB, MP, CPW, R>;
-    static DeviceOnce configured;  // per device: the attribute is a per-device property
-    if (configured.need()) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024);
-        if (e != cudaSuccess) return check_cuda(e);
-        configured.done();
-    }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)pl.grid);
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = pl.smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = g_pdl_mode > 0 ? 1 : 0;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, p);
-    count_launch();
-    return check_cuda(e);
+    constexpr auto kern = mmv_kernel<BITS, TB, MP, CPW, R>;
+    const int rc = allow_dynamic_smem<kern>(110 * 1024);
+    if (rc != GBXQ_OK) return rc;
+    return launch(kern, dim3((unsigned)pl.grid), dim3(kThreads), pl.smem, st, true, p);
 }
 
 template <int BITS, int TB, int MP, int CPW>
@@ -586,9 +561,6 @@ int launch_tb(const MmvParams& p, const Plan& pl, cudaStream_t st) {
 
 }  // namespace
 
-void mmv_set_pdl_mode(int mode) { g_pdl_mode = mode < 0 ? 0 : (mode > 2 ? 2 : mode); }
-int mmv_get_pdl_mode() { return g_pdl_mode; }
-
 bool mmv_supported(int64_t M, int64_t N, int64_t K, int bits, int gs, int dtype, const void* x, const void* w,
                    const void* y) {
     if (dtype != GBXQ_BF16 || M < 1 || N < 1) return false;
@@ -622,7 +594,7 @@ int launch_mmv(const void* x, const uint32_t* w, const void* s, const void* b, c
     p.stages = pl.stages;
     p.slot_bytes = pl.slot_bytes;
     p.sb_off = pl.sb_off;
-    p.early_weights = g_pdl_mode >= 2 ? 1 : 0;
+    p.early_weights = pdl_early_weights();
     switch (bits) {
         case 2: return launch_tb<2>(p, pl, st);
         case 4: return launch_tb<4>(p, pl, st);

@@ -41,26 +41,10 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) mmv8_kernel(const Mmv8Para
 
 template <int BITS, int GS, int MT, int CPW, int R, bool PARTIAL>
 int launch_inst2(const Mmv8Params& p, const ArParams& ar, const Plan& pl, cudaStream_t st) {
-    auto kern = mmv8_kernel<BITS, GS, MT, CPW, R, PARTIAL>;
-    static DeviceOnce configured;  // per device: the attribute is a per-device property
-    if (configured.need()) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemCap);
-        if (e != cudaSuccess) return check_cuda(e);
-        configured.done();
-    }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)pl.grid);
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = pl.smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = mmv_get_pdl_mode() > 0 ? 1 : 0;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, p, ar);
-    count_launch();
-    return check_cuda(e);
+    constexpr auto kern = mmv8_kernel<BITS, GS, MT, CPW, R, PARTIAL>;
+    const int rc = allow_dynamic_smem<kern>(kSmemCap);
+    if (rc != GBXQ_OK) return rc;
+    return launch(kern, dim3((unsigned)pl.grid), dim3(kThreads), pl.smem, st, true, p, ar);
 }
 
 template <int BITS, int GS, int MT, int CPW, int R>
@@ -144,7 +128,7 @@ int launch_mmv8_ar(const void* x, const uint32_t* w, const void* s, const void* 
     if (((uintptr_t)s | (uintptr_t)b) & 15) return GBXQ_EUNSUPPORTED;
     const Plan pl = make_plan(M, N, K, bits, gs, 0, true, true);
     if (!pl.ok || pl.cpw * pl.mt > 8) return GBXQ_EUNSUPPORTED;
-    Mmv8Params p = make_params(pl, x, w, s, b, bias, y, M, N, K, bits, gs, mmv_get_pdl_mode() >= 2 ? 1 : 0);
+    Mmv8Params p = make_params(pl, x, w, s, b, bias, y, M, N, K, bits, gs, pdl_early_weights());
     ArParams ar{};
     if (comm != nullptr && comm->world > 1) {
         if (comm->world > 8 || comm->rank < 0 || comm->rank >= comm->world) return GBXQ_ESHAPE;

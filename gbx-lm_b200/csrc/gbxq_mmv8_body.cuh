@@ -44,8 +44,6 @@ __device__ __forceinline__ unsigned long long gtime() {
         if (p.dbg != nullptr && threadIdx.x == 0 && (p.dbg_all != 0 || blockIdx.x == 0))           \
             p.dbg[(p.dbg_all != 0 ? (size_t)blockIdx.x * 8 : 0) + (i)] = gtime();                  \
     } while (0)
-__device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void griddep_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
 template <int NWORD> __device__ __forceinline__ void lds_words(const uint8_t* addr, uint32_t (&w)[NWORD]) {
     if constexpr (NWORD == 1) {
@@ -254,7 +252,7 @@ __device__ __forceinline__ void mmv8_body(const Mmv8Params& p, const int bid, ui
             fence_mbar_init();
         }
         __syncthreads();
-        if (threadIdx.x == 0) griddep_launch();  // the next kernel of the stream may become resident now
+        if (threadIdx.x == 0) griddep_launch_dependents();  // the next kernel of the stream may become resident now
     } else {
         // every earlier call this one depends on must be complete on ALL CTAs before x is read or y overwritten
         if (threadIdx.x == 0 && sc->wait_cnt != nullptr && !sc->dead) {
@@ -689,11 +687,6 @@ struct Plan {
     uint32_t slot_bytes, sb_off;
     size_t smem;
 };
-
-inline int env_int(const char* name, int dflt) {
-    const char* v = getenv(name);
-    return v ? atoi(v) : dflt;
-}
 
 // grid_want > 0: the number of CTAs this layer may use (a segment of a grouped launch); 0: the whole device
 inline Plan make_plan(int64_t M, int64_t N, int64_t K, int bits, int gs, int grid_want = 0, bool allow_r16 = true,

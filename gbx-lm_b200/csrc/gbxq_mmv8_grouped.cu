@@ -59,26 +59,10 @@ __global__ void __launch_bounds__(kThreads, kMinCtas) mmv8_grouped_kernel(const 
 
 template <int GS, int MT, int CPW, int R, bool ODD>
 int launch_inst2(const GroupParams& gp, int grid, size_t smem, cudaStream_t st) {
-    auto kern = mmv8_grouped_kernel<GS, MT, CPW, R, ODD>;
-    static DeviceOnce configured;  // per device: the attribute is a per-device property
-    if (configured.need()) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemCap);
-        if (e != cudaSuccess) return check_cuda(e);
-        configured.done();
-    }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = mmv_get_pdl_mode() > 0 ? 1 : 0;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, gp);
-    count_launch();
-    return check_cuda(e);
+    constexpr auto kern = mmv8_grouped_kernel<GS, MT, CPW, R, ODD>;
+    const int rc = allow_dynamic_smem<kern>(kSmemCap);
+    if (rc != GBXQ_OK) return rc;
+    return launch(kern, dim3((unsigned)grid), dim3(kThreads), smem, st, true, gp);
 }
 
 template <int GS, int MT, int CPW, int R>
@@ -152,7 +136,7 @@ int launch_mmv8_grouped(const gbxq_segment* segs, int nseg, const void* x, int64
     Plan first{};
     size_t smem = 0;
     int grid = 0;
-    const int early = mmv_get_pdl_mode() >= 2 ? 1 : 0;
+    const int early = pdl_early_weights();
     for (int i = 0; i < nseg; i++) {
         const gbxq_segment& sg = segs[i];
         const Plan pl = make_plan(M, sg.N, K, sg.bits, gs, ctas[i]);

@@ -33,12 +33,6 @@ constexpr int kChunk = 256;    // keys per CTA of qattn_partial (fixed: the comb
 constexpr int kThreads = 256;
 constexpr float kLog2e = 1.4426950408889634f;
 
-// the same PDL discipline as the glue kernels (gbxq_glue.cu): wait for the producers, then let the next kernel in
-__device__ __forceinline__ void pdl_wait_then_trigger() {
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-}
-
 __device__ __forceinline__ float bf(const __nv_bfloat16 v) { return __bfloat162float(v); }
 __device__ __forceinline__ __nv_bfloat16 tobf(float v) { return __float2bfloat16_rn(v); }
 
@@ -414,21 +408,6 @@ __global__ void __launch_bounds__(D) qattn_combine_kernel(const float* __restric
     out[((size_t)b * Hq + h) * D + d] = tobf(nv > 0 && l > 0.f ? o / l : 0.f);
 }
 
-template <typename... KArgs, typename... Args>
-cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = mmv_get_pdl_mode() > 0 ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
-}
-
 int check_common(int B, int Hq, int Hkv, int D, int64_t max_len, int bits, int gs) {
     if (bits != 2 && bits != 3 && bits != 4 && bits != 6 && bits != 8) return GBXQ_EINVAL_BITS;
     if (gs != 32 && gs != 64 && gs != 128) return GBXQ_EINVAL_GROUP;
@@ -441,13 +420,11 @@ int64_t chunks_of(int64_t attend_len) { return (attend_len + kChunk - 1) / kChun
 
 template <int D, int BITS>
 int launch_rope_q(const QCacheWrite& a, cudaStream_t st) {
-    const cudaError_t e = launch_pdl(rope_cache_q_kernel<D, BITS>, dim3(a.Hq + 2 * a.Hkv, a.B), dim3(32), 0, st,
+    return launch(rope_cache_q_kernel<D, BITS>, dim3(a.Hq + 2 * a.Hkv, a.B), dim3(32), 0, st, true,
         reinterpret_cast<__nv_bfloat16*>(a.q), reinterpret_cast<const __nv_bfloat16*>(a.k),
         reinterpret_cast<const __nv_bfloat16*>(a.v), a.pos, a.inv_freq, a.kq, reinterpret_cast<__nv_bfloat16*>(a.ks),
         reinterpret_cast<__nv_bfloat16*>(a.kb), a.vq, reinterpret_cast<__nv_bfloat16*>(a.vs),
         reinterpret_cast<__nv_bfloat16*>(a.vb), a.Hq, a.Hkv, a.max_len, a.keep, a.gs);
-    count_launch();
-    return check_cuda(e);
 }
 
 template <int D>
@@ -464,26 +441,19 @@ int rope_q_bits(const QCacheWrite& a, cudaStream_t st) {
 template <int D, int BITS, int GMAX>
 int launch_qattn_t(const QAttn& a, cudaStream_t st) {
     using P = QAttnPlan<D, BITS, GMAX>;
-    auto kern = qattn_partial_kernel<D, BITS, GMAX>;
-    static DeviceOnce configured;  // per device: the attribute is a per-device property
-    if (configured.need()) {
-        const cudaError_t ea = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, P::BYTES);
-        if (ea != cudaSuccess) return check_cuda(ea);
-        configured.done();
-    }
+    constexpr auto kern = qattn_partial_kernel<D, BITS, GMAX>;
+    int rc = allow_dynamic_smem<kern>(P::BYTES);
+    if (rc != GBXQ_OK) return rc;
     const int nch = (int)chunks_of(a.attend_len);
     float* ws = reinterpret_cast<float*>(a.ws);
     const float qscale = a.scale * kLog2e;
-    cudaError_t e = launch_pdl(kern, dim3(nch, a.Hkv, a.B), dim3(kThreads), (size_t)P::BYTES, st,
+    rc = launch(kern, dim3(nch, a.Hkv, a.B), dim3(kThreads), (size_t)P::BYTES, st, true,
         reinterpret_cast<const __nv_bfloat16*>(a.q), a.kq, reinterpret_cast<const __nv_bfloat16*>(a.ks),
         reinterpret_cast<const __nv_bfloat16*>(a.kb), a.vq, reinterpret_cast<const __nv_bfloat16*>(a.vs),
         reinterpret_cast<const __nv_bfloat16*>(a.vb), a.pos, ws, a.Hq, a.Hkv, a.max_len, a.attend_len, nch, a.gs, qscale);
-    count_launch();
-    if (e != cudaSuccess) return check_cuda(e);
-    e = launch_pdl(qattn_combine_kernel<D>, dim3(a.Hq, a.B), dim3(D), 0, st, (const float*)ws, a.pos,
-                   reinterpret_cast<__nv_bfloat16*>(a.out), a.Hq, a.attend_len, nch);
-    count_launch();
-    return check_cuda(e);
+    if (rc != GBXQ_OK) return rc;
+    return launch(qattn_combine_kernel<D>, dim3(a.Hq, a.B), dim3(D), 0, st, true, (const float*)ws, a.pos,
+                  reinterpret_cast<__nv_bfloat16*>(a.out), a.Hq, a.attend_len, nch);
 }
 
 template <int D, int BITS>

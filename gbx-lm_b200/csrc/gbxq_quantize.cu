@@ -202,9 +202,8 @@ int launch_t(const void* w, uint32_t* q, void* s, void* b, int64_t total, int64_
     int64_t blocks = (nchunks + kWarps - 1) / kWarps;
     const int64_t cap = (int64_t)device_sm_count() * ctas_per_sm<BITS, GS, T>();  // one resident wave, grid-stride beyond
     if (blocks > cap) blocks = cap;
-    quantize_kernel<BITS, GS, T><<<(unsigned)blocks, kWarps * 32, 0, st>>>((const T*)w, q, (T*)s, (T*)b, total, K, map);
-    count_launch();
-    return check_cuda(cudaGetLastError());
+    return launch(quantize_kernel<BITS, GS, T>, dim3((unsigned)blocks), dim3(kWarps * 32), 0, st, false, (const T*)w, q, (T*)s,
+                  (T*)b, total, K, map);
 }
 
 template <int BITS, int GS>

@@ -139,12 +139,12 @@ skinny_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
     __syncthreads();
     // programmatic dependent launch, as in the mmv8 kernels: the next kernel of the stream may become resident now;
     // x and y are touched only after griddepcontrol.wait (a no-op for plain launches)
-    if (threadIdx.x == 0) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    if (threadIdx.x == 0) griddep_launch_dependents();
 
     if (warp == kWarps) {
         // ===================== producer: a handful of TMA boxes per stage =====================
         if (lane == 0) {
-            if (!p.early_weights) asm volatile("griddepcontrol.wait;" ::: "memory");
+            if (!p.early_weights) griddep_wait();
             const uint32_t box_bytes = (uint32_t)p.rs * 128u;
             for (int it = 0; it < ns; it++) {
                 const int s = it % kStages;
@@ -167,7 +167,7 @@ skinny_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant_
         // ===================== consumer warps =====================
         const int g = lane >> 2, t = lane & 3;
         const uint32_t ring_u32 = smem_u32(ring);
-        asm volatile("griddepcontrol.wait;" ::: "memory");  // x (and y) belong to the previous kernels of the stream
+        griddep_wait();  // x (and y) belong to the previous kernels of the stream
 
         struct Pre {            // per-stage operands fetched one stage ahead
             uint4 xn[NT][(CQ * 2 + 15) / 16];  // this thread's quarter of tokens g (+8), natural order (CQ bf16)
@@ -431,25 +431,10 @@ Plan make_plan(int64_t N, int64_t K, int bits, int gs, int nt = 1) {
 template <int BITS, int QW, bool SB_TMA, int NT>
 int launch_inst3(const CUtensorMap& tw, const CUtensorMap& ts, const CUtensorMap& tb, const SkinnyParams& p, size_t smem, int grid,
                  cudaStream_t st) {
-    static DeviceOnce configured;  // per device: the attribute is a per-device property
-    if (configured.need()) {
-        cudaError_t e = cudaFuncSetAttribute(skinny_kernel<BITS, QW, SB_TMA, NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        if (e != cudaSuccess) return check_cuda(e);
-        configured.done();
-    }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = mmv_get_pdl_mode() > 0 ? 1 : 0;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, skinny_kernel<BITS, QW, SB_TMA, NT>, tw, ts, tb, p);
-    count_launch();
-    return check_cuda(e);
+    constexpr auto kern = skinny_kernel<BITS, QW, SB_TMA, NT>;
+    const int rc = allow_dynamic_smem<kern>(227 * 1024);
+    if (rc != GBXQ_OK) return rc;
+    return launch(kern, dim3((unsigned)grid), dim3(kThreads), smem, st, true, tw, ts, tb, p);
 }
 
 template <int BITS, int QW, bool SB_TMA>
@@ -496,7 +481,7 @@ int launch_skinny(const void* x, const uint32_t* w, const void* s, const void* b
     p.nbox = pl.nbox;
     p.sb_off = pl.sb_off;
     p.slot_bytes = pl.slot;
-    p.early_weights = mmv_get_pdl_mode() >= 2 ? 1 : 0;
+    p.early_weights = pdl_early_weights();
     CUtensorMap tw, ts, tb;
     memset(&ts, 0, sizeof(ts));
     memset(&tb, 0, sizeof(tb));

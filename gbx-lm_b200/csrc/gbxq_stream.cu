@@ -215,26 +215,25 @@ __global__ void __launch_bounds__(kThreads, kMinCtas)
 }
 
 template <int GS, int MT> int launch_inst(const gbxq_stream_info* info, const void* blob, void* counters, cudaStream_t st) {
-    auto kern = stream_kernel<GS, MT>;
-    static DeviceOnce configured;            // per device: attribute and occupancy are per-device properties
+    constexpr auto kern = stream_kernel<GS, MT>;
+    static DeviceOnce configured;            // per device: occupancy is a per-device property
     static std::atomic<int> max_grid_of[64];  // resident CTAs of this kernel per device
     const int dev = DeviceOnce::dev();
     if (dev < 0) return GBXQ_ECUDA;
     if (configured.need()) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStreamSmemMax);
-        if (e != cudaSuccess) return check_cuda(e);
+        const int rc = allow_dynamic_smem<kern>((int)kStreamSmemMax);
+        if (rc != GBXQ_OK) return rc;
         int per_sm = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, kStreamSmemMax);
+        const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, kStreamSmemMax);
         if (e != cudaSuccess) return check_cuda(e);
         max_grid_of[dev].store(per_sm * device_sm_count(), std::memory_order_relaxed);
         configured.done();
     }
     if (info->grid > max_grid_of[dev].load(std::memory_order_relaxed)) return GBXQ_EUNSUPPORTED;  // every CTA must be resident
-    kern<<<info->grid, kThreads, (size_t)info->smem_bytes, st>>>(reinterpret_cast<const StreamCallDev*>(blob), info->ncalls,
-                                                              reinterpret_cast<unsigned*>(counters), info->stages,
-                                                              info->slot_bytes);
-    count_launch();
-    return check_cuda(cudaGetLastError());
+    // no PDL: the chain reads its first x without griddep_wait() (mmv8_body with STREAM = true)
+    return launch(kern, dim3(info->grid), dim3(kThreads), (size_t)info->smem_bytes, st, false,
+                  reinterpret_cast<const StreamCallDev*>(blob), info->ncalls, reinterpret_cast<unsigned*>(counters), info->stages,
+                  info->slot_bytes);
 }
 
 }  // namespace
