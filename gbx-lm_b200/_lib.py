@@ -44,6 +44,10 @@ EXPORTS = (
     "gbxq_rope_cache_quantized_ring",
     "gbxq_decode_attention_quantized",
     "gbxq_decode_attention_quantized_workspace_bytes",
+    "gbxq_rope_cache_rows",
+    "gbxq_decode_attention_rows",
+    "gbxq_rope_cache_quantized_rows",
+    "gbxq_decode_attention_quantized_rows",
     "gbxq_add_rmsnorm",
     "gbxq_silu_mul",
     "gbxq_head_gemv",
@@ -166,6 +170,14 @@ def get() -> ctypes.CDLL:
     lib.gbxq_decode_attention_quantized_workspace_bytes.argtypes = [ci, ci, ci, ci, i64]
     lib.gbxq_decode_attention_quantized.restype = ci
     lib.gbxq_decode_attention_quantized.argtypes = [vp] * 9 + [ci, ci, ci, ci, i64, i64, cf, ci, ci, vp, sz, vp]
+    lib.gbxq_rope_cache_rows.restype = ci
+    lib.gbxq_rope_cache_rows.argtypes = [vp, vp, vp, vp, vp, vp, vp, ci, ci, ci, ci, i64, i64, vp]
+    lib.gbxq_decode_attention_rows.restype = ci
+    lib.gbxq_decode_attention_rows.argtypes = [vp, vp, vp, vp, vp, ci, ci, ci, ci, i64, i64, cf, vp]
+    lib.gbxq_rope_cache_quantized_rows.restype = ci
+    lib.gbxq_rope_cache_quantized_rows.argtypes = [vp] * 11 + [ci, ci, ci, ci, i64, i64, ci, ci, vp]
+    lib.gbxq_decode_attention_quantized_rows.restype = ci
+    lib.gbxq_decode_attention_quantized_rows.argtypes = [vp] * 9 + [ci, ci, ci, ci, i64, i64, cf, ci, ci, vp, sz, vp]
     lib.gbxq_add_rmsnorm.restype = ci
     lib.gbxq_add_rmsnorm.argtypes = [vp, vp, vp, cf, vp, vp, i64, ci, vp]
     lib.gbxq_silu_mul.restype = ci

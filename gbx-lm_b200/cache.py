@@ -213,6 +213,12 @@ class StaticKVCache:
         return head_dim in (64, 128) and self.max_len <= DECODE_ATTENTION_MAX_KEYS
 
     def update(self, k: torch.Tensor, v: torch.Tensor, positions: torch.Tensor):
+        """k / v [B, n_kv, L, D] at positions int64 [L], or a decode step's [B, n_kv, 1, D] at per-row positions [B, 1]."""
+        if positions.dim() == 2:
+            rows = torch.arange(k.shape[0], device=k.device)
+            self.keys[rows, :, positions[:, 0]] = k[:, :, 0]
+            self.values[rows, :, positions[:, 0]] = v[:, :, 0]
+            return
         self.keys.index_copy_(2, positions, k)
         self.values.index_copy_(2, positions, v)
 
@@ -262,6 +268,11 @@ class StaticQuantizedKVCache:
         """k / v [B, n_kv, L, D] quantized into positions [at, at + L) (ops.quantize_into, one launch per side)."""
         ops.quantize_into(k, self.keys, at, self.group_size, self.bits)
         ops.quantize_into(v, self.values, at, self.group_size, self.bits)
+
+    def update_row(self, b: int, k: torch.Tensor, v: torch.Tensor, at: int):
+        """`update` of batch row b alone: k / v [1, n_kv, L, D] into that row's positions [at, at + L)."""
+        ops.quantize_into(k, tuple(t[b:b + 1] for t in self.keys), at, self.group_size, self.bits)
+        ops.quantize_into(v, tuple(t[b:b + 1] for t in self.values), at, self.group_size, self.bits)
 
     def prefix(self, n: int):
         return tuple(t[:, :, :n] for t in self.keys), tuple(t[:, :, :n] for t in self.values)

@@ -26,10 +26,12 @@ __device__ __forceinline__ __nv_bfloat16 tobf(float v) { return __float2bfloat16
 __global__ void rope_cache_kernel(__nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ k,
                                   const __nv_bfloat16* __restrict__ v, const int64_t* __restrict__ pos_p,
                                   const float* __restrict__ inv_freq, __nv_bfloat16* __restrict__ kc,
-                                  __nv_bfloat16* __restrict__ vc, int Hq, int Hkv, int D, int64_t max_len, int64_t keep) {
+                                  __nv_bfloat16* __restrict__ vc, int Hq, int Hkv, int D, int64_t max_len, int64_t keep,
+                                  int pos_stride) {
     const int h = blockIdx.x, b = blockIdx.y, i = threadIdx.x, half = D / 2;
     pdl_wait_then_trigger();
-    const int64_t pos = *pos_p;  // the RoPE angle is the absolute position's; k / v go to its cache row
+    // the RoPE angle is the absolute position's; k / v go to its cache row.  pos_stride 0: one position for every row
+    const int64_t pos = pos_p[(size_t)b * pos_stride];
     const int64_t row = kv_cache_row(pos, max_len, keep);
     if (row < 0) return;  // never write outside the cache
     if (h < Hq + Hkv) {
@@ -64,14 +66,15 @@ __global__ void __launch_bounds__(256) decode_attention_kernel(const __nv_bfloat
                                                                const __nv_bfloat16* __restrict__ vc,
                                                                const int64_t* __restrict__ pos_p,
                                                                __nv_bfloat16* __restrict__ out, int Hq, int Hkv,
-                                                               int64_t max_len, int64_t attend_len, float scale) {
+                                                               int64_t max_len, int64_t attend_len, float scale,
+                                                               int pos_stride) {
     constexpr int SPLITS = 256 / D;
     extern __shared__ float sc[];
     __shared__ float qs[D], red[8], part[SPLITS][D];
     const int h = blockIdx.x, b = blockIdx.y, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int hk = h / (Hq / Hkv);
     pdl_wait_then_trigger();
-    int64_t last = *pos_p;  // keys 0 .. pos are visible
+    int64_t last = pos_p[(size_t)b * pos_stride];  // keys 0 .. pos of this row are visible
     if (last >= attend_len) last = attend_len - 1;
     const int n = (int)(last + 1);
     const __nv_bfloat16* kp = kc + ((size_t)b * Hkv + hk) * max_len * D;
@@ -195,15 +198,16 @@ __global__ void __launch_bounds__(256) silu_mul_kernel(const __nv_bfloat16* __re
 }  // namespace
 
 int launch_rope_cache(void* q, const void* k, const void* v, const int64_t* pos, const float* inv_freq, void* kc, void* vc,
-                      int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep, cudaStream_t st) {
+                      int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep, int pos_stride, cudaStream_t st) {
     if (B < 1 || Hq < 1 || Hkv < 1 || D < 2 || (D & 1) || D / 2 > 1024 || max_len < 1 || keep >= max_len) return GBXQ_ESHAPE;
     return launch(rope_cache_kernel, dim3(Hq + 2 * Hkv, B), dim3(D / 2), 0, st, true,
         reinterpret_cast<__nv_bfloat16*>(q), reinterpret_cast<const __nv_bfloat16*>(k), reinterpret_cast<const __nv_bfloat16*>(v),
-        pos, inv_freq, reinterpret_cast<__nv_bfloat16*>(kc), reinterpret_cast<__nv_bfloat16*>(vc), Hq, Hkv, D, max_len, keep);
+        pos, inv_freq, reinterpret_cast<__nv_bfloat16*>(kc), reinterpret_cast<__nv_bfloat16*>(vc), Hq, Hkv, D, max_len, keep, pos_stride);
 }
 
 int launch_decode_attention(const void* q, const void* kc, const void* vc, const int64_t* pos, void* out, int B, int Hq,
-                            int Hkv, int D, int64_t max_len, int64_t attend_len, float scale, cudaStream_t st) {
+                            int Hkv, int D, int64_t max_len, int64_t attend_len, float scale, int pos_stride,
+                            cudaStream_t st) {
     if (B < 1 || Hq < 1 || Hkv < 1 || Hq % Hkv || max_len < 1 || attend_len < 1 || attend_len > max_len) return GBXQ_ESHAPE;
     const dim3 grid(Hq, B);
     auto Q = reinterpret_cast<const __nv_bfloat16*>(q);
@@ -216,8 +220,8 @@ int launch_decode_attention(const void* q, const void* kc, const void* vc, const
     if (rc == GBXQ_OK) rc = allow_dynamic_smem<decode_attention_kernel<128>>(49152 * 4);
     if (rc != GBXQ_OK) return rc;
     switch (D) {
-        case 64: return launch(decode_attention_kernel<64>, grid, dim3(256), smem, st, true, Q, K, V, pos, O, Hq, Hkv, max_len, attend_len, scale);
-        case 128: return launch(decode_attention_kernel<128>, grid, dim3(256), smem, st, true, Q, K, V, pos, O, Hq, Hkv, max_len, attend_len, scale);
+        case 64: return launch(decode_attention_kernel<64>, grid, dim3(256), smem, st, true, Q, K, V, pos, O, Hq, Hkv, max_len, attend_len, scale, pos_stride);
+        case 128: return launch(decode_attention_kernel<128>, grid, dim3(256), smem, st, true, Q, K, V, pos, O, Hq, Hkv, max_len, attend_len, scale, pos_stride);
     }
     return GBXQ_EUNSUPPORTED;
 }

@@ -69,13 +69,14 @@ __global__ void __launch_bounds__(32) rope_cache_q_kernel(__nv_bfloat16* __restr
                                                           __nv_bfloat16* __restrict__ ks, __nv_bfloat16* __restrict__ kb,
                                                           uint32_t* __restrict__ vq, __nv_bfloat16* __restrict__ vs,
                                                           __nv_bfloat16* __restrict__ vb, int Hq, int Hkv, int64_t max_len,
-                                                          int64_t keep, int gs) {
+                                                          int64_t keep, int gs, int pos_stride) {
     constexpr int EPL = D / 32, HALF = D / 2, W = D * BITS / 32;
     __shared__ uint32_t codes_s[D];
     __shared__ __align__(8) uint8_t bytes_s[D * BITS / 8 + 8];
     const int h = blockIdx.x, b = blockIdx.y, lane = threadIdx.x;
     pdl_wait_then_trigger();
-    const int64_t pos = *pos_p;  // the RoPE angle is the absolute position's; k / v go to its cache row
+    // the RoPE angle is the absolute position's; k / v go to its cache row.  pos_stride 0: one position for every row
+    const int64_t pos = pos_p[(size_t)b * pos_stride];
     const int64_t slot = kv_cache_row(pos, max_len, keep);
     if (slot < 0) return;  // never write outside the cache
     float val[EPL];
@@ -198,7 +199,7 @@ __global__ void __launch_bounds__(kThreads, 2) qattn_partial_kernel(
     const __nv_bfloat16* __restrict__ q, const uint32_t* __restrict__ kq, const __nv_bfloat16* __restrict__ ks,
     const __nv_bfloat16* __restrict__ kb, const uint32_t* __restrict__ vq, const __nv_bfloat16* __restrict__ vs,
     const __nv_bfloat16* __restrict__ vb, const int64_t* __restrict__ pos_p, float* __restrict__ ws, int Hq, int Hkv,
-    int64_t max_len, int64_t attend_len, int nch, int gs, float qscale) {
+    int64_t max_len, int64_t attend_len, int nch, int gs, float qscale, int pos_stride) {
     using P = QAttnPlan<D, BITS, GMAX>;
     constexpr int W = P::W, RUNS = P::RUNS;
     extern __shared__ __align__(16) uint8_t smem[];
@@ -218,7 +219,7 @@ __global__ void __launch_bounds__(kThreads, 2) qattn_partial_kernel(
     const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
     const int G = Hq / Hkv, ng = D / gs;
     pdl_wait_then_trigger();
-    int64_t last = *pos_p;  // keys 0 .. pos are visible
+    int64_t last = pos_p[(size_t)b * pos_stride];  // keys 0 .. pos of this row are visible
     if (last >= attend_len) last = attend_len - 1;
     const int64_t n = last + 1;
     const int64_t j0 = (int64_t)chunk * kChunk;
@@ -389,10 +390,11 @@ __global__ void __launch_bounds__(kThreads, 2) qattn_partial_kernel(
 // grid (Hq, B), D threads: the chunks with visible keys, in chunk order
 template <int D>
 __global__ void __launch_bounds__(D) qattn_combine_kernel(const float* __restrict__ ws, const int64_t* __restrict__ pos_p,
-                                                          __nv_bfloat16* __restrict__ out, int Hq, int64_t attend_len, int nch) {
+                                                          __nv_bfloat16* __restrict__ out, int Hq, int64_t attend_len, int nch,
+                                                          int pos_stride) {
     const int h = blockIdx.x, b = blockIdx.y, d = threadIdx.x;
     pdl_wait_then_trigger();
-    int64_t last = *pos_p;
+    int64_t last = pos_p[(size_t)b * pos_stride];
     if (last >= attend_len) last = attend_len - 1;
     const int nv = last < 0 ? 0 : (int)((last + kChunk) / kChunk);
     const float* base = ws + ((size_t)b * Hq + h) * (size_t)nch * (D + 2);
@@ -424,7 +426,7 @@ int launch_rope_q(const QCacheWrite& a, cudaStream_t st) {
         reinterpret_cast<__nv_bfloat16*>(a.q), reinterpret_cast<const __nv_bfloat16*>(a.k),
         reinterpret_cast<const __nv_bfloat16*>(a.v), a.pos, a.inv_freq, a.kq, reinterpret_cast<__nv_bfloat16*>(a.ks),
         reinterpret_cast<__nv_bfloat16*>(a.kb), a.vq, reinterpret_cast<__nv_bfloat16*>(a.vs),
-        reinterpret_cast<__nv_bfloat16*>(a.vb), a.Hq, a.Hkv, a.max_len, a.keep, a.gs);
+        reinterpret_cast<__nv_bfloat16*>(a.vb), a.Hq, a.Hkv, a.max_len, a.keep, a.gs, a.pos_stride);
 }
 
 template <int D>
@@ -450,10 +452,10 @@ int launch_qattn_t(const QAttn& a, cudaStream_t st) {
     rc = launch(kern, dim3(nch, a.Hkv, a.B), dim3(kThreads), (size_t)P::BYTES, st, true,
         reinterpret_cast<const __nv_bfloat16*>(a.q), a.kq, reinterpret_cast<const __nv_bfloat16*>(a.ks),
         reinterpret_cast<const __nv_bfloat16*>(a.kb), a.vq, reinterpret_cast<const __nv_bfloat16*>(a.vs),
-        reinterpret_cast<const __nv_bfloat16*>(a.vb), a.pos, ws, a.Hq, a.Hkv, a.max_len, a.attend_len, nch, a.gs, qscale);
+        reinterpret_cast<const __nv_bfloat16*>(a.vb), a.pos, ws, a.Hq, a.Hkv, a.max_len, a.attend_len, nch, a.gs, qscale, a.pos_stride);
     if (rc != GBXQ_OK) return rc;
     return launch(qattn_combine_kernel<D>, dim3(a.Hq, a.B), dim3(D), 0, st, true, (const float*)ws, a.pos,
-                  reinterpret_cast<__nv_bfloat16*>(a.out), a.Hq, a.attend_len, nch);
+                  reinterpret_cast<__nv_bfloat16*>(a.out), a.Hq, a.attend_len, nch, a.pos_stride);
 }
 
 template <int D, int BITS>

@@ -108,9 +108,10 @@ class RoPE(nn.Module):
         self.register_buffer("inv_freq", rope_inv_freq(dims, base, scaling), persistent=False)
 
     def forward(self, x: torch.Tensor, positions: torch.Tensor) -> torch.Tensor:
-        # x [B, H, L, D]; positions int64 [L]
-        ang = positions.to(torch.float32)[:, None] * self.inv_freq[None, :]  # [L, D/2]
-        cos, sin = ang.cos()[None, None], ang.sin()[None, None]
+        # x [B, H, L, D]; positions int64 [L] (shared by the rows) or [B, L] (per row)
+        ang = positions.to(torch.float32)[..., None] * self.inv_freq  # [L, D/2] or [B, L, D/2]
+        ang = ang[None, None] if ang.dim() == 2 else ang[:, None]
+        cos, sin = ang.cos(), ang.sin()
         h = self.dims // 2
         x1, x2 = x[..., :h].float(), x[..., h : 2 * h].float()
         out = torch.cat([x1 * cos - x2 * sin, x1 * sin + x2 * cos], dim=-1)
@@ -159,7 +160,10 @@ class Attention(nn.Module):  # gbx_lm/models/qllama.py:39-96
         # one grouped launch for the three projections of x (ref qllama.py:76 calls them back to back)
         q, k, v = ops.quantized_matmul_grouped(x, (self.q_proj, self.k_proj, self.v_proj))
         quantized = isinstance(cache, StaticQuantizedKVCache)
+        per_row = positions.dim() == 2  # [B, 1]: a decode step whose rows sit at different positions
         if fused_decode_ok(x, L, cache) and self.takes_fused_decode(cache):
+            if per_row:
+                positions = positions.reshape(B)
             # decode step: RoPE + cache write in one launch, one-query attention in another (SURVEY.md 8f rank 2); over
             # the quantized cache the attention is split-K on the codes (+ its combine launch)
             qh = q.view(B, self.n_heads, self.head_dim)
@@ -175,6 +179,9 @@ class Attention(nn.Module):  # gbx_lm/models/qllama.py:39-96
                 ops.rope_cache(qh, kh, vh, positions, self.rope.inv_freq, cache.keys, cache.values, keep=cache.keep)
                 out = ops.decode_attention(qh, cache.keys, cache.values, positions, self.scale, attend_len)
             return self.tp.row_parallel(self.o_proj, out.view(B, 1, -1))
+        if per_row and cache is not None and cache.keep is not None:
+            raise ValueError("per-row positions on a rotating cache need the fused decode path (the unfused ring glue "
+                             "works on one shared offset)")
         q = self.rope(q.view(B, L, self.n_heads, -1).transpose(1, 2), positions)
         k = self.rope(k.view(B, L, self.n_kv_heads, -1).transpose(1, 2), positions)
         v = v.view(B, L, self.n_kv_heads, -1).transpose(1, 2)
@@ -191,7 +198,11 @@ class Attention(nn.Module):  # gbx_lm/models/qllama.py:39-96
             # the rows are written at the HOST offset (Model.forward has already advanced it past these L positions), so
             # this path is not graph-capturable
             T = cache.offset
-            cache.update(k, v, T - L)
+            if per_row:  # each row at its own position (read back to the host)
+                for b, p in enumerate(positions[:, 0].tolist()):
+                    cache.update_row(b, k[b:b + 1], v[b:b + 1], p)
+            else:
+                cache.update(k, v, T - L)
             keys, values = cache.prefix(T)
         else:
             cache.update(k, v, positions)
@@ -200,13 +211,16 @@ class Attention(nn.Module):  # gbx_lm/models/qllama.py:39-96
         if ring:
             visible = cache.visible(key_positions, positions)
         else:  # causal over absolute positions: key j visible to query at position p iff j <= p
-            visible = torch.arange(T, device=x.device)[None, :] <= positions[:, None]
+            visible = torch.arange(T, device=x.device) <= positions[..., None]  # [L, T], per row [B, L, T]
         if quantized:
             # the reference's attention on the codes (gbx_lm/models/base.py:65-98), with its additive mask
-            mask = torch.zeros((L, T), dtype=q.dtype, device=x.device).masked_fill_(~visible, float("-inf"))
+            mask = torch.zeros(visible.shape, dtype=q.dtype, device=x.device).masked_fill_(~visible, float("-inf"))
+            if per_row:  # against the scores [B, Hq, L, T], or [B, Hkv, Hq / Hkv, L, T] under GQA
+                mask = mask.view(B, *[1] * (1 if self.n_heads == self.n_kv_heads else 2), L, T)
             out = quantized_scaled_dot_product_attention(q, keys, values, self.scale, mask, cache.group_size, cache.bits)
         else:
-            out = F.scaled_dot_product_attention(q, keys, values, attn_mask=visible[None, None], scale=self.scale,
+            mask = visible[:, None] if per_row else visible[None, None]
+            out = F.scaled_dot_product_attention(q, keys, values, attn_mask=mask, scale=self.scale,
                                                  enable_gqa=self.n_heads != self.n_kv_heads)
         if ring:
             cache.store(keys, values, cache.offset - L, L)
@@ -287,9 +301,14 @@ class Model(nn.Module):  # gbx_lm/models/qllama.py:177-209
             self.lm_head = nn.Linear(args.hidden_size, args.vocab_size, bias=False)
 
     def forward(self, inputs: torch.Tensor, cache: Optional[List[Union[StaticKVCache, StaticQuantizedKVCache]]] = None,
-                positions: Optional[torch.Tensor] = None, attend_len: Optional[int] = None, hidden_states: bool = False):
-        """inputs int64 [B, L].  positions int64 [L] (absolute); default = cache offset .. offset+L.
-        attend_len: number of cache positions attended (None = whole static cache, for graph replay)."""
+                positions: Optional[torch.Tensor] = None, attend_len: Optional[int] = None, hidden_states: bool = False,
+                head_columns: Optional[torch.Tensor] = None):
+        """inputs int64 [B, L].  positions int64 [L] (absolute, shared by the rows); default = cache offset .. offset+L.
+        A decode step (L = 1) may instead give each row its own position, int64 [B, 1]; the caller keeps the caches'
+        offsets then.  attend_len: number of cache positions attended (None = whole static cache, for graph replay).
+        head_columns int64 [B]: only column head_columns[b] of row b goes through the vocabulary projection (logits
+        [B, 1, V], hidden states [B, 1, H]) -- what a batched prefill needs, without the [B, L, V] logits of every
+        position; None: every position."""
         L = inputs.shape[1]
         if positions is None:
             off = cache[0].offset if cache is not None else 0
@@ -299,6 +318,8 @@ class Model(nn.Module):  # gbx_lm/models/qllama.py:177-209
                     c.offset = off + L
                 attend_len = cache[0].attend_len  # off + L; at most the window on a rotating cache
         out = self.model(inputs, positions, cache, attend_len)
+        if head_columns is not None:
+            out = out[torch.arange(out.shape[0], device=out.device), head_columns][:, None]
         # vocabulary projection (qllama.py:194-198): decode-sized inputs go through the streaming bf16 GEMV
         # (gbxq_head_gemv), prefill through the dense matmul
         head = self.model.embed_tokens.weight if self.args.tie_word_embeddings else self.lm_head.weight

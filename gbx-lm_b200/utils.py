@@ -5,6 +5,7 @@
     make_shards/save_weights gbx_lm/utils.py:967-988, 1055-1104
     save_config              gbx_lm/utils.py:1107-1127
     generate_step            gbx_lm/utils.py:217-338   (batch-1 prefill in 2048-token chunks + greedy decode)
+    batch_generate           (new) greedy decode of B prompts of different lengths in one batch
 
 The on-disk layout is exactly what gba2mlx emits (gbx_lm/gba2mlx.py:47-65): `model*.safetensors` with
 `<module>.{qweight,scales,zeros[,bias]}`, metadata {"format": "mlx"}, `config.json` carrying
@@ -309,9 +310,11 @@ def fast_argmax(x: torch.Tensor) -> torch.Tensor:
 
 class DecodeGraph:
     """One decode step (token ids [B,1] -> logits) captured in a CUDA graph: the whole step --
-    7*L QuantizedLinear launches plus the glue -- replays as one submission (SURVEY.md 7.2 item 1)."""
+    7*L QuantizedLinear launches plus the glue -- replays as one submission (SURVEY.md 7.2 item 1).
+    per_row: the B rows sit at their own positions, `pos` int64 [B] (prompts of different lengths), instead of one
+    shared position `pos` [1]."""
 
-    def __init__(self, model, cache, batch: int = 1):
+    def __init__(self, model, cache, batch: int = 1, per_row: bool = False):
         # the unfused quantized and rotating paths write at the HOST offset, which a replay cannot advance
         if any((isinstance(c, StaticQuantizedKVCache) or c.keep is not None) and not layer.self_attn.takes_fused_decode(c)
                for layer, c in zip(model.layers, cache)):
@@ -320,30 +323,41 @@ class DecodeGraph:
         self.model, self.cache = model, cache
         dev = cache[0].device
         self.tok = torch.zeros((batch, 1), dtype=torch.long, device=dev)
-        self.pos = torch.zeros((1,), dtype=torch.long, device=dev)
+        self.pos = torch.zeros((batch if per_row else 1,), dtype=torch.long, device=dev)
+        self.per_row = per_row
         self.logits = None
         self.graph = None
 
-    def capture(self, tokens: torch.Tensor, position: int, device_loop: int = 0):
+    def _set(self, tokens: torch.Tensor, position) -> None:
+        self.tok.copy_(tokens.reshape(self.tok.shape))
+        if self.per_row:
+            self.pos.copy_(position)
+        else:
+            self.pos.fill_(position)
+
+    def _positions(self) -> torch.Tensor:
+        return self.pos[:, None] if self.per_row else self.pos
+
+    def capture(self, tokens: torch.Tensor, position, device_loop: int = 0):
         """Warm-up + capture at (tokens, position) = the step that will be replayed first, so the KV
         entries written during warm-up/capture are exactly the ones that step writes anyway.
         device_loop = n > 0: the greedy sampler is part of the graph -- argmax of the logits (= argmax of the
         log-probabilities, utils.py:285,305-306), fed back as the next step's token, position advanced and the token
-        appended to `self.out` [n] on the device -- so that n steps replay back to back without a host round trip."""
-        self.tok.copy_(tokens.reshape(self.tok.shape))
-        self.pos.fill_(position)
+        appended to `self.out` [n] on the device -- so that n steps replay back to back without a host round trip.
+        position: an int, or with per_row an int64 [B] device tensor."""
+        self._set(tokens, position)
         s = torch.cuda.Stream()
         s.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(s), torch.no_grad():
             for _ in range(2):
-                self.model(self.tok, self.cache, positions=self.pos, attend_len=None)
+                self.model(self.tok, self.cache, positions=self._positions(), attend_len=None)
         torch.cuda.current_stream().wait_stream(s)
         if device_loop:
             self.out = torch.zeros((device_loop, self.tok.shape[0]), dtype=torch.long, device=self.tok.device)
             self.idx = torch.zeros((1,), dtype=torch.long, device=self.tok.device)
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph), torch.no_grad():
-            self.logits = self.model(self.tok, self.cache, positions=self.pos, attend_len=None)
+            self.logits = self.model(self.tok, self.cache, positions=self._positions(), attend_len=None)
             if device_loop:
                 nxt = fast_argmax(self.logits[:, -1, :])  # [B]; bf16 -> fp32 is order preserving, so no cast
                 self.out.index_copy_(0, self.idx, nxt[None])
@@ -352,12 +366,13 @@ class DecodeGraph:
                 self.idx.add_(1)
         return self
 
-    def step(self, tokens: torch.Tensor, position: int) -> torch.Tensor:
-        self.tok.copy_(tokens.reshape(self.tok.shape))
-        self.pos.fill_(position)
+    def step(self, tokens: torch.Tensor, position) -> torch.Tensor:
+        """One replay at `position` (as in `capture`); the caches' offset becomes the largest position + 1."""
+        self._set(tokens, position)
         self.graph.replay()
+        last = int(position.max()) if self.per_row else position
         for c in self.cache:
-            c.offset = position + 1
+            c.offset = last + 1
         return self.logits[:, -1, :]
 
 
@@ -372,37 +387,100 @@ def _kv_quantizer(cache: list, kv_bits: Optional[int], kv_group_size: int, quant
     return step
 
 
-def _decode_graph(model, cache, tok, position: int, device_loop: int = 0) -> Optional[DecodeGraph]:
-    """A captured decode step, or None where the cache cannot be captured (a quantized or rotating cache off the fused
-    path)."""
+def _decode_graph(model, cache, tok, position, device_loop: int = 0) -> Optional[DecodeGraph]:
+    """A captured decode step for the rows of `tok` [B] at `position` (an int, or an int64 [B] device tensor of per-row
+    positions), or None where the cache cannot be captured (a quantized or rotating cache off the fused path)."""
     try:
-        dg = DecodeGraph(model, cache)
+        dg = DecodeGraph(model, cache, batch=tok.numel(), per_row=isinstance(position, torch.Tensor))
     except ValueError:
         return None
     return dg.capture(tok, position, device_loop=device_loop)
 
 
-def _prompt_cache(model, run_len: int, max_kv_size: Optional[int]) -> list:
+def _prompt_cache(model, run_len: int, max_kv_size: Optional[int], batch: int = 1) -> list:
     """Flat caches for a run of `run_len` positions, or rotating caches of window max_kv_size."""
     if max_kv_size is None:
-        return qllama.make_prompt_cache(model, 1, run_len)
-    return qllama.make_prompt_cache(model, 1, max_kv_size, keep=DEFAULT_KV_KEEP)
+        return qllama.make_prompt_cache(model, batch, run_len)
+    return qllama.make_prompt_cache(model, batch, max_kv_size, keep=DEFAULT_KV_KEEP)
+
+
+def _prefill_chunks(model, tokens: torch.Tensor, cache: list, prefill_step_size: int, kv: dict,
+                    last: Optional[List[int]] = None) -> torch.Tensor:
+    """tokens [B, L] through the model in `prefill_step_size` chunks at the shared positions 0 .. L-1, with the conversion
+    rule of `generate_step` applied after every model call.  Returns the logits [B, V] of the final column, or with
+    `last` (one column per row) those of column last[b] of row b: each chunk sends only those columns through the
+    vocabulary projection (Model.forward head_columns)."""
+    quantize_cache = _kv_quantizer(cache, **kv)
+    L = tokens.shape[1]
+    out = None
+    with torch.no_grad():
+        for c0 in range(0, L, prefill_step_size):
+            chunk = tokens[:, c0:c0 + prefill_step_size]
+            n = chunk.shape[1]
+            if last is None:
+                logits = model(chunk, cache)
+                if c0 + n == L:
+                    out = logits[:, -1, :]
+            else:
+                here = [c0 <= j < c0 + n for j in last]
+                cols = torch.tensor([min(max(j - c0, 0), n - 1) for j in last], device=tokens.device)
+                logits = model(chunk, cache, head_columns=cols)[:, 0]
+                if any(here):
+                    keep = torch.tensor(here, device=tokens.device)[:, None]
+                    out = logits if out is None else torch.where(keep, logits, out)
+            quantize_cache()
+    return out
 
 
 def prefill(model, prompt: torch.Tensor, cache: list, prefill_step_size: int = 2048, kv_bits: Optional[int] = None,
             kv_group_size: int = 64, quantized_kv_start: int = 0) -> torch.Tensor:
     """The prompt (token ids [n], on the model's device) through the model in `prefill_step_size` chunks, with the
     conversion rule of `generate_step` applied after every model call; returns the logits of the last position [1, V]."""
-    quantize_cache = _kv_quantizer(cache, kv_bits, kv_group_size, quantized_kv_start)
-    y = prompt.reshape(-1)
-    with torch.no_grad():
-        while y.numel() > prefill_step_size:
-            model(y[:prefill_step_size][None], cache)
-            quantize_cache()
-            y = y[prefill_step_size:]
-        logits = model(y[None], cache)[:, -1, :]
-        quantize_cache()
-    return logits
+    kv = dict(kv_bits=kv_bits, kv_group_size=kv_group_size, quantized_kv_start=quantized_kv_start)
+    return _prefill_chunks(model, prompt.reshape(1, -1), cache, prefill_step_size, kv)
+
+
+def _conversion_segments(cache: list, steps: int, pos0: int, kv_bits: Optional[int], quantized_kv_start: int) -> List[int]:
+    """Replay counts of the captured decode: replay i takes the caches' offset to pos0 + i + 1, and the reference
+    converts after the call that takes the offset past quantized_kv_start, i.e. after replay
+    max(0, quantized_kv_start - pos0): the replays up to there are one segment, the rest a second one on a graph of the
+    quantized step."""
+    head = steps
+    if kv_bits is not None and isinstance(cache[0], StaticKVCache):
+        head = min(max(quantized_kv_start - pos0, 0) + 1, steps)
+    return [head] + ([steps - head] if head < steps else [])
+
+
+def _device_decode(model, cache: list, tok: torch.Tensor, position, pos0: int, steps: int, kv: dict, where: str):
+    """`steps` greedy decode steps as replays of captured steps with the sampler inside (DecodeGraph device_loop), split
+    at the kv_bits conversion (_conversion_segments).  tok [B]: the first tokens; position: the first replay's position
+    (an int, or int64 [B] per row); pos0: the caches' offset before it.  Returns (first tokens as a list, the time after
+    the first capture, [n, B] token tensors of the segments); the caches' offset is left at pos0 + steps."""
+    per_row = isinstance(position, torch.Tensor)
+    outs, offset = [], pos0
+    for i, n in enumerate(_conversion_segments(cache, steps, pos0, kv["kv_bits"], kv["quantized_kv_start"])):
+        if i:  # at the conversion: convert the caches, continue from the last token on a graph of the quantized step
+            for c in cache:
+                c.offset = offset
+            maybe_quantize_kv_cache(cache, kv["quantized_kv_start"], kv["kv_group_size"], kv["kv_bits"])
+            tok = dg.tok[:, 0].clone()
+            position = dg.pos.clone() if per_row else position
+        # captured even for zero replays (max_tokens 1): the cache is checked for capturability all the same
+        dg = _decode_graph(model, cache, tok, position, device_loop=max(n, 1))
+        if dg is None:
+            raise ValueError(f"{where}: the quantized cache cannot be captured (unfused decode path)")
+        if i == 0:  # the capture of the first graph counts as prompt time
+            first = tok.tolist()
+            t_first = time.perf_counter()
+        for _ in range(n):
+            dg.graph.replay()
+        outs.append(dg.out[:n])
+        offset += n
+        if not per_row:
+            position += n
+    for c in cache:
+        c.offset = offset
+    return first, t_first, outs
 
 
 def generate_step(
@@ -478,42 +556,88 @@ def generate_tokens_device(model, prompt: torch.Tensor, max_tokens: int = 128, p
     t0 = time.perf_counter()
     tok = torch.argmax(prefill(model, y, cache, prefill_step_size, **kv).float(), dim=-1)
     pos0 = cache[0].offset
-    steps = max(max_tokens - 1, 0)
-    # replay i decodes position pos0 + i; the reference converts after the call that takes the offset past
-    # quantized_kv_start, i.e. after replay max(0, quantized_kv_start - pos0): the replays up to there are one segment,
-    # the rest a second one on a graph of the quantized step
-    head = steps
-    if kv_bits is not None and isinstance(cache[0], StaticKVCache):
-        head = min(max(quantized_kv_start - pos0, 0) + 1, steps)
-    segments = [head] + ([steps - head] if head < steps else [])
-    outs, pos = [], pos0
-    for i, n in enumerate(segments):
-        if i:  # at the conversion: convert the caches, continue from the last token on a graph of the quantized step
-            for c in cache:
-                c.offset = pos
-            maybe_quantize_kv_cache(cache, quantized_kv_start, kv_group_size, kv_bits)
-            tok = dg.tok[:, 0].clone()
-        # captured even for zero replays (max_tokens 1): the cache is checked for capturability all the same
-        dg = _decode_graph(model, cache, tok, pos, device_loop=max(n, 1))
-        if dg is None:
-            raise ValueError("generate_tokens_device: the quantized cache cannot be captured (unfused decode path)")
-        if i == 0:  # the capture of the first graph counts as prompt time
-            first = int(tok.item())
-            t_first = time.perf_counter()
-        for _ in range(n):
-            dg.graph.replay()
-        outs.append(dg.out[:n, 0])
-        pos += n
+    first, t_first, outs = _device_decode(model, cache, tok, pos0, pos0, max(max_tokens - 1, 0), kv,
+                                          "generate_tokens_device")
     torch.cuda.synchronize()
     t1 = time.perf_counter()
-    toks = [first] + [int(t) for o in outs for t in o.tolist()]
-    for c in cache:
-        c.offset = pos
+    toks = first + [int(t) for o in outs for t in o[:, 0].tolist()]
     stats = {
         "prompt_tokens": int(n_prompt), "prompt_tps": n_prompt / max(t_first - t0, 1e-9),
         "generation_tokens": len(toks), "generation_tps": max(len(toks) - 1, 1) / max(t1 - t_first, 1e-9),
     }
     return toks, stats
+
+
+def _pad_prompts(prompts, pad_id: int, max_kv_size: Optional[int]) -> Tuple[torch.Tensor, List[int]]:
+    """The prompts (1-D token-id tensors) right-padded with pad_id into one [B, Lmax] matrix, and their lengths."""
+    if len(prompts) == 0:
+        raise ValueError("batch_generate: no prompts")
+    if any(p.dim() != 1 for p in prompts):
+        raise ValueError("batch_generate: each prompt must be a 1-D tensor of token ids")
+    lens = [int(p.numel()) for p in prompts]
+    if min(lens) == 0:
+        raise ValueError(f"batch_generate: prompt {lens.index(0)} is empty")
+    if max_kv_size is not None and max(lens) > max_kv_size:
+        # the prefill ring logic (window_with / store_runs) runs on one shared offset: pads would push real tokens out
+        raise ValueError(f"batch_generate: the longest prompt ({max(lens)} tokens) exceeds max_kv_size = {max_kv_size}")
+    tokens = torch.full((len(prompts), max(lens)), int(pad_id), dtype=torch.long)
+    for b, p in enumerate(prompts):
+        tokens[b, :lens[b]] = p.to(torch.long)
+    return tokens, lens
+
+
+def batch_generate(model, prompts: List[torch.Tensor], max_tokens: int = 128, *, prefill_step_size: int = 2048,
+                   kv_bits: Optional[int] = None, kv_group_size: int = 64, quantized_kv_start: int = 0,
+                   max_kv_size: Optional[int] = None, pad_id: int = 0,
+                   use_cuda_graph: bool = True) -> Tuple[List[List[int]], dict]:
+    """Greedy generation of `max_tokens` tokens for each of B prompts of any lengths (1-D token-id tensors), in one batch.
+
+    The prompts are padded on the right to the longest, Lmax, and prefilled together at the shared positions
+    0 .. Lmax-1: under the causal mask no real token sees a pad, and row b's first token is the argmax at its column
+    len_b - 1.  Each decode step then runs the B rows at their own positions (row b's s-th step at len_b + s): the
+    step writes that row's cache row and attends that row's keys 0 .. len_b + s, so the pad keys of row b are
+    overwritten before any of its queries can see them, and no row's tokens depend on the pads or on the other rows.
+    kv_bits / kv_group_size / quantized_kv_start / max_kv_size as in generate_step (the conversion rule reads the
+    caches' offset, Lmax + steps so far); the longest prompt must fit max_kv_size.  use_cuda_graph: the captured step
+    with the sampler inside (as generate_tokens_device); False: eager steps, the same tokens.
+
+    Returns (the tokens of each row, stats) with the reference's timing definitions summed over the rows:
+    prompt_tps = prompt tokens / time to the first tokens, generation_tps = generated tokens / decode time."""
+    dev = next(model.parameters()).device
+    tokens, lens = _pad_prompts(prompts, pad_id, max_kv_size)
+    B, Lmax = tokens.shape
+    tokens = tokens.to(dev)
+    kv = dict(kv_bits=kv_bits, kv_group_size=kv_group_size, quantized_kv_start=quantized_kv_start)
+    cache = _prompt_cache(model, Lmax + max_tokens + 1, max_kv_size, batch=B)
+    steps = max(max_tokens - 1, 0)
+    t0 = time.perf_counter()
+    tok = fast_argmax(_prefill_chunks(model, tokens, cache, prefill_step_size, kv, last=[n - 1 for n in lens]))
+    position = torch.tensor(lens, dtype=torch.long, device=dev)  # of each row's first decode step
+    if use_cuda_graph:
+        first, t_first, outs = _device_decode(model, cache, tok, position, Lmax, steps, kv, "batch_generate")
+        rows = [first] + [r for o in outs for r in o.tolist()]
+    else:
+        quantize_cache = _kv_quantizer(cache, **kv)
+        rows = [tok.tolist()]
+        t_first = time.perf_counter()
+        with torch.no_grad():
+            for s in range(steps):
+                for c in cache:
+                    c.offset = Lmax + s + 1
+                logits = model(tok[:, None], cache, positions=position[:, None], attend_len=cache[0].attend_len)
+                quantize_cache()
+                tok = fast_argmax(logits[:, -1, :])
+                position = position + 1
+                rows.append(tok.tolist())
+    if tok.is_cuda:
+        torch.cuda.synchronize(dev)
+    t1 = time.perf_counter()
+    out = [list(r) for r in zip(*rows)]  # rows: the B tokens of each step
+    stats = {
+        "prompt_tokens": int(sum(lens)), "prompt_tps": sum(lens) / max(t_first - t0, 1e-9),
+        "generation_tokens": B * len(out[0]), "generation_tps": B * max(len(out[0]) - 1, 1) / max(t1 - t_first, 1e-9),
+    }
+    return out, stats
 
 
 def generate_tokens(model, prompt: torch.Tensor, max_tokens: int = 128, **kw) -> Tuple[List[int], dict]:

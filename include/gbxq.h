@@ -276,6 +276,26 @@ int gbxq_add_rmsnorm(const void* x, const void* r, const void* w, float eps, voi
 int gbxq_rope_cache_ring(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev,
                          void* k_cache, void* v_cache, int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep,
                          void* stream);
+
+/*
+ * Per-row positions: a decode step of B sequences that sit at different positions (prompts of different lengths).
+ * pos_dev is int64 [B] on the device, row b at position pos_dev[b]; everything else is as in the entry point each
+ * generalises, row by row.
+ *   gbxq_rope_cache_rows             gbxq_rope_cache / gbxq_rope_cache_ring with row b rotated at pos_dev[b] and its k / v
+ *                                    written to row pos_dev[b] (keep < 0: a flat cache) or ring_slot(pos_dev[b])
+ *                                    (0 <= keep < max_len: a rotating cache); keep >= max_len: GBXQ_ESHAPE.  A row whose
+ *                                    position is outside the cache writes nothing; the other rows are unaffected.
+ *   gbxq_decode_attention_rows       gbxq_decode_attention with row b attending keys [0, min(pos_dev[b], attend_len-1)]
+ *                                    of its own cache.
+ * With all B positions equal they are bitwise the shared-position entry points, and they enqueue the same launches.
+ * The quantized pair, gbxq_rope_cache_quantized_rows and gbxq_decode_attention_quantized_rows, is declared below.
+ */
+int gbxq_rope_cache_rows(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev,
+                         void* k_cache, void* v_cache, int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep,
+                         void* stream);
+int gbxq_decode_attention_rows(const void* q, const void* k_cache, const void* v_cache, const int64_t* pos_dev, void* out,
+                               int B, int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale,
+                               void* stream);
 int gbxq_silu_mul(const void* gate, const void* up, void* out, int64_t n, void* stream);
 
 /*
@@ -314,6 +334,20 @@ int gbxq_decode_attention_quantized(const void* q, const uint32_t* k_codes, cons
                                     const int64_t* pos_dev, void* out, int B, int Hq, int Hkv, int D, int64_t max_len,
                                     int64_t attend_len, float scale, int bits, int group_size, void* workspace,
                                     size_t workspace_bytes, void* stream);
+/* The per-row forms of the quantized pair (pos_dev int64 [B], one position per row; see gbxq_rope_cache_rows):
+ * gbxq_rope_cache_quantized_rows takes keep as gbxq_rope_cache_rows does (< 0 flat, [0, max_len) a ring, else
+ * GBXQ_ESHAPE).  In gbxq_decode_attention_quantized_rows, the chunks past a row's own position are empty partials, so
+ * each row's result is bitwise independent of attend_len and of the other rows; the workspace is sized as for
+ * gbxq_decode_attention_quantized. */
+int gbxq_rope_cache_quantized_rows(void* q, const void* k, const void* v, const int64_t* pos_dev,
+                                   const float* inv_freq_dev, uint32_t* k_codes, void* k_scales, void* k_biases,
+                                   uint32_t* v_codes, void* v_scales, void* v_biases, int B, int Hq, int Hkv, int D,
+                                   int64_t max_len, int64_t keep, int bits, int group_size, void* stream);
+int gbxq_decode_attention_quantized_rows(const void* q, const uint32_t* k_codes, const void* k_scales,
+                                         const void* k_biases, const uint32_t* v_codes, const void* v_scales,
+                                         const void* v_biases, const int64_t* pos_dev, void* out, int B, int Hq, int Hkv,
+                                         int D, int64_t max_len, int64_t attend_len, float scale, int bits,
+                                         int group_size, void* workspace, size_t workspace_bytes, void* stream);
 
 /*
  * Vocabulary projection of the decode step (SURVEY.md 8f rank 1): y[M,V] = x[M,K] . weight[V,K]^T with UNQUANTIZED bf16
