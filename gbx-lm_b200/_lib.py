@@ -40,14 +40,8 @@ EXPORTS = (
     "gbxq_rope_cache",
     "gbxq_decode_attention",
     "gbxq_rope_cache_quantized",
-    "gbxq_rope_cache_ring",
-    "gbxq_rope_cache_quantized_ring",
     "gbxq_decode_attention_quantized",
     "gbxq_decode_attention_quantized_workspace_bytes",
-    "gbxq_rope_cache_rows",
-    "gbxq_decode_attention_rows",
-    "gbxq_rope_cache_quantized_rows",
-    "gbxq_decode_attention_quantized_rows",
     "gbxq_add_rmsnorm",
     "gbxq_silu_mul",
     "gbxq_head_gemv",
@@ -157,27 +151,15 @@ def get() -> ctypes.CDLL:
     lib.gbxq_get_option.argtypes = [ci]
     cf = ctypes.c_float
     lib.gbxq_rope_cache.restype = ci
-    lib.gbxq_rope_cache.argtypes = [vp, vp, vp, vp, vp, vp, vp, ci, ci, ci, ci, i64, vp]
+    lib.gbxq_rope_cache.argtypes = [vp, vp, vp, vp, ci, vp, vp, vp, ci, ci, ci, ci, i64, i64, vp]
     lib.gbxq_decode_attention.restype = ci
-    lib.gbxq_decode_attention.argtypes = [vp, vp, vp, vp, vp, ci, ci, ci, ci, i64, i64, cf, vp]
+    lib.gbxq_decode_attention.argtypes = [vp, vp, vp, vp, ci, vp, ci, ci, ci, ci, i64, i64, cf, vp]
     lib.gbxq_rope_cache_quantized.restype = ci
-    lib.gbxq_rope_cache_quantized.argtypes = [vp] * 11 + [ci, ci, ci, ci, i64, ci, ci, vp]
-    lib.gbxq_rope_cache_ring.restype = ci
-    lib.gbxq_rope_cache_ring.argtypes = [vp, vp, vp, vp, vp, vp, vp, ci, ci, ci, ci, i64, i64, vp]
-    lib.gbxq_rope_cache_quantized_ring.restype = ci
-    lib.gbxq_rope_cache_quantized_ring.argtypes = [vp] * 11 + [ci, ci, ci, ci, i64, i64, ci, ci, vp]
+    lib.gbxq_rope_cache_quantized.argtypes = [vp] * 4 + [ci] + [vp] * 7 + [ci, ci, ci, ci, i64, i64, ci, ci, vp]
     lib.gbxq_decode_attention_quantized_workspace_bytes.restype = sz
     lib.gbxq_decode_attention_quantized_workspace_bytes.argtypes = [ci, ci, ci, ci, i64]
     lib.gbxq_decode_attention_quantized.restype = ci
-    lib.gbxq_decode_attention_quantized.argtypes = [vp] * 9 + [ci, ci, ci, ci, i64, i64, cf, ci, ci, vp, sz, vp]
-    lib.gbxq_rope_cache_rows.restype = ci
-    lib.gbxq_rope_cache_rows.argtypes = [vp, vp, vp, vp, vp, vp, vp, ci, ci, ci, ci, i64, i64, vp]
-    lib.gbxq_decode_attention_rows.restype = ci
-    lib.gbxq_decode_attention_rows.argtypes = [vp, vp, vp, vp, vp, ci, ci, ci, ci, i64, i64, cf, vp]
-    lib.gbxq_rope_cache_quantized_rows.restype = ci
-    lib.gbxq_rope_cache_quantized_rows.argtypes = [vp] * 11 + [ci, ci, ci, ci, i64, i64, ci, ci, vp]
-    lib.gbxq_decode_attention_quantized_rows.restype = ci
-    lib.gbxq_decode_attention_quantized_rows.argtypes = [vp] * 9 + [ci, ci, ci, ci, i64, i64, cf, ci, ci, vp, sz, vp]
+    lib.gbxq_decode_attention_quantized.argtypes = [vp] * 8 + [ci, vp, ci, ci, ci, ci, i64, i64, cf, ci, ci, vp, sz, vp]
     lib.gbxq_add_rmsnorm.restype = ci
     lib.gbxq_add_rmsnorm.argtypes = [vp, vp, vp, cf, vp, vp, i64, ci, vp]
     lib.gbxq_silu_mul.restype = ci
@@ -190,7 +172,7 @@ def get() -> ctypes.CDLL:
     lib.gbxq_allreduce_oneshot.argtypes = [vp, vp, i64, ci, vp, vp, i64, ci, ci, u32, vp]
     lib.gbxq_qmm_rowpar_allreduce.restype = ci
     lib.gbxq_qmm_rowpar_allreduce.argtypes = [vp, vp, vp, vp, vp, vp, i64, i64, i64, ci, ci, ci, ctypes.POINTER(Comm), vp]
-    if lib.gbxq_abi_version() != 1:
+    if lib.gbxq_abi_version() != 2:
         raise ImportError("libgbxq.so ABI version mismatch; rebuild with `python -m gbx_lm_b200.build --force`")
     _lib = lib
     return lib

@@ -306,8 +306,8 @@ class _Ring:
 
     -- the sinks and the last window - keep positions: min(p + 1, window) keys, the set a reference decode step sees.
 
-    A decode step writes its row on the device (gbxq_rope_cache_ring) and attends the first `attend_len` rows, which are
-    exactly the ring's contents in some order.  A call of L positions at off .. off + L - 1 that takes the ring past its
+    A decode step writes its row on the device (the `keep` argument of gbxq_rope_cache) and attends the first
+    `attend_len` rows, which are exactly the ring's contents in some order.  A call of L positions at off .. off + L - 1 that takes the ring past its
     window (`wraps`) attends `window_with` (the valid rows plus its own keys) under `visible`, then `store`s the
     positions that survive it."""
 

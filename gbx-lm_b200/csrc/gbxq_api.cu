@@ -298,97 +298,42 @@ int gbxq_dequantize(const uint32_t* qweight, const void* scales, const void* bia
     return launch_dequantize(qweight, scales, biases, w_out, N, K, bits, group_size, dtype, (cudaStream_t)stream);
 }
 
-int gbxq_rope_cache(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev, void* k_cache,
-                    void* v_cache, int B, int Hq, int Hkv, int D, int64_t max_len, void* stream) {
-    if (!q || !k || !v || !pos_dev || !inv_freq_dev || !k_cache || !v_cache) return GBXQ_ENULL;
-    return launch_rope_cache(q, k, v, pos_dev, inv_freq_dev, k_cache, v_cache, B, Hq, Hkv, D, max_len, -1, 0,
+int gbxq_rope_cache(void* q, const void* k, const void* v, const int64_t* pos_dev, int pos_stride,
+                    const float* inv_freq_dev, void* k_cache, void* v_cache, int B, int Hq, int Hkv, int D,
+                    int64_t max_len, int64_t keep, void* stream) {
+    return launch_rope_cache(q, k, v, pos_dev, pos_stride, inv_freq_dev, k_cache, v_cache, B, Hq, Hkv, D, max_len, keep,
                              (cudaStream_t)stream);
 }
 
-int gbxq_rope_cache_ring(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev,
-                         void* k_cache, void* v_cache, int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep,
-                         void* stream) {
-    if (!q || !k || !v || !pos_dev || !inv_freq_dev || !k_cache || !v_cache) return GBXQ_ENULL;
-    if (keep < 0 || keep >= max_len) return GBXQ_ESHAPE;
-    return launch_rope_cache(q, k, v, pos_dev, inv_freq_dev, k_cache, v_cache, B, Hq, Hkv, D, max_len, keep, 0,
-                             (cudaStream_t)stream);
+int gbxq_decode_attention(const void* q, const void* k_cache, const void* v_cache, const int64_t* pos_dev,
+                          int pos_stride, void* out, int B, int Hq, int Hkv, int D, int64_t max_len,
+                          int64_t attend_len, float scale, void* stream) {
+    return launch_decode_attention(q, k_cache, v_cache, pos_dev, pos_stride, out, B, Hq, Hkv, D, max_len, attend_len,
+                                   scale, (cudaStream_t)stream);
 }
 
-int gbxq_rope_cache_rows(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev,
-                         void* k_cache, void* v_cache, int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep,
-                         void* stream) {
-    if (!q || !k || !v || !pos_dev || !inv_freq_dev || !k_cache || !v_cache) return GBXQ_ENULL;
-    if (keep >= max_len) return GBXQ_ESHAPE;
-    return launch_rope_cache(q, k, v, pos_dev, inv_freq_dev, k_cache, v_cache, B, Hq, Hkv, D, max_len, keep < 0 ? -1 : keep,
-                             1, (cudaStream_t)stream);
-}
-
-int gbxq_decode_attention(const void* q, const void* k_cache, const void* v_cache, const int64_t* pos_dev, void* out, int B,
-                          int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale, void* stream) {
-    if (!q || !k_cache || !v_cache || !pos_dev || !out) return GBXQ_ENULL;
-    return launch_decode_attention(q, k_cache, v_cache, pos_dev, out, B, Hq, Hkv, D, max_len, attend_len, scale, 0,
-                                   (cudaStream_t)stream);
-}
-
-int gbxq_decode_attention_rows(const void* q, const void* k_cache, const void* v_cache, const int64_t* pos_dev, void* out,
-                               int B, int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale,
-                               void* stream) {
-    if (!q || !k_cache || !v_cache || !pos_dev || !out) return GBXQ_ENULL;
-    return launch_decode_attention(q, k_cache, v_cache, pos_dev, out, B, Hq, Hkv, D, max_len, attend_len, scale, 1,
-                                   (cudaStream_t)stream);
-}
-
-int gbxq_rope_cache_quantized(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev,
-                              uint32_t* k_codes, void* k_scales, void* k_biases, uint32_t* v_codes, void* v_scales,
-                              void* v_biases, int B, int Hq, int Hkv, int D, int64_t max_len, int bits, int group_size,
-                              void* stream) {
-    const QCacheWrite a{q, k, v, pos_dev, inv_freq_dev, k_codes, k_scales, k_biases, v_codes, v_scales, v_biases,
-                        B, Hq, Hkv, D, max_len, bits, group_size, -1};
-    return launch_rope_cache_quantized(a, (cudaStream_t)stream);
-}
-
-int gbxq_rope_cache_quantized_ring(void* q, const void* k, const void* v, const int64_t* pos_dev,
-                                   const float* inv_freq_dev, uint32_t* k_codes, void* k_scales, void* k_biases,
-                                   uint32_t* v_codes, void* v_scales, void* v_biases, int B, int Hq, int Hkv, int D,
-                                   int64_t max_len, int64_t keep, int bits, int group_size, void* stream) {
-    if (keep < 0 || keep >= max_len) return GBXQ_ESHAPE;
-    const QCacheWrite a{q, k, v, pos_dev, inv_freq_dev, k_codes, k_scales, k_biases, v_codes, v_scales, v_biases,
-                        B, Hq, Hkv, D, max_len, bits, group_size, keep};
-    return launch_rope_cache_quantized(a, (cudaStream_t)stream);
-}
-
-int gbxq_rope_cache_quantized_rows(void* q, const void* k, const void* v, const int64_t* pos_dev,
-                                   const float* inv_freq_dev, uint32_t* k_codes, void* k_scales, void* k_biases,
-                                   uint32_t* v_codes, void* v_scales, void* v_biases, int B, int Hq, int Hkv, int D,
-                                   int64_t max_len, int64_t keep, int bits, int group_size, void* stream) {
-    if (keep >= max_len) return GBXQ_ESHAPE;
-    const QCacheWrite a{q, k, v, pos_dev, inv_freq_dev, k_codes, k_scales, k_biases, v_codes, v_scales, v_biases,
-                        B, Hq, Hkv, D, max_len, bits, group_size, keep < 0 ? -1 : keep, 1};
-    return launch_rope_cache_quantized(a, (cudaStream_t)stream);
+int gbxq_rope_cache_quantized(void* q, const void* k, const void* v, const int64_t* pos_dev, int pos_stride,
+                              const float* inv_freq_dev, uint32_t* k_codes, void* k_scales, void* k_biases,
+                              uint32_t* v_codes, void* v_scales, void* v_biases, int B, int Hq, int Hkv, int D,
+                              int64_t max_len, int64_t keep, int bits, int group_size, void* stream) {
+    return launch_rope_cache_quantized({q, k, v, pos_dev, pos_stride, inv_freq_dev, k_codes, k_scales, k_biases, v_codes,
+                                        v_scales, v_biases, B, Hq, Hkv, D, max_len, keep, bits, group_size},
+                                       (cudaStream_t)stream);
 }
 
 size_t gbxq_decode_attention_quantized_workspace_bytes(int B, int Hq, int Hkv, int D, int64_t attend_len) {
     return qattn_workspace_bytes(B, Hq, Hkv, D, attend_len);
 }
 
-int gbxq_decode_attention_quantized(const void* q, const uint32_t* k_codes, const void* k_scales, const void* k_biases,
-                                    const uint32_t* v_codes, const void* v_scales, const void* v_biases,
-                                    const int64_t* pos_dev, void* out, int B, int Hq, int Hkv, int D, int64_t max_len,
-                                    int64_t attend_len, float scale, int bits, int group_size, void* workspace,
-                                    size_t workspace_bytes, void* stream) {
-    const QAttn a{q, k_codes, k_scales, k_biases, v_codes, v_scales, v_biases, pos_dev, out, B, Hq, Hkv, D, max_len,
-                  attend_len, scale, bits, group_size, workspace, workspace_bytes};
-    return launch_decode_attention_quantized(a, (cudaStream_t)stream);
-}
-
-int gbxq_decode_attention_quantized_rows(const void* q, const uint32_t* k_codes, const void* k_scales,
-                                         const void* k_biases, const uint32_t* v_codes, const void* v_scales,
-                                         const void* v_biases, const int64_t* pos_dev, void* out, int B, int Hq, int Hkv,
-                                         int D, int64_t max_len, int64_t attend_len, float scale, int bits,
-                                         int group_size, void* workspace, size_t workspace_bytes, void* stream) {
-    const QAttn a{q, k_codes, k_scales, k_biases, v_codes, v_scales, v_biases, pos_dev, out, B, Hq, Hkv, D, max_len,
-                  attend_len, scale, bits, group_size, workspace, workspace_bytes, 1};
-    return launch_decode_attention_quantized(a, (cudaStream_t)stream);
+int gbxq_decode_attention_quantized(const void* q, const uint32_t* k_codes, const void* k_scales,
+                                    const void* k_biases, const uint32_t* v_codes, const void* v_scales,
+                                    const void* v_biases, const int64_t* pos_dev, int pos_stride, void* out, int B,
+                                    int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale,
+                                    int bits, int group_size, void* workspace, size_t workspace_bytes, void* stream) {
+    return launch_decode_attention_quantized({q, k_codes, k_scales, k_biases, v_codes, v_scales, v_biases, pos_dev,
+                                              pos_stride, out, B, Hq, Hkv, D, max_len, attend_len, scale, bits,
+                                              group_size, workspace, workspace_bytes},
+                                             (cudaStream_t)stream);
 }
 
 int gbxq_add_rmsnorm(const void* x, const void* r, const void* w, float eps, void* h_out, void* y_out, int64_t rows, int H,

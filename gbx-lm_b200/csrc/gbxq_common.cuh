@@ -283,12 +283,13 @@ int stream_plan(const gbxq_stream_call* calls, int ncalls, int64_t M, int dtype,
                 gbxq_stream_info* info);
 void stream_debug_patch(void* host_blob, int ncalls, unsigned long long* dbg_dev);
 int launch_stream(const gbxq_stream_info* info, const void* blob, void* counters, cudaStream_t st);
-// keep < 0: a flat cache; keep in [0, max_len): a rotating cache with keep sink rows (kv_cache_row).
-// pos_stride 0: pos[0] is the position of every batch row; 1: pos[b] is row b's
-int launch_rope_cache(void* q, const void* k, const void* v, const int64_t* pos, const float* inv_freq, void* kc, void* vc,
-                      int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep, int pos_stride, cudaStream_t st);
-int launch_decode_attention(const void* q, const void* kc, const void* vc, const int64_t* pos, void* out, int B, int Hq,
-                            int Hkv, int D, int64_t max_len, int64_t attend_len, float scale, int pos_stride,
+// The decode-step cache write and attention (gbxq_glue.cu / gbxq_qattn.cu).  pos_stride 0: pos[0] is the position of
+// every batch row; 1: pos[b] is row b's; else GBXQ_ESHAPE.  keep < 0: a flat cache; keep in [0, max_len): a rotating
+// cache with keep sink rows (kv_cache_row); else GBXQ_ESHAPE.  The launchers check every argument.
+int launch_rope_cache(void* q, const void* k, const void* v, const int64_t* pos, int pos_stride, const float* inv_freq,
+                      void* kc, void* vc, int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep, cudaStream_t st);
+int launch_decode_attention(const void* q, const void* kc, const void* vc, const int64_t* pos, int pos_stride, void* out,
+                            int B, int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale,
                             cudaStream_t st);
 // arguments of the quantized-cache decode step (gbxq_qattn.cu): one (codes, scales, biases) triple per side, bf16
 struct QCacheWrite {
@@ -296,16 +297,15 @@ struct QCacheWrite {
     const void* k;
     const void* v;
     const int64_t* pos;
+    int pos_stride;
     const float* inv_freq;
     uint32_t* kq;
     void *ks, *kb;
     uint32_t* vq;
     void *vs, *vb;
     int B, Hq, Hkv, D;
-    int64_t max_len;
+    int64_t max_len, keep;
     int bits, gs;
-    int64_t keep;  // < 0: a flat cache; else the sink rows of a rotating cache (kv_cache_row)
-    int pos_stride = 0;  // 0: pos[0] for every batch row; 1: pos[b] for row b
 };
 struct QAttn {
     const void* q;
@@ -314,6 +314,7 @@ struct QAttn {
     const uint32_t* vq;
     const void *vs, *vb;
     const int64_t* pos;
+    int pos_stride;
     void* out;
     int B, Hq, Hkv, D;
     int64_t max_len, attend_len;
@@ -321,7 +322,6 @@ struct QAttn {
     int bits, gs;
     void* ws;
     size_t ws_bytes;
-    int pos_stride = 0;  // as QCacheWrite::pos_stride
 };
 int launch_rope_cache_quantized(const QCacheWrite& a, cudaStream_t st);
 int launch_decode_attention_quantized(const QAttn& a, cudaStream_t st);

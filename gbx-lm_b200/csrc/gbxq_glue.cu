@@ -197,18 +197,22 @@ __global__ void __launch_bounds__(256) silu_mul_kernel(const __nv_bfloat16* __re
 
 }  // namespace
 
-int launch_rope_cache(void* q, const void* k, const void* v, const int64_t* pos, const float* inv_freq, void* kc, void* vc,
-                      int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep, int pos_stride, cudaStream_t st) {
+int launch_rope_cache(void* q, const void* k, const void* v, const int64_t* pos, int pos_stride, const float* inv_freq,
+                      void* kc, void* vc, int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep, cudaStream_t st) {
+    if (!q || !k || !v || !pos || !inv_freq || !kc || !vc) return GBXQ_ENULL;
     if (B < 1 || Hq < 1 || Hkv < 1 || D < 2 || (D & 1) || D / 2 > 1024 || max_len < 1 || keep >= max_len) return GBXQ_ESHAPE;
+    if (pos_stride != 0 && pos_stride != 1) return GBXQ_ESHAPE;
     return launch(rope_cache_kernel, dim3(Hq + 2 * Hkv, B), dim3(D / 2), 0, st, true,
         reinterpret_cast<__nv_bfloat16*>(q), reinterpret_cast<const __nv_bfloat16*>(k), reinterpret_cast<const __nv_bfloat16*>(v),
         pos, inv_freq, reinterpret_cast<__nv_bfloat16*>(kc), reinterpret_cast<__nv_bfloat16*>(vc), Hq, Hkv, D, max_len, keep, pos_stride);
 }
 
-int launch_decode_attention(const void* q, const void* kc, const void* vc, const int64_t* pos, void* out, int B, int Hq,
-                            int Hkv, int D, int64_t max_len, int64_t attend_len, float scale, int pos_stride,
+int launch_decode_attention(const void* q, const void* kc, const void* vc, const int64_t* pos, int pos_stride, void* out,
+                            int B, int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale,
                             cudaStream_t st) {
+    if (!q || !kc || !vc || !pos || !out) return GBXQ_ENULL;
     if (B < 1 || Hq < 1 || Hkv < 1 || Hq % Hkv || max_len < 1 || attend_len < 1 || attend_len > max_len) return GBXQ_ESHAPE;
+    if (pos_stride != 0 && pos_stride != 1) return GBXQ_ESHAPE;
     const dim3 grid(Hq, B);
     auto Q = reinterpret_cast<const __nv_bfloat16*>(q);
     auto K = reinterpret_cast<const __nv_bfloat16*>(kc);

@@ -480,6 +480,7 @@ int launch_rope_cache_quantized(const QCacheWrite& a, cudaStream_t st) {
     const int rc = check_common(a.B, a.Hq, a.Hkv, a.D, a.max_len, a.bits, a.gs);
     if (rc != GBXQ_OK) return rc;
     if (a.keep >= a.max_len) return GBXQ_ESHAPE;
+    if (a.pos_stride != 0 && a.pos_stride != 1) return GBXQ_ESHAPE;
     if (!a.q || !a.k || !a.v || !a.pos || !a.inv_freq || !a.kq || !a.ks || !a.kb || !a.vq || !a.vs || !a.vb) return GBXQ_ENULL;
     if (((uintptr_t)a.kq | (uintptr_t)a.vq) & 3) return GBXQ_EALIGN;
     return a.D == 64 ? rope_q_bits<64>(a, st) : rope_q_bits<128>(a, st);
@@ -494,6 +495,7 @@ int launch_decode_attention_quantized(const QAttn& a, cudaStream_t st) {
     const int rc = check_common(a.B, a.Hq, a.Hkv, a.D, a.max_len, a.bits, a.gs);
     if (rc != GBXQ_OK) return rc;
     if (a.attend_len < 1 || a.attend_len > a.max_len || chunks_of(a.attend_len) > 65535 * 64) return GBXQ_ESHAPE;
+    if (a.pos_stride != 0 && a.pos_stride != 1) return GBXQ_ESHAPE;
     if (!a.q || !a.kq || !a.ks || !a.kb || !a.vq || !a.vs || !a.vb || !a.pos || !a.out || !a.ws) return GBXQ_ENULL;
     if (a.ws_bytes < qattn_workspace_bytes(a.B, a.Hq, a.Hkv, a.D, a.attend_len)) return GBXQ_EWORKSPACE;
     if (((uintptr_t)a.kq | (uintptr_t)a.vq) & 3 || ((uintptr_t)a.ws & 15)) return GBXQ_EALIGN;

@@ -522,17 +522,16 @@ def _check_keep(keep: Optional[int], max_len: int, where: str) -> Optional[int]:
     return keep
 
 
-def _per_row(position: torch.Tensor, b: int, q: torch.Tensor, where: str) -> bool:
-    """Whether `position` gives one position per batch row (int64 [B], B > 1: the `_rows` entry points) rather than one
-    shared by all rows (int64 [1]).  A per-row tensor must be contiguous on the device of q."""
+def _pos_stride(position: torch.Tensor, b: int, q: torch.Tensor, where: str) -> int:
+    """The pos_stride of the decode-step entry points for `position`: 0 for int64 [1] (one position shared by all rows),
+    1 for int64 [B] (row b at position[b]).  The kernels read it, so it must be contiguous on the device of q."""
     if position.dim() != 1 or position.numel() not in (1, b):
         raise ValueError(f"{where}: position must be int64 [1] (shared) or [B] = [{b}] (one per row), "
                          f"got {tuple(position.shape)}")
-    if position.numel() == 1:
-        return False
     if position.dtype != torch.int64 or position.device != q.device or not position.is_contiguous():
-        raise ValueError(f"{where}: per-row positions must be a contiguous int64 [B] tensor on the device of q")
-    return True
+        raise ValueError(f"{where}: position must be a contiguous int64 tensor on the device of q, "
+                         f"got {position.dtype} on {position.device}")
+    return 0 if position.numel() == 1 else 1
 
 
 def rope_cache(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, position: torch.Tensor, inv_freq: torch.Tensor,
@@ -540,27 +539,19 @@ def rope_cache(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, position: torc
     """gbxq_rope_cache: q [B,Hq,D] rotated IN PLACE (returned), k rotated and v copied into the caches [B,Hkv,max_len,D] at
     `position` (int64 device tensor [1]).  Replaces RoPE + cache.update of a decode step (gbx_lm/models/qllama.py:83-88).
     keep = an int: the caches are a rotating window of max_len rows with `keep` sinks, and k / v go to row
-    ring_slot(position) (gbxq_rope_cache_ring; cache.ring_slot).  position int64 [B]: row b at position[b]
-    (gbxq_rope_cache_rows)."""
+    ring_slot(position) (cache.ring_slot).  position int64 [B]: row b at position[b]."""
     _bf16c(q, k, v, k_cache, v_cache)
     b, hq, d = q.shape
     hkv, max_len = k_cache.shape[1], k_cache.shape[2]
-    if position.dtype != torch.int64 or inv_freq.dtype != torch.float32 or inv_freq.numel() != d // 2:
-        raise ValueError("rope_cache: position int64 [1], inv_freq float32 [D/2]")
+    if inv_freq.dtype != torch.float32 or inv_freq.numel() != d // 2:
+        raise ValueError("rope_cache: inv_freq float32 [D/2]")
     keep = _check_keep(keep, max_len, "rope_cache")
-    rows = _per_row(position, b, q, "rope_cache")
-    args = (q.data_ptr(), k.data_ptr(), v.data_ptr(), position.data_ptr(), inv_freq.data_ptr(), k_cache.data_ptr(),
-            v_cache.data_ptr(), b, hq, hkv, d, max_len)
-    lib = _lib.get()
+    stride = _pos_stride(position, b, q, "rope_cache")
     with torch.cuda.device(q.device):
-        if rows:
-            rc = lib.gbxq_rope_cache_rows(*args, -1 if keep is None else keep, _stream())
-            name = "gbxq_rope_cache_rows"
-        elif keep is None:
-            rc, name = lib.gbxq_rope_cache(*args, _stream()), "gbxq_rope_cache"
-        else:
-            rc, name = lib.gbxq_rope_cache_ring(*args, keep, _stream()), "gbxq_rope_cache_ring"
-    _lib.check(rc, name)
+        rc = _lib.get().gbxq_rope_cache(q.data_ptr(), k.data_ptr(), v.data_ptr(), position.data_ptr(), stride,
+                                        inv_freq.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), b, hq, hkv, d,
+                                        max_len, -1 if keep is None else keep, _stream())
+    _lib.check(rc, "gbxq_rope_cache")
     return q
 
 
@@ -568,19 +559,17 @@ def decode_attention(q: torch.Tensor, k_cache: torch.Tensor, v_cache: torch.Tens
                      attend_len: Optional[int] = None) -> torch.Tensor:
     """gbxq_decode_attention: one query row per head, q [B,Hq,D], against the static caches, keys 0..position visible
     (and < attend_len), GQA.  Returns [B,Hq,D].  Replaces mask + scaled_dot_product_attention (qllama.py:90-93).
-    position int64 [B]: row b sees keys 0..position[b] (gbxq_decode_attention_rows)."""
+    position int64 [B]: row b sees keys 0..position[b]."""
     _bf16c(q, k_cache, v_cache)
     b, hq, d = q.shape
     hkv, max_len = k_cache.shape[1], k_cache.shape[2]
-    lib = _lib.get()
-    fn, name = lib.gbxq_decode_attention, "gbxq_decode_attention"
-    if _per_row(position, b, q, "decode_attention"):
-        fn, name = lib.gbxq_decode_attention_rows, "gbxq_decode_attention_rows"
+    stride = _pos_stride(position, b, q, "decode_attention")
     out = torch.empty_like(q)
     with torch.cuda.device(q.device):
-        rc = fn(q.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), position.data_ptr(), out.data_ptr(), b, hq, hkv, d,
-                max_len, int(attend_len or max_len), float(scale), _stream())
-    _lib.check(rc, name)
+        rc = _lib.get().gbxq_decode_attention(q.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), position.data_ptr(),
+                                              stride, out.data_ptr(), b, hq, hkv, d, max_len,
+                                              int(attend_len or max_len), float(scale), _stream())
+    _lib.check(rc, "gbxq_decode_attention")
     return out
 
 
@@ -621,31 +610,22 @@ def rope_cache_quantized(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, posi
     `position` (int64 device tensor [1]) of its (codes, scales, biases) triple -- bit-identical to `rope_cache` into a bf16
     row followed by `quantize_into` of that row.  The quantized counterpart of `rope_cache` (RoPE +
     QuantizedKVCache.update_and_fetch, gbx_lm/models/cache.py:172-185).  keep = an int: row ring_slot(position) of a
-    rotating cache, as `rope_cache` (gbxq_rope_cache_quantized_ring).  position int64 [B]: row b at position[b]
-    (gbxq_rope_cache_quantized_rows)."""
+    rotating cache, as `rope_cache`.  position int64 [B]: row b at position[b]."""
     group_size, bits = int(group_size), int(bits)
     b, hq, hkv, d, max_len = _check_qcache(q, k_cache3, v_cache3, group_size, bits)
     _bf16c(k, v)
     if tuple(k.shape) != (b, hkv, d) or tuple(v.shape) != (b, hkv, d):
         raise ValueError(f"rope_cache_quantized: k / v must be [B, Hkv, D] = {(b, hkv, d)}")
-    if (position.dtype != torch.int64 or position.device != q.device or inv_freq.dtype != torch.float32
-            or inv_freq.numel() != d // 2 or inv_freq.device != q.device):
-        raise ValueError("rope_cache_quantized: position int64 [1], inv_freq float32 [D/2], on the device of q")
+    if inv_freq.dtype != torch.float32 or inv_freq.numel() != d // 2 or inv_freq.device != q.device:
+        raise ValueError("rope_cache_quantized: inv_freq float32 [D/2] on the device of q")
     keep = _check_keep(keep, max_len, "rope_cache_quantized")
-    rows = _per_row(position, b, q, "rope_cache_quantized")
-    args = (q.data_ptr(), k.data_ptr(), v.data_ptr(), position.data_ptr(), inv_freq.data_ptr(),
-            *[t.data_ptr() for t in k_cache3], *[t.data_ptr() for t in v_cache3], b, hq, hkv, d, max_len)
-    lib = _lib.get()
+    stride = _pos_stride(position, b, q, "rope_cache_quantized")
     with torch.cuda.device(q.device):
-        if rows:
-            rc = lib.gbxq_rope_cache_quantized_rows(*args, -1 if keep is None else keep, bits, group_size, _stream())
-            name = "gbxq_rope_cache_quantized_rows"
-        elif keep is None:
-            rc, name = lib.gbxq_rope_cache_quantized(*args, bits, group_size, _stream()), "gbxq_rope_cache_quantized"
-        else:
-            rc = lib.gbxq_rope_cache_quantized_ring(*args, keep, bits, group_size, _stream())
-            name = "gbxq_rope_cache_quantized_ring"
-    _lib.check(rc, name)
+        rc = _lib.get().gbxq_rope_cache_quantized(
+            q.data_ptr(), k.data_ptr(), v.data_ptr(), position.data_ptr(), stride, inv_freq.data_ptr(),
+            *[t.data_ptr() for t in k_cache3], *[t.data_ptr() for t in v_cache3], b, hq, hkv, d, max_len,
+            -1 if keep is None else keep, bits, group_size, _stream())
+    _lib.check(rc, "gbxq_rope_cache_quantized")
     return q
 
 
@@ -669,28 +649,23 @@ def decode_attention_quantized(q: torch.Tensor, k_cache3, v_cache3, position: to
     """gbxq_decode_attention_quantized: one query row per head, q [B,Hq,D], against the quantized triples, keys
     0..position visible (and < attend_len, default the whole cache), GQA.  Returns [B,Hq,D] bf16.  The result does not
     depend on attend_len beyond the clamp (bitwise).  Replaces quantized_scaled_dot_product_attention at decode
-    (gbx_lm/models/base.py:65-98).  position int64 [B]: row b sees keys 0..position[b]
-    (gbxq_decode_attention_quantized_rows)."""
+    (gbx_lm/models/base.py:65-98).  position int64 [B]: row b sees keys 0..position[b]."""
     group_size, bits = int(group_size), int(bits)
     b, hq, hkv, d, max_len = _check_qcache(q, k_cache3, v_cache3, group_size, bits)
     attend_len = int(max_len if attend_len is None else attend_len)
     if not 1 <= attend_len <= max_len:
         raise ValueError(f"decode_attention_quantized: attend_len {attend_len} outside [1, {max_len}]")
-    if position.dtype != torch.int64 or position.device != q.device:
-        raise ValueError("decode_attention_quantized: position must be an int64 [1] tensor on the device of q")
+    stride = _pos_stride(position, b, q, "decode_attention_quantized")
     lib = _lib.get()
-    fn, name = lib.gbxq_decode_attention_quantized, "gbxq_decode_attention_quantized"
-    if _per_row(position, b, q, "decode_attention_quantized"):
-        fn, name = lib.gbxq_decode_attention_quantized_rows, "gbxq_decode_attention_quantized_rows"
     need = int(lib.gbxq_decode_attention_quantized_workspace_bytes(b, hq, hkv, d, attend_len))
     out = torch.empty_like(q)
     with torch.cuda.device(q.device):
         ws = _qattn_workspace(q.device, need)
-        rc = fn(
+        rc = lib.gbxq_decode_attention_quantized(
             q.data_ptr(), *[t.data_ptr() for t in k_cache3], *[t.data_ptr() for t in v_cache3], position.data_ptr(),
-            out.data_ptr(), b, hq, hkv, d, max_len, attend_len, float(scale), bits, group_size, ws.data_ptr(), ws.numel(),
-            _stream())
-    _lib.check(rc, name)
+            stride, out.data_ptr(), b, hq, hkv, d, max_len, attend_len, float(scale), bits, group_size, ws.data_ptr(),
+            ws.numel(), _stream())
+    _lib.check(rc, "gbxq_decode_attention_quantized")
     return out
 
 

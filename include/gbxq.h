@@ -46,7 +46,7 @@
 extern "C" {
 #endif
 
-#define GBXQ_ABI_VERSION 1
+#define GBXQ_ABI_VERSION 2
 
 typedef enum gbxq_status {
     GBXQ_OK = 0,
@@ -240,62 +240,47 @@ uint64_t gbxq_launch_count(void);
 /*
  * Decode-step glue (SURVEY.md 8f rank 2: the fusions either side of the path).  What the reference's callers do
  * between the QuantizedLinear forwards of a block at decode (one new token per sequence), as four launches instead of
- * ~45 framework launches; bf16 tensors, fp32 arithmetic, the step's position read from DEVICE memory so that a CUDA
+ * ~45 framework launches; bf16 tensors, fp32 arithmetic, the step's positions read from DEVICE memory so that a CUDA
  * graph can replay the step.
- *   gbxq_rope_cache       q[B,Hq,D] rotated in place, k[B,Hkv,D] rotated into k_cache[B,Hkv,max_len,D] at *pos, v copied
- *                         into v_cache at *pos (mx.fast.rope traditional=False + cache.update_and_fetch,
- *                         gbx_lm/models/qllama.py:83-88); inv_freq f32 [D/2] already carries the rope scaling
- *   gbxq_decode_attention out[B,Hq,D] = softmax(scale * q . K[0..min(*pos, attend_len-1)]) . V, GQA by Hq/Hkv
+ *
+ * Positions: pos_dev is int64 on the device and row b of the batch is at p_b = pos_dev[b * pos_stride].
+ *   pos_stride 0: pos_dev[0] is the position of every row; 1: pos_dev[b] is row b's (B sequences at different
+ *   positions, e.g. prompts of different lengths; no counterpart in the reference, whose generate_step is batch-1).
+ *   Other values return GBXQ_ESHAPE.  At B = 1 the two are the same call, and with all B positions equal stride 1 is
+ *   bitwise stride 0 and enqueues the same launches.
+ * Cache rows: the cache writes take `keep`, the layout of a cache of max_len rows.
+ *   keep < 0: a flat cache; position p goes to row p, and nothing is written for p outside [0, max_len).
+ *   0 <= keep < max_len: a ROTATING cache (the reference's RotatingKVCache, gbx_lm/models/cache.py:280-420): window
+ *     W = max_len rows, of which the first `keep` are attention sinks; position p goes to row
+ *         ring_slot(p) = p                                   if p < W
+ *                      = keep + (p - keep) mod (W - keep)    otherwise
+ *     computed on the device, so a captured decode step wraps without the host.  Below W it is the flat cache's row.
+ *   keep >= max_len: GBXQ_ESHAPE.
+ *   The RoPE angle is the absolute position, q is rotated in place, and nothing outside row b's slot is written (the
+ *   other rows of the batch are unaffected).
+ * The attention calls attend keys [0, min(p_b, attend_len-1)] of row b's cache.  Over a ring, with max_len = W and
+ * attend_len = min(tokens so far, W) (a replayed graph: W), those rows are exactly the ring's contents -- the sinks and
+ * the last W - keep positions.  Softmax does not depend on the order of the rows, so the result is the windowed
+ * attention up to the order of summation.
+ *
+ *   gbxq_rope_cache       q[B,Hq,D] rotated in place, k[B,Hkv,D] rotated into k_cache[B,Hkv,max_len,D] and v copied
+ *                         into v_cache, each at row b's cache row (mx.fast.rope traditional=False +
+ *                         cache.update_and_fetch, gbx_lm/models/qllama.py:83-88); inv_freq f32 [D/2] already carries
+ *                         the rope scaling
+ *   gbxq_decode_attention out[B,Hq,D] = softmax(scale * q . K[0..min(p_b, attend_len-1)]) . V, GQA by Hq/Hkv
  *                         (scaled_dot_product_attention, qllama.py:90-93); D = 64 or 128
  *   gbxq_add_rmsnorm      h = x + r (r NULL: h = x), y = RMSNorm(h) * w; h_out may be NULL or alias x
  *                         (residual + nn.RMSNorm, qllama.py:137-141)
  *   gbxq_silu_mul         out = silu(gate) * up (qllama.py:115), n elements, n % 8 == 0
  */
-int gbxq_rope_cache(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev,
-                    void* k_cache, void* v_cache, int B, int Hq, int Hkv, int D, int64_t max_len, void* stream);
-int gbxq_decode_attention(const void* q, const void* k_cache, const void* v_cache, const int64_t* pos_dev, void* out,
-                          int B, int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale, void* stream);
+int gbxq_rope_cache(void* q, const void* k, const void* v, const int64_t* pos_dev, int pos_stride,
+                    const float* inv_freq_dev, void* k_cache, void* v_cache, int B, int Hq, int Hkv, int D,
+                    int64_t max_len, int64_t keep, void* stream);
+int gbxq_decode_attention(const void* q, const void* k_cache, const void* v_cache, const int64_t* pos_dev,
+                          int pos_stride, void* out, int B, int Hq, int Hkv, int D, int64_t max_len,
+                          int64_t attend_len, float scale, void* stream);
 int gbxq_add_rmsnorm(const void* x, const void* r, const void* w, float eps, void* h_out, void* y_out, int64_t rows,
                      int H, void* stream);
-
-/*
- * The cache writes of a ROTATING KV cache (the reference's RotatingKVCache, gbx_lm/models/cache.py:280-420): window W =
- * max_len rows, of which the first `keep` are attention sinks, 0 <= keep < max_len (else GBXQ_ESHAPE).  Absolute
- * position p is stored in row
- *     ring_slot(p) = p                                   if p < W
- *                  = keep + (p - keep) mod (W - keep)    otherwise
- * gbxq_rope_cache_ring / gbxq_rope_cache_quantized_ring are gbxq_rope_cache / gbxq_rope_cache_quantized with k and v
- * written to row ring_slot(*pos) instead of row *pos: the RoPE angle is the absolute *pos, q is rotated in place, and
- * nothing else is written.  For *pos < max_len they are bitwise the flat entry points.  The slot is computed on the
- * device, so a captured decode step wraps without the host.
- * No attention entry point of its own: gbxq_decode_attention and gbxq_decode_attention_quantized attend rows
- * [0, min(*pos, attend_len-1)], and with max_len = W and attend_len = min(tokens so far, W) (a replayed graph: W) those
- * rows are exactly the ring's contents -- the sinks and the last W - keep positions.  Softmax does not depend on the
- * order of the rows, so the result is the windowed attention up to the order of summation.
- */
-int gbxq_rope_cache_ring(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev,
-                         void* k_cache, void* v_cache, int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep,
-                         void* stream);
-
-/*
- * Per-row positions: a decode step of B sequences that sit at different positions (prompts of different lengths).
- * pos_dev is int64 [B] on the device, row b at position pos_dev[b]; everything else is as in the entry point each
- * generalises, row by row.
- *   gbxq_rope_cache_rows             gbxq_rope_cache / gbxq_rope_cache_ring with row b rotated at pos_dev[b] and its k / v
- *                                    written to row pos_dev[b] (keep < 0: a flat cache) or ring_slot(pos_dev[b])
- *                                    (0 <= keep < max_len: a rotating cache); keep >= max_len: GBXQ_ESHAPE.  A row whose
- *                                    position is outside the cache writes nothing; the other rows are unaffected.
- *   gbxq_decode_attention_rows       gbxq_decode_attention with row b attending keys [0, min(pos_dev[b], attend_len-1)]
- *                                    of its own cache.
- * With all B positions equal they are bitwise the shared-position entry points, and they enqueue the same launches.
- * The quantized pair, gbxq_rope_cache_quantized_rows and gbxq_decode_attention_quantized_rows, is declared below.
- */
-int gbxq_rope_cache_rows(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev,
-                         void* k_cache, void* v_cache, int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep,
-                         void* stream);
-int gbxq_decode_attention_rows(const void* q, const void* k_cache, const void* v_cache, const int64_t* pos_dev, void* out,
-                               int B, int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale,
-                               void* stream);
 int gbxq_silu_mul(const void* gate, const void* up, void* out, int64_t n, void* stream);
 
 /*
@@ -304,50 +289,34 @@ int gbxq_silu_mul(const void* gate, const void* up, void* out, int64_t n, void* 
  * gbx_lm/models/base.py:65-98).  Each side of the cache is a triple in the layout of gbxq_quantize, position-major:
  *     codes uint32 [B, Hkv, max_len, D*bits/32],  scales / biases bf16 [B, Hkv, max_len, D/group_size]
  * bits in {2,3,4,6,8}, group_size in {32,64,128} with group_size <= D, D in {64, 128}, Hq/Hkv <= 8; other shapes return
- * GBXQ_EUNSUPPORTED (nothing enqueued).
+ * GBXQ_EUNSUPPORTED (nothing enqueued).  pos_dev / pos_stride and keep are as for gbxq_rope_cache /
+ * gbxq_decode_attention above.
  *   gbxq_rope_cache_quantized       q rotated in place as gbxq_rope_cache does; k rotated and v copied, each quantized
- *                                   into row *pos of its triple.  Codes, scales and biases are bit-identical to
- *                                   gbxq_rope_cache into a bf16 row followed by gbxq_quantize_rows of that row.  Nothing
- *                                   outside row *pos is written (nothing at all if *pos is outside [0, max_len)).
- *   gbxq_decode_attention_quantized out[B,Hq,D] = softmax(scale * q . K[0..min(*pos, attend_len-1)]) . V over the
+ *                                   into row b's cache row of its triple.  Codes, scales and biases are bit-identical
+ *                                   to gbxq_rope_cache into a bf16 row followed by gbxq_quantize_rows of that row.
+ *                                   Nothing outside that row is written (nothing at all for a position outside a flat
+ *                                   cache).
+ *   gbxq_decode_attention_quantized out[B,Hq,D] = softmax(scale * q . K[0..min(p_b, attend_len-1)]) . V over the
  *                                   triples, fp32 inside.  Keys are split into chunks of 256 positions, one CTA per
  *                                   (chunk, kv head, batch) for all query heads of the group, and the partial results
- *                                   are combined by a second launch in chunk order: the result does not depend on
- *                                   attend_len or max_len (bitwise), and there is no context limit.  `workspace` holds
- *                                   the partials: at least gbxq_decode_attention_quantized_workspace_bytes(B, Hq, Hkv, D,
- *                                   attend_len) bytes, 16-byte aligned, no initialisation needed; a workspace serves
- *                                   the calls of one stream one after another.  Returns 0 from the size query for
- *                                   unsupported arguments.
+ *                                   are combined by a second launch in chunk order; the chunks past a row's own
+ *                                   position are empty partials.  So each row's result does not depend on attend_len,
+ *                                   max_len or the other rows (bitwise), and there is no context limit.  `workspace`
+ *                                   holds the partials: at least gbxq_decode_attention_quantized_workspace_bytes(B, Hq,
+ *                                   Hkv, D, attend_len) bytes, 16-byte aligned, no initialisation needed; a workspace
+ *                                   serves the calls of one stream one after another.  Returns 0 from the size query
+ *                                   for unsupported arguments.
  */
-int gbxq_rope_cache_quantized(void* q, const void* k, const void* v, const int64_t* pos_dev, const float* inv_freq_dev,
-                              uint32_t* k_codes, void* k_scales, void* k_biases, uint32_t* v_codes, void* v_scales,
-                              void* v_biases, int B, int Hq, int Hkv, int D, int64_t max_len, int bits, int group_size,
-                              void* stream);
-/* gbxq_rope_cache_quantized writing row ring_slot(*pos) of a rotating cache (see gbxq_rope_cache_ring). */
-int gbxq_rope_cache_quantized_ring(void* q, const void* k, const void* v, const int64_t* pos_dev,
-                                   const float* inv_freq_dev, uint32_t* k_codes, void* k_scales, void* k_biases,
-                                   uint32_t* v_codes, void* v_scales, void* v_biases, int B, int Hq, int Hkv, int D,
-                                   int64_t max_len, int64_t keep, int bits, int group_size, void* stream);
+int gbxq_rope_cache_quantized(void* q, const void* k, const void* v, const int64_t* pos_dev, int pos_stride,
+                              const float* inv_freq_dev, uint32_t* k_codes, void* k_scales, void* k_biases,
+                              uint32_t* v_codes, void* v_scales, void* v_biases, int B, int Hq, int Hkv, int D,
+                              int64_t max_len, int64_t keep, int bits, int group_size, void* stream);
 size_t gbxq_decode_attention_quantized_workspace_bytes(int B, int Hq, int Hkv, int D, int64_t attend_len);
-int gbxq_decode_attention_quantized(const void* q, const uint32_t* k_codes, const void* k_scales, const void* k_biases,
-                                    const uint32_t* v_codes, const void* v_scales, const void* v_biases,
-                                    const int64_t* pos_dev, void* out, int B, int Hq, int Hkv, int D, int64_t max_len,
-                                    int64_t attend_len, float scale, int bits, int group_size, void* workspace,
-                                    size_t workspace_bytes, void* stream);
-/* The per-row forms of the quantized pair (pos_dev int64 [B], one position per row; see gbxq_rope_cache_rows):
- * gbxq_rope_cache_quantized_rows takes keep as gbxq_rope_cache_rows does (< 0 flat, [0, max_len) a ring, else
- * GBXQ_ESHAPE).  In gbxq_decode_attention_quantized_rows, the chunks past a row's own position are empty partials, so
- * each row's result is bitwise independent of attend_len and of the other rows; the workspace is sized as for
- * gbxq_decode_attention_quantized. */
-int gbxq_rope_cache_quantized_rows(void* q, const void* k, const void* v, const int64_t* pos_dev,
-                                   const float* inv_freq_dev, uint32_t* k_codes, void* k_scales, void* k_biases,
-                                   uint32_t* v_codes, void* v_scales, void* v_biases, int B, int Hq, int Hkv, int D,
-                                   int64_t max_len, int64_t keep, int bits, int group_size, void* stream);
-int gbxq_decode_attention_quantized_rows(const void* q, const uint32_t* k_codes, const void* k_scales,
-                                         const void* k_biases, const uint32_t* v_codes, const void* v_scales,
-                                         const void* v_biases, const int64_t* pos_dev, void* out, int B, int Hq, int Hkv,
-                                         int D, int64_t max_len, int64_t attend_len, float scale, int bits,
-                                         int group_size, void* workspace, size_t workspace_bytes, void* stream);
+int gbxq_decode_attention_quantized(const void* q, const uint32_t* k_codes, const void* k_scales,
+                                    const void* k_biases, const uint32_t* v_codes, const void* v_scales,
+                                    const void* v_biases, const int64_t* pos_dev, int pos_stride, void* out, int B,
+                                    int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale,
+                                    int bits, int group_size, void* workspace, size_t workspace_bytes, void* stream);
 
 /*
  * Vocabulary projection of the decode step (SURVEY.md 8f rank 1): y[M,V] = x[M,K] . weight[V,K]^T with UNQUANTIZED bf16

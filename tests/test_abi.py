@@ -17,7 +17,7 @@ def _declared_functions():
     return sorted(set(re.findall(r"\b(gbxq_[a-z_0-9]+)\s*\(", hdr)))
 
 
-def test_header_symbols_exported():
+def test_header_symbols_exported_at_abi_version_2():
     from gbx_lm_b200 import _lib
 
     lib = _lib.get()
@@ -26,7 +26,7 @@ def test_header_symbols_exported():
     for n in names:
         assert hasattr(lib, n), f"{n} declared in include/gbxq.h but not exported"
     assert sorted(_lib.EXPORTS) == names
-    assert lib.gbxq_abi_version() == 1
+    assert lib.gbxq_abi_version() == 2
 
 
 def test_no_torch_types_in_abi():

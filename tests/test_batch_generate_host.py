@@ -1,7 +1,7 @@
-"""CPU tests of batched generation with per-row prompt lengths: the four per-row entry points of libgbxq refuse bad
-arguments with the documented status codes before touching CUDA, and `utils.batch_generate` checks its arguments, pads
-the prompts on the right, reads each row's first token at its own last column and steps each row at its own position
-(a stub model stands in for qllama.Model)."""
+"""CPU tests of batched generation with per-row prompt lengths: the four decode-step entry points of libgbxq refuse bad
+arguments with the documented status codes before touching CUDA, at both position strides, and `utils.batch_generate`
+checks its arguments, pads the prompts on the right, reads each row's first token at its own last column and steps each
+row at its own position (a stub model stands in for qllama.Model)."""
 import ctypes
 from types import SimpleNamespace
 
@@ -14,45 +14,55 @@ from oracle import mlx_affine as A
 ESHAPE, ENULL, EINVAL_BITS, EINVAL_GROUP, EWORKSPACE, EUNSUPPORTED = -3, -6, -1, -2, -8, -9
 
 
-def test_rows_abi_validation_without_gpu():
-    from gbx_lm_b200 import _lib
-
-    lib = _lib.get()
+def _decode_entries(lib, stride):
+    """gbxq_rope_cache, gbxq_rope_cache_quantized, gbxq_decode_attention and gbxq_decode_attention_quantized at one
+    pos_stride; every other argument is valid unless a keyword overrides it."""
     p = ctypes.c_void_p(256)  # never dereferenced: validation fails first
 
     def rope(keep=-1, max_len=64, B=2, Hq=8, Hkv=2, D=128, null=False):
-        return lib.gbxq_rope_cache_rows(None if null else p, p, p, p, p, p, p, B, Hq, Hkv, D, max_len, keep, None)
+        return lib.gbxq_rope_cache(None if null else p, p, p, p, stride, p, p, p, B, Hq, Hkv, D, max_len, keep, None)
 
     def qrope(keep=-1, max_len=64, B=2, Hq=8, Hkv=2, D=128, bits=4, gs=64, null=False):
-        return lib.gbxq_rope_cache_quantized_rows(p, p, p, None if null else p, p, p, p, p, p, p, p, B, Hq, Hkv, D, max_len,
-                                                  keep, bits, gs, None)
+        return lib.gbxq_rope_cache_quantized(p, p, p, None if null else p, stride, p, p, p, p, p, p, p, B, Hq, Hkv, D,
+                                             max_len, keep, bits, gs, None)
 
     def attn(attend_len=64, max_len=64, B=2, Hq=8, Hkv=2, D=128, null=False):
-        return lib.gbxq_decode_attention_rows(p, p, p, None if null else p, p, B, Hq, Hkv, D, max_len, attend_len, 0.1,
-                                              None)
+        return lib.gbxq_decode_attention(p, p, p, None if null else p, stride, p, B, Hq, Hkv, D, max_len, attend_len, 0.1,
+                                         None)
 
     def qattn(attend_len=64, max_len=64, B=2, Hq=8, Hkv=2, D=128, bits=4, gs=64, ws=1 << 30, null=False):
-        return lib.gbxq_decode_attention_quantized_rows(p, p, p, p, p, p, p, None if null else p, p, B, Hq, Hkv, D, max_len,
-                                                        attend_len, 0.1, bits, gs, p, ws, None)
+        return lib.gbxq_decode_attention_quantized(p, p, p, p, p, p, p, None if null else p, stride, p, B, Hq, Hkv, D,
+                                                   max_len, attend_len, 0.1, bits, gs, p, ws, None)
 
-    for f in (rope, qrope):
-        assert f(keep=64) == ESHAPE and f(keep=100) == ESHAPE and f(keep=0, max_len=0) == ESHAPE  # keep >= max_len
-        assert f(null=True) == ENULL and f(keep=4, null=True) == ENULL  # flat and ring
-        assert f(B=0) == ESHAPE
-    assert rope(D=63) == ESHAPE
-    assert qrope(bits=5) == EINVAL_BITS and qrope(gs=16) == EINVAL_GROUP
-    assert qrope(D=96) == EUNSUPPORTED and qrope(Hq=16, Hkv=1) == EUNSUPPORTED and qrope(D=64, gs=128) == EUNSUPPORTED
-    assert qrope(Hq=6, Hkv=4) == ESHAPE
-    assert attn(null=True) == ENULL
-    assert attn(attend_len=65) == ESHAPE and attn(attend_len=0) == ESHAPE and attn(Hq=6, Hkv=4) == ESHAPE
-    assert attn(B=0) == ESHAPE
-    assert attn(attend_len=49153, max_len=49153) == EUNSUPPORTED  # one float of shared memory per visible key
-    assert qattn(null=True) == ENULL
-    assert qattn(attend_len=65) == ESHAPE and qattn(Hq=6, Hkv=4) == ESHAPE
-    assert qattn(D=96) == EUNSUPPORTED and qattn(Hq=16, Hkv=1) == EUNSUPPORTED
-    assert qattn(bits=7) == EINVAL_BITS
-    need = lib.gbxq_decode_attention_quantized_workspace_bytes(2, 8, 2, 128, 64)
-    assert need > 0 and qattn(ws=need - 1) == EWORKSPACE
+    return rope, qrope, attn, qattn
+
+
+def test_decode_step_abi_validation_without_gpu():
+    from gbx_lm_b200 import _lib
+
+    lib = _lib.get()
+    for stride in (0, 1):  # one position for every row, one per row
+        rope, qrope, attn, qattn = _decode_entries(lib, stride)
+        for f in (rope, qrope):
+            assert f(keep=64) == ESHAPE and f(keep=100) == ESHAPE and f(keep=0, max_len=0) == ESHAPE  # keep >= max_len
+            assert f(null=True) == ENULL and f(keep=4, null=True) == ENULL  # flat and ring
+            assert f(B=0) == ESHAPE
+        assert rope(D=63) == ESHAPE
+        assert qrope(bits=5) == EINVAL_BITS and qrope(gs=16) == EINVAL_GROUP
+        assert qrope(D=96) == EUNSUPPORTED and qrope(Hq=16, Hkv=1) == EUNSUPPORTED and qrope(D=64, gs=128) == EUNSUPPORTED
+        assert qrope(Hq=6, Hkv=4) == ESHAPE
+        assert attn(null=True) == ENULL
+        assert attn(attend_len=65) == ESHAPE and attn(attend_len=0) == ESHAPE and attn(Hq=6, Hkv=4) == ESHAPE
+        assert attn(B=0) == ESHAPE
+        assert attn(attend_len=49153, max_len=49153) == EUNSUPPORTED  # one float of shared memory per visible key
+        assert qattn(null=True) == ENULL
+        assert qattn(attend_len=65) == ESHAPE and qattn(Hq=6, Hkv=4) == ESHAPE
+        assert qattn(D=96) == EUNSUPPORTED and qattn(Hq=16, Hkv=1) == EUNSUPPORTED
+        assert qattn(bits=7) == EINVAL_BITS
+        need = lib.gbxq_decode_attention_quantized_workspace_bytes(2, 8, 2, 128, 64)
+        assert need > 0 and qattn(ws=need - 1) == EWORKSPACE
+    for stride in (-1, 2):  # neither
+        assert [f() for f in _decode_entries(lib, stride)] == [ESHAPE] * 4
 
 
 VOCAB = 64

@@ -1,9 +1,9 @@
-"""GPU tests of batched generation with per-row prompt lengths: the per-row (`_rows`) cache-write and attention entry
-points against the shared-position ones (bitwise, with equal positions) and against B = 1 calls row by row (bitwise,
-with distinct positions; nothing else written), `batch_generate` against the shared-position path, each row's
-independence of the pads and of the other rows at batches that reach every matmul kernel family, the fp32 reference
-(flat, 8-bit and wrapping rotating caches), graph / eager / in-decode conversion, fused against unfused per-row decode,
-and the launches of a ragged decode step."""
+"""GPU tests of batched generation with per-row prompt lengths: the cache-write and attention ops with per-row
+positions (pos_stride 1) against one shared position (pos_stride 0; bitwise, with equal positions) and against B = 1
+calls row by row (bitwise, with distinct positions; nothing else written), `batch_generate` against the shared-position
+path, each row's independence of the pads and of the other rows at batches that reach every matmul kernel family, the
+fp32 reference (flat, 8-bit and wrapping rotating caches), graph / eager / in-decode conversion, fused against unfused
+per-row decode, and the launches of a ragged decode step."""
 import copy
 
 import pytest

@@ -61,6 +61,32 @@ def test_decode_attention_matches_sdpa(cuda_device, D, Hq, Hkv, pos):
     assert (got2 - want).abs().max() <= 1e-2 * want.abs().max() + 1e-3
 
 
+@pytest.mark.parametrize("op", ("rope_cache", "decode_attention", "rope_cache_quantized", "decode_attention_quantized"))
+def test_ops_refuse_positions_the_kernels_cannot_read(cuda_device, op):
+    """The kernels read `position` as int64 in device memory: an int32 [1] or a host int64 [1] position is a ValueError
+    before anything is launched."""
+    B, Hq, Hkv, D, max_len, bits, gs = 2, 8, 2, 128, 64, 4, 64
+    bf = dict(dtype=torch.bfloat16, device=cuda_device)
+    q, k = torch.zeros((B, Hq, D), **bf), torch.zeros((B, Hkv, D), **bf)
+    kc = torch.zeros((B, Hkv, max_len, D), **bf)
+    inv = torch.ones(D // 2, dtype=torch.float32, device=cuda_device)
+    c3 = (torch.zeros((B, Hkv, max_len, D * bits // 32), dtype=torch.int32, device=cuda_device).view(torch.uint32),
+          torch.zeros((B, Hkv, max_len, D // gs), **bf), torch.zeros((B, Hkv, max_len, D // gs), **bf))
+    call = {
+        "rope_cache": lambda p: ops.rope_cache(q, k, k, p, inv, kc, kc),
+        "decode_attention": lambda p: ops.decode_attention(q, kc, kc, p, 0.1),
+        "rope_cache_quantized": lambda p: ops.rope_cache_quantized(q, k, k, p, inv, c3, c3, gs, bits),
+        "decode_attention_quantized": lambda p: ops.decode_attention_quantized(q, c3, c3, p, 0.1, gs, bits),
+    }[op]
+    call(torch.zeros(1, dtype=torch.int64, device=cuda_device))  # the same call with a valid position launches
+    for bad in (torch.zeros(1, dtype=torch.int32, device=cuda_device), torch.zeros(1, dtype=torch.int64)):
+        n0 = ops.launch_count()
+        with pytest.raises(ValueError, match=f"{op}: position"):
+            call(bad)
+        assert ops.launch_count() == n0, (op, bad.dtype, bad.device)
+    torch.cuda.synchronize()
+
+
 @pytest.mark.parametrize("H", (256, 4096, 8192))
 def test_add_rmsnorm_and_silu_mul_match_torch(cuda_device, H):
     g = torch.Generator(device=cuda_device).manual_seed(H)

@@ -11,40 +11,41 @@ import torch
 from oracle import mlx_affine as A
 
 
-def _rope_q(lib, **kw):
+def _rope_q(lib, stride=0, **kw):
     p = ctypes.c_void_p(256)  # never dereferenced: validation fails first
     a = dict(B=1, Hq=8, Hkv=2, D=128, max_len=64, bits=4, gs=64)
     a.update(kw)
-    return lib.gbxq_rope_cache_quantized(p, p, p, p, p, p, p, p, p, p, p, a["B"], a["Hq"], a["Hkv"], a["D"], a["max_len"],
-                                         a["bits"], a["gs"], None)
+    return lib.gbxq_rope_cache_quantized(p, p, p, p, stride, p, p, p, p, p, p, p, a["B"], a["Hq"], a["Hkv"], a["D"],
+                                         a["max_len"], -1, a["bits"], a["gs"], None)
 
 
-def _attn_q(lib, ws=None, ws_bytes=1 << 30, **kw):
+def _attn_q(lib, stride=0, ws=None, ws_bytes=1 << 30, **kw):
     p = ctypes.c_void_p(256)
     a = dict(B=1, Hq=8, Hkv=2, D=128, max_len=64, attend_len=64, bits=4, gs=64)
     a.update(kw)
-    return lib.gbxq_decode_attention_quantized(p, p, p, p, p, p, p, p, p, a["B"], a["Hq"], a["Hkv"], a["D"], a["max_len"],
-                                               a["attend_len"], 0.1, a["bits"], a["gs"], ws if ws is not None else p,
-                                               ws_bytes, None)
+    return lib.gbxq_decode_attention_quantized(p, p, p, p, p, p, p, p, stride, p, a["B"], a["Hq"], a["Hkv"], a["D"],
+                                               a["max_len"], a["attend_len"], 0.1, a["bits"], a["gs"],
+                                               ws if ws is not None else p, ws_bytes, None)
 
 
-def test_quantized_decode_abi_validation_without_gpu():
+def test_quantized_decode_abi_validation_at_both_strides_without_gpu():
     from gbx_lm_b200 import _lib
 
     lib = _lib.get()
-    for f in (_rope_q, _attn_q):
-        assert f(lib, bits=5) == -1 and f(lib, bits=1) == -1 and f(lib, bits=16) == -1
-        assert f(lib, gs=16) == -2 and f(lib, gs=256) == -2
-        assert f(lib, D=64, gs=128) == -9                # group larger than the head
-        assert f(lib, D=96, gs=32) == -9 and f(lib, D=256) == -9
-        assert f(lib, Hq=6, Hkv=4) == -3                 # Hq % Hkv
-        assert f(lib, Hq=32, Hkv=2) == -9                # GQA ratio above 8
-        assert f(lib, B=0) == -3 and f(lib, Hkv=0) == -3 and f(lib, max_len=0) == -3
-    assert _attn_q(lib, attend_len=0) == -3 and _attn_q(lib, attend_len=65) == -3
-    assert _attn_q(lib, ws_bytes=16) == -8               # workspace too small
-    assert _attn_q(lib, ws=ctypes.c_void_p(264)) == -5   # workspace not 16-byte aligned
-    assert lib.gbxq_decode_attention_quantized(None, None, None, None, None, None, None, None, None, 1, 8, 2, 128, 64, 64,
-                                               0.1, 4, 64, None, 0, None) == -6
+    for s in (0, 1):  # at B = 1 the shared and the per-row position are the same call
+        for f in (_rope_q, _attn_q):
+            assert f(lib, s, bits=5) == -1 and f(lib, s, bits=1) == -1 and f(lib, s, bits=16) == -1
+            assert f(lib, s, gs=16) == -2 and f(lib, s, gs=256) == -2
+            assert f(lib, s, D=64, gs=128) == -9                # group larger than the head
+            assert f(lib, s, D=96, gs=32) == -9 and f(lib, s, D=256) == -9
+            assert f(lib, s, Hq=6, Hkv=4) == -3                 # Hq % Hkv
+            assert f(lib, s, Hq=32, Hkv=2) == -9                # GQA ratio above 8
+            assert f(lib, s, B=0) == -3 and f(lib, s, Hkv=0) == -3 and f(lib, s, max_len=0) == -3
+        assert _attn_q(lib, s, attend_len=0) == -3 and _attn_q(lib, s, attend_len=65) == -3
+        assert _attn_q(lib, s, ws_bytes=16) == -8               # workspace too small
+        assert _attn_q(lib, s, ws=ctypes.c_void_p(264)) == -5   # workspace not 16-byte aligned
+        assert lib.gbxq_decode_attention_quantized(None, None, None, None, None, None, None, None, s, None, 1, 8, 2, 128,
+                                                   64, 64, 0.1, 4, 64, None, 0, None) == -6
 
 
 def test_quantized_decode_workspace_query():

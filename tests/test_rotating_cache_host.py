@@ -109,19 +109,37 @@ def test_rotating_cache_validation():
     assert ops._check_keep(None, 8, "rope_cache") is None and ops._check_keep(0, 8, "rope_cache") == 0
 
 
-def test_ring_abi_validation_without_gpu():
-    """The ring entry points refuse keep outside [0, max_len) with GBXQ_ESHAPE before touching CUDA."""
+def test_position_stride_rule():
+    """The position of the four decode-step ops: a contiguous int64 [1] (pos_stride 0, shared by the rows) or [B]
+    (pos_stride 1) on the device of q; anything else is a ValueError."""
+    from gbx_lm_b200 import ops
+
+    q = torch.zeros((3, 8, 64), dtype=torch.bfloat16)
+    i64 = lambda *shape: torch.zeros(shape, dtype=torch.int64)  # noqa: E731
+    assert ops._pos_stride(i64(1), 3, q, "rope_cache") == 0
+    assert ops._pos_stride(i64(3), 3, q, "rope_cache") == 1
+    assert ops._pos_stride(i64(1), 1, q[:1], "rope_cache") == 0
+    for bad in (i64(2), i64(4), i64(3, 1), i64(), torch.zeros(1, dtype=torch.int32), torch.zeros(3, dtype=torch.int32),
+                torch.zeros(3, dtype=torch.float32), i64(6)[::2]):
+        with pytest.raises(ValueError, match="rope_cache: position"):
+            ops._pos_stride(bad, 3, q, "rope_cache")
+
+
+def test_keep_abi_validation_without_gpu():
+    """The cache writes refuse keep >= max_len with GBXQ_ESHAPE before touching CUDA."""
     from gbx_lm_b200 import _lib
 
     lib = _lib.get()
     p = ctypes.c_void_p(256)  # never dereferenced: validation fails first
-    ring = lambda keep, max_len=64: lib.gbxq_rope_cache_ring(p, p, p, p, p, p, p, 1, 8, 2, 128, max_len, keep, None)
-    qring = lambda keep, max_len=64, bits=4: lib.gbxq_rope_cache_quantized_ring(
-        p, p, p, p, p, p, p, p, p, p, p, 1, 8, 2, 128, max_len, keep, bits, 64, None)
-    for f in (ring, qring):
-        assert f(64) == -3 and f(-1) == -3 and f(100) == -3 and f(0, max_len=0) == -3
-    assert qring(4, bits=5) == -1
-    assert lib.gbxq_rope_cache_ring(None, p, p, p, p, p, p, 1, 8, 2, 128, 64, 4, None) == -6
+    for stride in (0, 1):  # at B = 1 the shared and the per-row position are the same call
+        ring = lambda keep, max_len=64: lib.gbxq_rope_cache(p, p, p, p, stride, p, p, p, 1, 8, 2, 128, max_len, keep,
+                                                            None)
+        qring = lambda keep, max_len=64, bits=4: lib.gbxq_rope_cache_quantized(
+            p, p, p, p, stride, p, p, p, p, p, p, p, 1, 8, 2, 128, max_len, keep, bits, 64, None)
+        for f in (ring, qring):
+            assert f(64) == -3 and f(100) == -3 and f(0, max_len=0) == -3
+        assert qring(4, bits=5) == -1
+        assert lib.gbxq_rope_cache(None, p, p, p, stride, p, p, p, 1, 8, 2, 128, 64, 4, None) == -6
 
 
 def _oracle_quantize(x, group_size, bits):
