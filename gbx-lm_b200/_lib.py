@@ -42,6 +42,10 @@ EXPORTS = (
     "gbxq_rope_cache_quantized",
     "gbxq_decode_attention_quantized",
     "gbxq_decode_attention_quantized_workspace_bytes",
+    "gbxq_rope_cache_multi",
+    "gbxq_decode_attention_multi",
+    "gbxq_rope_cache_quantized_multi",
+    "gbxq_decode_attention_quantized_multi",
     "gbxq_add_rmsnorm",
     "gbxq_silu_mul",
     "gbxq_head_gemv",
@@ -160,6 +164,16 @@ def get() -> ctypes.CDLL:
     lib.gbxq_decode_attention_quantized_workspace_bytes.argtypes = [ci, ci, ci, ci, i64]
     lib.gbxq_decode_attention_quantized.restype = ci
     lib.gbxq_decode_attention_quantized.argtypes = [vp] * 8 + [ci, vp, ci, ci, ci, ci, i64, i64, cf, ci, ci, vp, sz, vp]
+    # the `_multi` forms: T after B, no keep
+    lib.gbxq_rope_cache_multi.restype = ci
+    lib.gbxq_rope_cache_multi.argtypes = [vp, vp, vp, vp, ci, vp, vp, vp, ci, ci, ci, ci, ci, i64, vp]
+    lib.gbxq_decode_attention_multi.restype = ci
+    lib.gbxq_decode_attention_multi.argtypes = [vp, vp, vp, vp, ci, vp, ci, ci, ci, ci, ci, i64, i64, cf, vp]
+    lib.gbxq_rope_cache_quantized_multi.restype = ci
+    lib.gbxq_rope_cache_quantized_multi.argtypes = [vp] * 4 + [ci] + [vp] * 7 + [ci, ci, ci, ci, ci, i64, ci, ci, vp]
+    lib.gbxq_decode_attention_quantized_multi.restype = ci
+    lib.gbxq_decode_attention_quantized_multi.argtypes = ([vp] * 8 + [ci, vp, ci, ci, ci, ci, ci, i64, i64, cf, ci, ci, vp,
+                                                          sz, vp])
     lib.gbxq_add_rmsnorm.restype = ci
     lib.gbxq_add_rmsnorm.argtypes = [vp, vp, vp, cf, vp, vp, i64, ci, vp]
     lib.gbxq_silu_mul.restype = ci

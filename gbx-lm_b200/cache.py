@@ -213,14 +213,19 @@ class StaticKVCache:
         return head_dim in (64, 128) and self.max_len <= DECODE_ATTENTION_MAX_KEYS
 
     def update(self, k: torch.Tensor, v: torch.Tensor, positions: torch.Tensor):
-        """k / v [B, n_kv, L, D] at positions int64 [L], or a decode step's [B, n_kv, 1, D] at per-row positions [B, 1]."""
+        """k / v [B, n_kv, L, D] at positions int64 [L] shared by the rows, or at per-row positions [B, L]."""
         if positions.dim() == 2:
-            rows = torch.arange(k.shape[0], device=k.device)
-            self.keys[rows, :, positions[:, 0]] = k[:, :, 0]
-            self.values[rows, :, positions[:, 0]] = v[:, :, 0]
+            rows = torch.arange(k.shape[0], device=k.device)[:, None]
+            self.keys[rows, :, positions] = k.transpose(1, 2)  # the indexed view is [B, L, n_kv, D]
+            self.values[rows, :, positions] = v.transpose(1, 2)
             return
         self.keys.index_copy_(2, positions, k)
         self.values.index_copy_(2, positions, v)
+
+    # the reference's interface: `trim(n)` moves `offset` back by n positions.  The rows past it are dead -- every later
+    # call writes a position before any query can see it
+    is_trimmable = _BlockStore.is_trimmable
+    trim = _BlockStore.trim
 
     def to_quantized(self, group_size: int = 64, bits: int = 4) -> "StaticQuantizedKVCache":
         """The static quantized cache holding these positions (as `KVCache.to_quantized`): the whole buffers are
@@ -276,6 +281,9 @@ class StaticQuantizedKVCache:
 
     def prefix(self, n: int):
         return tuple(t[:, :, :n] for t in self.keys), tuple(t[:, :, :n] for t in self.values)
+
+    is_trimmable = _BlockStore.is_trimmable  # as StaticKVCache
+    trim = _BlockStore.trim
 
 
 # The sink count of the reference's rotating caches: generate_step builds them through make_prompt_cache, which passes
@@ -344,6 +352,13 @@ class _Ring:
         """bool [L, T]: whether the query at positions[i] sees the key at key_positions[j]."""
         j, p = key_positions[None, :], positions[:, None]
         return (j <= p) & ((j < self.keep) | (j > p - (self.max_len - self.keep)))
+
+    def is_trimmable(self) -> bool:
+        """False: a ring that has wrapped has overwritten the rows a rewind would expose (the reference refuses it too)."""
+        return False
+
+    def trim(self, n: int) -> int:
+        raise ValueError("a rotating KV cache cannot be rewound")
 
     def wraps(self) -> bool:
         """Whether the model call that has just advanced `offset` past its positions reaches beyond the window."""
@@ -437,3 +452,16 @@ def maybe_quantize_kv_cache(prompt_cache: list, quantized_kv_start: int, kv_grou
         return
     prompt_cache[:] = [c.to_quantized(group_size=kv_group_size, bits=kv_bits) if isinstance(c, (KVCache, StaticKVCache))
                        else c for c in prompt_cache]
+
+
+def can_trim_prompt_cache(cache: list) -> bool:
+    """gbx_lm/models/cache.py: whether every cache of the list can be rewound."""
+    return all(c.is_trimmable() for c in cache)
+
+
+def trim_prompt_cache(cache: list, num_tokens: int) -> int:
+    """gbx_lm/models/cache.py: moves every cache of the list back by num_tokens positions; returns how many positions
+    were trimmed (0 when the list cannot be rewound)."""
+    if not cache or not can_trim_prompt_cache(cache):
+        return 0
+    return [c.trim(num_tokens) for c in cache][0]

@@ -301,14 +301,28 @@ int gbxq_dequantize(const uint32_t* qweight, const void* scales, const void* bia
 int gbxq_rope_cache(void* q, const void* k, const void* v, const int64_t* pos_dev, int pos_stride,
                     const float* inv_freq_dev, void* k_cache, void* v_cache, int B, int Hq, int Hkv, int D,
                     int64_t max_len, int64_t keep, void* stream) {
-    return launch_rope_cache(q, k, v, pos_dev, pos_stride, inv_freq_dev, k_cache, v_cache, B, Hq, Hkv, D, max_len, keep,
+    return launch_rope_cache(q, k, v, pos_dev, pos_stride, inv_freq_dev, k_cache, v_cache, B, 1, Hq, Hkv, D, max_len, keep,
+                             (cudaStream_t)stream);
+}
+
+int gbxq_rope_cache_multi(void* q, const void* k, const void* v, const int64_t* pos_dev, int pos_stride,
+                          const float* inv_freq_dev, void* k_cache, void* v_cache, int B, int T, int Hq, int Hkv, int D,
+                          int64_t max_len, void* stream) {
+    return launch_rope_cache(q, k, v, pos_dev, pos_stride, inv_freq_dev, k_cache, v_cache, B, T, Hq, Hkv, D, max_len, -1,
                              (cudaStream_t)stream);
 }
 
 int gbxq_decode_attention(const void* q, const void* k_cache, const void* v_cache, const int64_t* pos_dev,
                           int pos_stride, void* out, int B, int Hq, int Hkv, int D, int64_t max_len,
                           int64_t attend_len, float scale, void* stream) {
-    return launch_decode_attention(q, k_cache, v_cache, pos_dev, pos_stride, out, B, Hq, Hkv, D, max_len, attend_len,
+    return launch_decode_attention(q, k_cache, v_cache, pos_dev, pos_stride, out, B, 1, Hq, Hkv, D, max_len, attend_len,
+                                   scale, (cudaStream_t)stream);
+}
+
+int gbxq_decode_attention_multi(const void* q, const void* k_cache, const void* v_cache, const int64_t* pos_dev,
+                                int pos_stride, void* out, int B, int T, int Hq, int Hkv, int D, int64_t max_len,
+                                int64_t attend_len, float scale, void* stream) {
+    return launch_decode_attention(q, k_cache, v_cache, pos_dev, pos_stride, out, B, T, Hq, Hkv, D, max_len, attend_len,
                                    scale, (cudaStream_t)stream);
 }
 
@@ -317,7 +331,16 @@ int gbxq_rope_cache_quantized(void* q, const void* k, const void* v, const int64
                               uint32_t* v_codes, void* v_scales, void* v_biases, int B, int Hq, int Hkv, int D,
                               int64_t max_len, int64_t keep, int bits, int group_size, void* stream) {
     return launch_rope_cache_quantized({q, k, v, pos_dev, pos_stride, inv_freq_dev, k_codes, k_scales, k_biases, v_codes,
-                                        v_scales, v_biases, B, Hq, Hkv, D, max_len, keep, bits, group_size},
+                                        v_scales, v_biases, B, 1, Hq, Hkv, D, max_len, keep, bits, group_size},
+                                       (cudaStream_t)stream);
+}
+
+int gbxq_rope_cache_quantized_multi(void* q, const void* k, const void* v, const int64_t* pos_dev, int pos_stride,
+                                    const float* inv_freq_dev, uint32_t* k_codes, void* k_scales, void* k_biases,
+                                    uint32_t* v_codes, void* v_scales, void* v_biases, int B, int T, int Hq, int Hkv,
+                                    int D, int64_t max_len, int bits, int group_size, void* stream) {
+    return launch_rope_cache_quantized({q, k, v, pos_dev, pos_stride, inv_freq_dev, k_codes, k_scales, k_biases, v_codes,
+                                        v_scales, v_biases, B, T, Hq, Hkv, D, max_len, -1, bits, group_size},
                                        (cudaStream_t)stream);
 }
 
@@ -331,7 +354,19 @@ int gbxq_decode_attention_quantized(const void* q, const uint32_t* k_codes, cons
                                     int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale,
                                     int bits, int group_size, void* workspace, size_t workspace_bytes, void* stream) {
     return launch_decode_attention_quantized({q, k_codes, k_scales, k_biases, v_codes, v_scales, v_biases, pos_dev,
-                                              pos_stride, out, B, Hq, Hkv, D, max_len, attend_len, scale, bits,
+                                              pos_stride, out, B, 1, Hq, Hkv, D, max_len, attend_len, scale, bits,
+                                              group_size, workspace, workspace_bytes},
+                                             (cudaStream_t)stream);
+}
+
+int gbxq_decode_attention_quantized_multi(const void* q, const uint32_t* k_codes, const void* k_scales,
+                                          const void* k_biases, const uint32_t* v_codes, const void* v_scales,
+                                          const void* v_biases, const int64_t* pos_dev, int pos_stride, void* out, int B,
+                                          int T, int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len,
+                                          float scale, int bits, int group_size, void* workspace,
+                                          size_t workspace_bytes, void* stream) {
+    return launch_decode_attention_quantized({q, k_codes, k_scales, k_biases, v_codes, v_scales, v_biases, pos_dev,
+                                              pos_stride, out, B, T, Hq, Hkv, D, max_len, attend_len, scale, bits,
                                               group_size, workspace, workspace_bytes},
                                              (cudaStream_t)stream);
 }

@@ -285,11 +285,15 @@ void stream_debug_patch(void* host_blob, int ncalls, unsigned long long* dbg_dev
 int launch_stream(const gbxq_stream_info* info, const void* blob, void* counters, cudaStream_t st);
 // The decode-step cache write and attention (gbxq_glue.cu / gbxq_qattn.cu).  pos_stride 0: pos[0] is the position of
 // every batch row; 1: pos[b] is row b's; else GBXQ_ESHAPE.  keep < 0: a flat cache; keep in [0, max_len): a rotating
-// cache with keep sink rows (kv_cache_row); else GBXQ_ESHAPE.  The launchers check every argument.
+// cache with keep sink rows (kv_cache_row); else GBXQ_ESHAPE.  T in [1, kMaxBlockTokens]: T consecutive tokens per
+// batch row at pos .. pos + T - 1 (a verify block; the `_multi` entry points pass keep = -1).  The launchers check
+// every argument.
+constexpr int kMaxBlockTokens = 8;
 int launch_rope_cache(void* q, const void* k, const void* v, const int64_t* pos, int pos_stride, const float* inv_freq,
-                      void* kc, void* vc, int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep, cudaStream_t st);
+                      void* kc, void* vc, int B, int T, int Hq, int Hkv, int D, int64_t max_len, int64_t keep,
+                      cudaStream_t st);
 int launch_decode_attention(const void* q, const void* kc, const void* vc, const int64_t* pos, int pos_stride, void* out,
-                            int B, int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale,
+                            int B, int T, int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale,
                             cudaStream_t st);
 // arguments of the quantized-cache decode step (gbxq_qattn.cu): one (codes, scales, biases) triple per side, bf16
 struct QCacheWrite {
@@ -303,7 +307,7 @@ struct QCacheWrite {
     void *ks, *kb;
     uint32_t* vq;
     void *vs, *vb;
-    int B, Hq, Hkv, D;
+    int B, T, Hq, Hkv, D;
     int64_t max_len, keep;
     int bits, gs;
 };
@@ -316,7 +320,7 @@ struct QAttn {
     const int64_t* pos;
     int pos_stride;
     void* out;
-    int B, Hq, Hkv, D;
+    int B, T, Hq, Hkv, D;
     int64_t max_len, attend_len;
     float scale;
     int bits, gs;

@@ -21,23 +21,24 @@ namespace {
 __device__ __forceinline__ float bf(const __nv_bfloat16 v) { return __bfloat162float(v); }
 __device__ __forceinline__ __nv_bfloat16 tobf(float v) { return __float2bfloat16_rn(v); }
 
-// grid (Hq + 2 Hkv, B), block D/2 threads.  Head h < Hq: rotate q in place; Hq <= h < Hq+Hkv: rotate k into the cache;
-// else copy v into the cache.
+// grid (Hq + 2 Hkv, B * T), block D/2 threads.  Row r = b * T + t of q / k / v is token t of batch row b, at position
+// p_b + t (T > 1: a verify block of consecutive tokens; cache row b receives all of them).  Head h < Hq: rotate q in
+// place; Hq <= h < Hq+Hkv: rotate k into the cache; else copy v into the cache.
 __global__ void rope_cache_kernel(__nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ k,
                                   const __nv_bfloat16* __restrict__ v, const int64_t* __restrict__ pos_p,
                                   const float* __restrict__ inv_freq, __nv_bfloat16* __restrict__ kc,
                                   __nv_bfloat16* __restrict__ vc, int Hq, int Hkv, int D, int64_t max_len, int64_t keep,
-                                  int pos_stride) {
-    const int h = blockIdx.x, b = blockIdx.y, i = threadIdx.x, half = D / 2;
+                                  int pos_stride, int T) {
+    const int h = blockIdx.x, r = blockIdx.y, b = r / T, i = threadIdx.x, half = D / 2;
     pdl_wait_then_trigger();
     // the RoPE angle is the absolute position's; k / v go to its cache row.  pos_stride 0: one position for every row
-    const int64_t pos = pos_p[(size_t)b * pos_stride];
+    const int64_t pos = pos_p[(size_t)b * pos_stride] + r % T;
     const int64_t row = kv_cache_row(pos, max_len, keep);
     if (row < 0) return;  // never write outside the cache
     if (h < Hq + Hkv) {
         const bool isq = h < Hq;
-        const __nv_bfloat16* src = isq ? q + ((size_t)b * Hq + h) * D : k + ((size_t)b * Hkv + (h - Hq)) * D;
-        __nv_bfloat16* dst = isq ? q + ((size_t)b * Hq + h) * D : kc + (((size_t)b * Hkv + (h - Hq)) * max_len + row) * D;
+        const __nv_bfloat16* src = isq ? q + ((size_t)r * Hq + h) * D : k + ((size_t)r * Hkv + (h - Hq)) * D;
+        __nv_bfloat16* dst = isq ? q + ((size_t)r * Hq + h) * D : kc + (((size_t)b * Hkv + (h - Hq)) * max_len + row) * D;
         const float ang = __fmul_rn((float)pos, inv_freq[i]);
         const float c = cosf(ang), s = sinf(ang);
         const float x1 = bf(src[i]), x2 = bf(src[i + half]);
@@ -48,14 +49,15 @@ __global__ void rope_cache_kernel(__nv_bfloat16* __restrict__ q, const __nv_bflo
         dst[i + half] = tobf(o2);
     } else {
         const int hv = h - Hq - Hkv;
-        const __nv_bfloat16* src = v + ((size_t)b * Hkv + hv) * D;
+        const __nv_bfloat16* src = v + ((size_t)r * Hkv + hv) * D;
         __nv_bfloat16* dst = vc + (((size_t)b * Hkv + hv) * max_len + row) * D;
         dst[i] = src[i];
         dst[i + half] = src[i + half];
     }
 }
 
-// grid (Hq, B), block 256 threads, dynamic shared memory = one float per visible key.
+// grid (Hq, B * T), block 256 threads, dynamic shared memory = one float per visible key.  Query row r = b * T + t reads
+// cache row b with keys 0 .. p_b + t visible: a verify block's t-th query is exactly a single query at p_b + t.
 // Phase 1: one THREAD per key (keys tid, tid + 256, ...): the 16-byte loads of a key row are independent, so a block
 // has thousands of bytes in flight instead of one dependent load per warp and key (the first version of this kernel
 // walked the keys with an online softmax per warp and was latency-bound: +0.5 ms per 8B token at 100 keys).  Block max /
@@ -67,19 +69,19 @@ __global__ void __launch_bounds__(256) decode_attention_kernel(const __nv_bfloat
                                                                const int64_t* __restrict__ pos_p,
                                                                __nv_bfloat16* __restrict__ out, int Hq, int Hkv,
                                                                int64_t max_len, int64_t attend_len, float scale,
-                                                               int pos_stride) {
+                                                               int pos_stride, int T) {
     constexpr int SPLITS = 256 / D;
     extern __shared__ float sc[];
     __shared__ float qs[D], red[8], part[SPLITS][D];
-    const int h = blockIdx.x, b = blockIdx.y, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int h = blockIdx.x, r = blockIdx.y, b = r / T, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int hk = h / (Hq / Hkv);
     pdl_wait_then_trigger();
-    int64_t last = pos_p[(size_t)b * pos_stride];  // keys 0 .. pos of this row are visible
+    int64_t last = pos_p[(size_t)b * pos_stride] + r % T;  // keys 0 .. pos of this query are visible
     if (last >= attend_len) last = attend_len - 1;
     const int n = (int)(last + 1);
     const __nv_bfloat16* kp = kc + ((size_t)b * Hkv + hk) * max_len * D;
     const __nv_bfloat16* vp = vc + ((size_t)b * Hkv + hk) * max_len * D;
-    if (tid < D) qs[tid] = bf(q[((size_t)b * Hq + h) * D + tid]) * scale;
+    if (tid < D) qs[tid] = bf(q[((size_t)r * Hq + h) * D + tid]) * scale;
     __syncthreads();
     float lmax = -INFINITY;
     for (int j = tid; j < n; j += 256) {
@@ -125,7 +127,7 @@ __global__ void __launch_bounds__(256) decode_attention_kernel(const __nv_bfloat
         float o = 0.f;
 #pragma unroll
         for (int sp = 0; sp < SPLITS; sp++) o += part[sp][tid];
-        out[((size_t)b * Hq + h) * D + tid] = tobf(n > 0 && l > 0.f ? o / l : 0.f);
+        out[((size_t)r * Hq + h) * D + tid] = tobf(n > 0 && l > 0.f ? o / l : 0.f);
     }
 }
 
@@ -198,22 +200,24 @@ __global__ void __launch_bounds__(256) silu_mul_kernel(const __nv_bfloat16* __re
 }  // namespace
 
 int launch_rope_cache(void* q, const void* k, const void* v, const int64_t* pos, int pos_stride, const float* inv_freq,
-                      void* kc, void* vc, int B, int Hq, int Hkv, int D, int64_t max_len, int64_t keep, cudaStream_t st) {
+                      void* kc, void* vc, int B, int T, int Hq, int Hkv, int D, int64_t max_len, int64_t keep, cudaStream_t st) {
     if (!q || !k || !v || !pos || !inv_freq || !kc || !vc) return GBXQ_ENULL;
     if (B < 1 || Hq < 1 || Hkv < 1 || D < 2 || (D & 1) || D / 2 > 1024 || max_len < 1 || keep >= max_len) return GBXQ_ESHAPE;
     if (pos_stride != 0 && pos_stride != 1) return GBXQ_ESHAPE;
-    return launch(rope_cache_kernel, dim3(Hq + 2 * Hkv, B), dim3(D / 2), 0, st, true,
+    if (T < 1 || T > kMaxBlockTokens || (int64_t)B * T > 65535) return GBXQ_ESHAPE;  // B * T: grid.y
+    return launch(rope_cache_kernel, dim3(Hq + 2 * Hkv, B * T), dim3(D / 2), 0, st, true,
         reinterpret_cast<__nv_bfloat16*>(q), reinterpret_cast<const __nv_bfloat16*>(k), reinterpret_cast<const __nv_bfloat16*>(v),
-        pos, inv_freq, reinterpret_cast<__nv_bfloat16*>(kc), reinterpret_cast<__nv_bfloat16*>(vc), Hq, Hkv, D, max_len, keep, pos_stride);
+        pos, inv_freq, reinterpret_cast<__nv_bfloat16*>(kc), reinterpret_cast<__nv_bfloat16*>(vc), Hq, Hkv, D, max_len, keep, pos_stride, T);
 }
 
 int launch_decode_attention(const void* q, const void* kc, const void* vc, const int64_t* pos, int pos_stride, void* out,
-                            int B, int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale,
+                            int B, int T, int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale,
                             cudaStream_t st) {
     if (!q || !kc || !vc || !pos || !out) return GBXQ_ENULL;
     if (B < 1 || Hq < 1 || Hkv < 1 || Hq % Hkv || max_len < 1 || attend_len < 1 || attend_len > max_len) return GBXQ_ESHAPE;
     if (pos_stride != 0 && pos_stride != 1) return GBXQ_ESHAPE;
-    const dim3 grid(Hq, B);
+    if (T < 1 || T > kMaxBlockTokens || (int64_t)B * T > 65535) return GBXQ_ESHAPE;  // B * T: grid.y
+    const dim3 grid(Hq, B * T);
     auto Q = reinterpret_cast<const __nv_bfloat16*>(q);
     auto K = reinterpret_cast<const __nv_bfloat16*>(kc);
     auto V = reinterpret_cast<const __nv_bfloat16*>(vc);
@@ -224,8 +228,8 @@ int launch_decode_attention(const void* q, const void* kc, const void* vc, const
     if (rc == GBXQ_OK) rc = allow_dynamic_smem<decode_attention_kernel<128>>(49152 * 4);
     if (rc != GBXQ_OK) return rc;
     switch (D) {
-        case 64: return launch(decode_attention_kernel<64>, grid, dim3(256), smem, st, true, Q, K, V, pos, O, Hq, Hkv, max_len, attend_len, scale, pos_stride);
-        case 128: return launch(decode_attention_kernel<128>, grid, dim3(256), smem, st, true, Q, K, V, pos, O, Hq, Hkv, max_len, attend_len, scale, pos_stride);
+        case 64: return launch(decode_attention_kernel<64>, grid, dim3(256), smem, st, true, Q, K, V, pos, O, Hq, Hkv, max_len, attend_len, scale, pos_stride, T);
+        case 128: return launch(decode_attention_kernel<128>, grid, dim3(256), smem, st, true, Q, K, V, pos, O, Hq, Hkv, max_len, attend_len, scale, pos_stride, T);
     }
     return GBXQ_EUNSUPPORTED;
 }

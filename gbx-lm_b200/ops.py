@@ -534,23 +534,46 @@ def _pos_stride(position: torch.Tensor, b: int, q: torch.Tensor, where: str) -> 
     return 0 if position.numel() == 1 else 1
 
 
+def _block(q: torch.Tensor, where: str, keep: Optional[int] = None):
+    """(B, T, Hq, D) of q: [B, Hq, D] is one token per row (T = 1, the single-token entry point); [B, T, Hq, D] is a block
+    of T consecutive tokens per row, at positions p_b .. p_b + T - 1 (the `_multi` entry points, flat caches only)."""
+    if q.dim() == 3:
+        return q.shape[0], 1, q.shape[1], q.shape[2]
+    if q.dim() != 4:
+        raise ValueError(f"{where}: q must be [B, Hq, D] or [B, T, Hq, D], got {tuple(q.shape)}")
+    if keep is not None:
+        raise ValueError(f"{where}: a block of T tokens per row needs a flat cache (keep=None)")
+    return tuple(q.shape)
+
+
 def rope_cache(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, position: torch.Tensor, inv_freq: torch.Tensor,
                k_cache: torch.Tensor, v_cache: torch.Tensor, keep: Optional[int] = None) -> torch.Tensor:
     """gbxq_rope_cache: q [B,Hq,D] rotated IN PLACE (returned), k rotated and v copied into the caches [B,Hkv,max_len,D] at
     `position` (int64 device tensor [1]).  Replaces RoPE + cache.update of a decode step (gbx_lm/models/qllama.py:83-88).
     keep = an int: the caches are a rotating window of max_len rows with `keep` sinks, and k / v go to row
-    ring_slot(position) (cache.ring_slot).  position int64 [B]: row b at position[b]."""
+    ring_slot(position) (cache.ring_slot).  position int64 [B]: row b at position[b].
+    q [B,T,Hq,D] (k / v [B,T,Hkv,D]), 1 <= T <= 8: gbxq_rope_cache_multi, token t of row b at position[b] + t, bitwise T
+    single-token calls; flat caches only."""
     _bf16c(q, k, v, k_cache, v_cache)
-    b, hq, d = q.shape
+    b, t, hq, d = _block(q, "rope_cache", keep)
     hkv, max_len = k_cache.shape[1], k_cache.shape[2]
+    kv_shape = (b, hkv, d) if q.dim() == 3 else (b, t, hkv, d)
+    if tuple(k.shape) != kv_shape or tuple(v.shape) != kv_shape:
+        raise ValueError(f"rope_cache: k / v must be {kv_shape}")
     if inv_freq.dtype != torch.float32 or inv_freq.numel() != d // 2:
         raise ValueError("rope_cache: inv_freq float32 [D/2]")
     keep = _check_keep(keep, max_len, "rope_cache")
     stride = _pos_stride(position, b, q, "rope_cache")
+    lib = _lib.get()
     with torch.cuda.device(q.device):
-        rc = _lib.get().gbxq_rope_cache(q.data_ptr(), k.data_ptr(), v.data_ptr(), position.data_ptr(), stride,
-                                        inv_freq.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), b, hq, hkv, d,
-                                        max_len, -1 if keep is None else keep, _stream())
+        if q.dim() == 4:
+            rc = lib.gbxq_rope_cache_multi(q.data_ptr(), k.data_ptr(), v.data_ptr(), position.data_ptr(), stride,
+                                           inv_freq.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), b, t, hq, hkv, d,
+                                           max_len, _stream())
+        else:
+            rc = lib.gbxq_rope_cache(q.data_ptr(), k.data_ptr(), v.data_ptr(), position.data_ptr(), stride,
+                                     inv_freq.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), b, hq, hkv, d,
+                                     max_len, -1 if keep is None else keep, _stream())
     _lib.check(rc, "gbxq_rope_cache")
     return q
 
@@ -559,32 +582,40 @@ def decode_attention(q: torch.Tensor, k_cache: torch.Tensor, v_cache: torch.Tens
                      attend_len: Optional[int] = None) -> torch.Tensor:
     """gbxq_decode_attention: one query row per head, q [B,Hq,D], against the static caches, keys 0..position visible
     (and < attend_len), GQA.  Returns [B,Hq,D].  Replaces mask + scaled_dot_product_attention (qllama.py:90-93).
-    position int64 [B]: row b sees keys 0..position[b]."""
+    position int64 [B]: row b sees keys 0..position[b].  q [B,T,Hq,D], 1 <= T <= 8: gbxq_decode_attention_multi, query t
+    of row b sees keys 0..position[b] + t (bitwise the single query there); returns [B,T,Hq,D]."""
     _bf16c(q, k_cache, v_cache)
-    b, hq, d = q.shape
+    b, t, hq, d = _block(q, "decode_attention")
     hkv, max_len = k_cache.shape[1], k_cache.shape[2]
     stride = _pos_stride(position, b, q, "decode_attention")
     out = torch.empty_like(q)
+    lib, attend_len = _lib.get(), int(attend_len or max_len)
     with torch.cuda.device(q.device):
-        rc = _lib.get().gbxq_decode_attention(q.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), position.data_ptr(),
-                                              stride, out.data_ptr(), b, hq, hkv, d, max_len,
-                                              int(attend_len or max_len), float(scale), _stream())
+        if q.dim() == 4:
+            rc = lib.gbxq_decode_attention_multi(q.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), position.data_ptr(),
+                                                 stride, out.data_ptr(), b, t, hq, hkv, d, max_len, attend_len,
+                                                 float(scale), _stream())
+        else:
+            rc = lib.gbxq_decode_attention(q.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), position.data_ptr(),
+                                           stride, out.data_ptr(), b, hq, hkv, d, max_len, attend_len, float(scale),
+                                           _stream())
     _lib.check(rc, "gbxq_decode_attention")
     return out
 
 
 def _check_qcache(q: torch.Tensor, k_cache3, v_cache3, group_size: int, bits: int):
-    """Shapes of the quantized-cache glue: q [B,Hq,D] bf16, triples (codes uint32 [B,Hkv,max_len,D*bits/32], scales /
-    biases bf16 [B,Hkv,max_len,D/group_size]), all contiguous on one CUDA device.  Returns (B, Hq, Hkv, D, max_len)."""
+    """Shapes of the quantized-cache glue: q [B,Hq,D] (or a block [B,T,Hq,D]) bf16, triples (codes uint32
+    [B,Hkv,max_len,D*bits/32], scales / biases bf16 [B,Hkv,max_len,D/group_size]), all contiguous on one CUDA device.
+    Returns (B, T, Hq, Hkv, D, max_len)."""
     if bits not in (2, 3, 4, 6, 8):
         raise ValueError(f"quantized cache: bits must be one of 2, 3, 4, 6, 8; got {bits}")
     if group_size not in (32, 64, 128):
         raise ValueError(f"quantized cache: group_size must be 32, 64 or 128; got {group_size}")
     if len(k_cache3) != 3 or len(v_cache3) != 3:
         raise ValueError("quantized cache: keys and values are (codes, scales, biases) triples")
-    if q.dim() != 3 or q.dtype != torch.bfloat16:
-        raise ValueError("quantized cache: q must be bf16 [B, Hq, D]")
-    b, hq, d = q.shape
+    if q.dim() not in (3, 4) or q.dtype != torch.bfloat16:
+        raise ValueError("quantized cache: q must be bf16 [B, Hq, D] or [B, T, Hq, D]")
+    b, t, hq, d = _block(q, "quantized cache")
     kq = k_cache3[0]
     if kq.dim() != 4:
         raise ValueError("quantized cache: codes must be [B, Hkv, max_len, D*bits/32]")
@@ -601,7 +632,7 @@ def _check_qcache(q: torch.Tensor, k_cache3, v_cache3, group_size: int, bits: in
     ts = [q, *k_cache3, *v_cache3]
     if not all(t.is_cuda and t.is_contiguous() for t in ts) or len({t.device for t in ts}) != 1:
         raise ValueError("quantized cache ops take contiguous tensors on one CUDA device (there is no CPU path)")
-    return b, hq, hkv, d, max_len
+    return b, t, hq, hkv, d, max_len
 
 
 def rope_cache_quantized(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, position: torch.Tensor, inv_freq: torch.Tensor,
@@ -610,21 +641,28 @@ def rope_cache_quantized(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, posi
     `position` (int64 device tensor [1]) of its (codes, scales, biases) triple -- bit-identical to `rope_cache` into a bf16
     row followed by `quantize_into` of that row.  The quantized counterpart of `rope_cache` (RoPE +
     QuantizedKVCache.update_and_fetch, gbx_lm/models/cache.py:172-185).  keep = an int: row ring_slot(position) of a
-    rotating cache, as `rope_cache`.  position int64 [B]: row b at position[b]."""
+    rotating cache, as `rope_cache`.  position int64 [B]: row b at position[b].  q [B,T,Hq,D] (k / v [B,T,Hkv,D]):
+    gbxq_rope_cache_quantized_multi, as `rope_cache` with a block; flat caches only."""
     group_size, bits = int(group_size), int(bits)
-    b, hq, hkv, d, max_len = _check_qcache(q, k_cache3, v_cache3, group_size, bits)
+    _block(q, "rope_cache_quantized", keep)  # a block needs a flat cache
+    b, t, hq, hkv, d, max_len = _check_qcache(q, k_cache3, v_cache3, group_size, bits)
     _bf16c(k, v)
-    if tuple(k.shape) != (b, hkv, d) or tuple(v.shape) != (b, hkv, d):
-        raise ValueError(f"rope_cache_quantized: k / v must be [B, Hkv, D] = {(b, hkv, d)}")
+    kv_shape = (b, hkv, d) if q.dim() == 3 else (b, t, hkv, d)
+    if tuple(k.shape) != kv_shape or tuple(v.shape) != kv_shape:
+        raise ValueError(f"rope_cache_quantized: k / v must be {kv_shape}")
     if inv_freq.dtype != torch.float32 or inv_freq.numel() != d // 2 or inv_freq.device != q.device:
         raise ValueError("rope_cache_quantized: inv_freq float32 [D/2] on the device of q")
     keep = _check_keep(keep, max_len, "rope_cache_quantized")
     stride = _pos_stride(position, b, q, "rope_cache_quantized")
+    lib = _lib.get()
+    ptrs = (q.data_ptr(), k.data_ptr(), v.data_ptr(), position.data_ptr(), stride, inv_freq.data_ptr(),
+            *[x.data_ptr() for x in k_cache3], *[x.data_ptr() for x in v_cache3])
     with torch.cuda.device(q.device):
-        rc = _lib.get().gbxq_rope_cache_quantized(
-            q.data_ptr(), k.data_ptr(), v.data_ptr(), position.data_ptr(), stride, inv_freq.data_ptr(),
-            *[t.data_ptr() for t in k_cache3], *[t.data_ptr() for t in v_cache3], b, hq, hkv, d, max_len,
-            -1 if keep is None else keep, bits, group_size, _stream())
+        if q.dim() == 4:
+            rc = lib.gbxq_rope_cache_quantized_multi(*ptrs, b, t, hq, hkv, d, max_len, bits, group_size, _stream())
+        else:
+            rc = lib.gbxq_rope_cache_quantized(*ptrs, b, hq, hkv, d, max_len, -1 if keep is None else keep, bits,
+                                               group_size, _stream())
     _lib.check(rc, "gbxq_rope_cache_quantized")
     return q
 
@@ -649,22 +687,28 @@ def decode_attention_quantized(q: torch.Tensor, k_cache3, v_cache3, position: to
     """gbxq_decode_attention_quantized: one query row per head, q [B,Hq,D], against the quantized triples, keys
     0..position visible (and < attend_len, default the whole cache), GQA.  Returns [B,Hq,D] bf16.  The result does not
     depend on attend_len beyond the clamp (bitwise).  Replaces quantized_scaled_dot_product_attention at decode
-    (gbx_lm/models/base.py:65-98).  position int64 [B]: row b sees keys 0..position[b]."""
+    (gbx_lm/models/base.py:65-98).  position int64 [B]: row b sees keys 0..position[b].  q [B,T,Hq,D], 1 <= T <= 8:
+    gbxq_decode_attention_quantized_multi, query t of row b at position[b] + t, bitwise the single query there, with each
+    chunk's codes read once for the T queries; returns [B,T,Hq,D]."""
     group_size, bits = int(group_size), int(bits)
-    b, hq, hkv, d, max_len = _check_qcache(q, k_cache3, v_cache3, group_size, bits)
+    b, t, hq, hkv, d, max_len = _check_qcache(q, k_cache3, v_cache3, group_size, bits)
     attend_len = int(max_len if attend_len is None else attend_len)
     if not 1 <= attend_len <= max_len:
         raise ValueError(f"decode_attention_quantized: attend_len {attend_len} outside [1, {max_len}]")
     stride = _pos_stride(position, b, q, "decode_attention_quantized")
     lib = _lib.get()
-    need = int(lib.gbxq_decode_attention_quantized_workspace_bytes(b, hq, hkv, d, attend_len))
+    need = int(lib.gbxq_decode_attention_quantized_workspace_bytes(b * t, hq, hkv, d, attend_len))
     out = torch.empty_like(q)
     with torch.cuda.device(q.device):
         ws = _qattn_workspace(q.device, need)
-        rc = lib.gbxq_decode_attention_quantized(
-            q.data_ptr(), *[t.data_ptr() for t in k_cache3], *[t.data_ptr() for t in v_cache3], position.data_ptr(),
-            stride, out.data_ptr(), b, hq, hkv, d, max_len, attend_len, float(scale), bits, group_size, ws.data_ptr(),
-            ws.numel(), _stream())
+        ptrs = (q.data_ptr(), *[x.data_ptr() for x in k_cache3], *[x.data_ptr() for x in v_cache3], position.data_ptr(),
+                stride, out.data_ptr())
+        if q.dim() == 4:
+            rc = lib.gbxq_decode_attention_quantized_multi(*ptrs, b, t, hq, hkv, d, max_len, attend_len, float(scale),
+                                                           bits, group_size, ws.data_ptr(), ws.numel(), _stream())
+        else:
+            rc = lib.gbxq_decode_attention_quantized(*ptrs, b, hq, hkv, d, max_len, attend_len, float(scale), bits,
+                                                     group_size, ws.data_ptr(), ws.numel(), _stream())
     _lib.check(rc, "gbxq_decode_attention_quantized")
     return out
 

@@ -93,8 +93,16 @@ def rope_inv_freq(dims: int, base: float, scaling: Optional[dict]) -> torch.Tens
 FUSED_DECODE = os.environ.get("GBXQ_FUSED_DECODE", "1") != "0"
 
 
-def fused_decode_ok(x: torch.Tensor, L: int, cache) -> bool:
-    return FUSED_DECODE and L == 1 and cache is not None and x.is_cuda and x.dtype == torch.bfloat16
+# The most tokens per row of one fused step: the `_multi` entry points of the decode-step kernels (include/gbxq.h)
+MAX_BLOCK_TOKENS = 8
+
+
+def fused_decode_ok(x: torch.Tensor, L: int, cache, block: bool = False) -> bool:
+    """Whether a model call of L tokens per row may take the fused decode step: L == 1, or with `block` (explicit
+    consecutive positions, Model.forward) 2 <= L <= MAX_BLOCK_TOKENS on a flat cache -- a verify block."""
+    if not (FUSED_DECODE and cache is not None and x.is_cuda and x.dtype == torch.bfloat16):
+        return False
+    return L == 1 or (block and 2 <= L <= MAX_BLOCK_TOKENS and cache.keep is None)
 
 
 class RoPE(nn.Module):
@@ -155,30 +163,32 @@ class Attention(nn.Module):  # gbx_lm/models/qllama.py:39-96
         return FUSED_DECODE and cache.fused_decode_fits(self.head_dim, self.n_heads, self.n_kv_heads)
 
     def forward(self, x, positions, cache: Optional[Union[StaticKVCache, StaticQuantizedKVCache]],
-                attend_len: Optional[int]):
+                attend_len: Optional[int], block: bool = False):
         B, L, _ = x.shape
         # one grouped launch for the three projections of x (ref qllama.py:76 calls them back to back)
         q, k, v = ops.quantized_matmul_grouped(x, (self.q_proj, self.k_proj, self.v_proj))
         quantized = isinstance(cache, StaticQuantizedKVCache)
-        per_row = positions.dim() == 2  # [B, 1]: a decode step whose rows sit at different positions
-        if fused_decode_ok(x, L, cache) and self.takes_fused_decode(cache):
-            if per_row:
-                positions = positions.reshape(B)
-            # decode step: RoPE + cache write in one launch, one-query attention in another (SURVEY.md 8f rank 2); over
-            # the quantized cache the attention is split-K on the codes (+ its combine launch)
-            qh = q.view(B, self.n_heads, self.head_dim)
-            kh, vh = k.view(B, self.n_kv_heads, self.head_dim), v.view(B, self.n_kv_heads, self.head_dim)
+        per_row = positions.dim() == 2  # [B, L]: rows that sit at different positions
+        if fused_decode_ok(x, L, cache, block) and self.takes_fused_decode(cache):
+            # the first position of each row (or of all rows): a block's tokens sit at start .. start + L - 1
+            start = positions[:, 0].contiguous() if per_row else positions[:1]
+            # decode step: RoPE + cache write in one launch, attention in another (SURVEY.md 8f rank 2); over the
+            # quantized cache the attention is split-K on the codes (+ its combine launch).  L > 1: a verify block, the
+            # same launches over [B, L, heads, D]
+            lead = (B,) if L == 1 else (B, L)
+            qh = q.view(*lead, self.n_heads, self.head_dim)
+            kh, vh = k.view(*lead, self.n_kv_heads, self.head_dim), v.view(*lead, self.n_kv_heads, self.head_dim)
             # (a rotating cache: the row is the position's ring slot, and the attention reads the whole window)
             if quantized:
                 gs, bits = cache.group_size, cache.bits
-                ops.rope_cache_quantized(qh, kh, vh, positions, self.rope.inv_freq, cache.keys, cache.values, gs, bits,
+                ops.rope_cache_quantized(qh, kh, vh, start, self.rope.inv_freq, cache.keys, cache.values, gs, bits,
                                          keep=cache.keep)
-                out = ops.decode_attention_quantized(qh, cache.keys, cache.values, positions, self.scale, gs, bits,
+                out = ops.decode_attention_quantized(qh, cache.keys, cache.values, start, self.scale, gs, bits,
                                                      attend_len)
             else:
-                ops.rope_cache(qh, kh, vh, positions, self.rope.inv_freq, cache.keys, cache.values, keep=cache.keep)
-                out = ops.decode_attention(qh, cache.keys, cache.values, positions, self.scale, attend_len)
-            return self.tp.row_parallel(self.o_proj, out.view(B, 1, -1))
+                ops.rope_cache(qh, kh, vh, start, self.rope.inv_freq, cache.keys, cache.values, keep=cache.keep)
+                out = ops.decode_attention(qh, cache.keys, cache.values, start, self.scale, attend_len)
+            return self.tp.row_parallel(self.o_proj, out.view(B, L, -1))
         if per_row and cache is not None and cache.keep is not None:
             raise ValueError("per-row positions on a rotating cache need the fused decode path (the unfused ring glue "
                              "works on one shared offset)")
@@ -198,7 +208,7 @@ class Attention(nn.Module):  # gbx_lm/models/qllama.py:39-96
             # the rows are written at the HOST offset (Model.forward has already advanced it past these L positions), so
             # this path is not graph-capturable
             T = cache.offset
-            if per_row:  # each row at its own position (read back to the host)
+            if per_row:  # each row at its own (consecutive) positions, read back to the host
                 for b, p in enumerate(positions[:, 0].tolist()):
                     cache.update_row(b, k[b:b + 1], v[b:b + 1], p)
             else:
@@ -269,17 +279,17 @@ class LlamaModel(nn.Module):  # gbx_lm/models/qllama.py:144-174
         self.layers = nn.ModuleList([TransformerBlock(args, tp, qkv_bias) for _ in range(args.num_hidden_layers)])
         self.norm = nn.RMSNorm(args.hidden_size, eps=args.rms_norm_eps)
 
-    def forward(self, inputs, positions, cache, attend_len):
+    def forward(self, inputs, positions, cache, attend_len, block: bool = False):
         h = self.embed_tokens(inputs)
         if cache is None:
             cache = [None] * len(self.layers)
-        if fused_decode_ok(h, inputs.shape[1], cache[0]) and h.shape[-1] % 8 == 0:
+        if fused_decode_ok(h, inputs.shape[1], cache[0], block) and h.shape[-1] % 8 == 0:
             # decode step: every residual add travels with the RMSNorm that follows it (one launch each); the add of a
             # block's MLP output happens in the next block's (or the final) norm launch
             resid, pend = h.contiguous(), None
             for layer, c in zip(self.layers, cache):
                 resid, n = ops.add_rmsnorm(resid, pend, layer.input_layernorm.weight, layer.input_layernorm.eps)
-                a = layer.self_attn(n, positions, c, attend_len)
+                a = layer.self_attn(n, positions, c, attend_len, block)
                 resid, n = ops.add_rmsnorm(resid, a, layer.post_attention_layernorm.weight, layer.post_attention_layernorm.eps)
                 pend = layer.mlp(n)
             return ops.add_rmsnorm(resid, pend, self.norm.weight, self.norm.eps, want_h=False)[1]
@@ -305,11 +315,14 @@ class Model(nn.Module):  # gbx_lm/models/qllama.py:177-209
                 head_columns: Optional[torch.Tensor] = None):
         """inputs int64 [B, L].  positions int64 [L] (absolute, shared by the rows); default = cache offset .. offset+L.
         A decode step (L = 1) may instead give each row its own position, int64 [B, 1]; the caller keeps the caches'
-        offsets then.  attend_len: number of cache positions attended (None = whole static cache, for graph replay).
+        offsets then.  Explicit positions with 2 <= L <= 8 must be consecutive in each row (int64 [L] shared, or [B, L]
+        per row): a verify block of speculative decoding, which takes the fused decode step on flat caches (its tokens
+        written at their positions, query t seeing keys 0 .. p_b + t); the caller keeps the offsets.  attend_len: number of cache positions attended (None = whole static cache, for graph replay).
         head_columns int64 [B]: only column head_columns[b] of row b goes through the vocabulary projection (logits
         [B, 1, V], hidden states [B, 1, H]) -- what a batched prefill needs, without the [B, L, V] logits of every
         position; None: every position."""
         L = inputs.shape[1]
+        block = positions is not None and L > 1
         if positions is None:
             off = cache[0].offset if cache is not None else 0
             positions = torch.arange(off, off + L, device=inputs.device)
@@ -317,7 +330,7 @@ class Model(nn.Module):  # gbx_lm/models/qllama.py:177-209
                 for c in cache:
                     c.offset = off + L
                 attend_len = cache[0].attend_len  # off + L; at most the window on a rotating cache
-        out = self.model(inputs, positions, cache, attend_len)
+        out = self.model(inputs, positions, cache, attend_len, block)
         if head_columns is not None:
             out = out[torch.arange(out.shape[0], device=out.device), head_columns][:, None]
         # vocabulary projection (qllama.py:194-198): decode-sized inputs go through the streaming bf16 GEMV

@@ -5,6 +5,7 @@
     make_shards/save_weights gbx_lm/utils.py:967-988, 1055-1104
     save_config              gbx_lm/utils.py:1107-1127
     generate_step            gbx_lm/utils.py:217-338   (batch-1 prefill in 2048-token chunks + greedy decode)
+    speculative_generate_step gbx_lm/utils.py:341-522  (a draft model proposes, the target verifies k + 1 tokens a step)
     batch_generate           (new) greedy decode of B prompts of different lengths in one batch
 
 The on-disk layout is exactly what gba2mlx emits (gbx_lm/gba2mlx.py:47-65): `model*.safetensors` with
@@ -25,7 +26,8 @@ import torch
 from torch import nn
 
 from . import qllama, qqwen2
-from .cache import DEFAULT_KV_KEEP, StaticKVCache, StaticQuantizedKVCache, maybe_quantize_kv_cache
+from .cache import (DEFAULT_KV_KEEP, StaticKVCache, StaticQuantizedKVCache, maybe_quantize_kv_cache,
+                    trim_prompt_cache)
 from .quantized_linear import QuantizedLinear
 from .tp import TPContext, proj_kind, shard_tensor
 
@@ -512,10 +514,6 @@ def generate_step(
     kv = dict(kv_bits=kv_bits, kv_group_size=kv_group_size, quantized_kv_start=quantized_kv_start)
     quantize_cache = _kv_quantizer(cache, **kv)
 
-    def _logprobs(logits):
-        logits = logits.float()
-        return logits - torch.logsumexp(logits, dim=-1, keepdim=True)
-
     with torch.no_grad():
         lp = _logprobs(prefill(model, y, cache, prefill_step_size, **kv))
         tok = sampler(lp)
@@ -539,18 +537,237 @@ def generate_step(
                 dg = _decode_graph(model, cache, tok, cache[0].offset)
 
 
+def _logprobs(logits: torch.Tensor) -> torch.Tensor:
+    logits = logits.float()
+    return logits - torch.logsumexp(logits, dim=-1, keepdim=True)
+
+
+# ------------------------------------------------------------------------------------------ speculative decoding
+def _check_speculative(model, draft_model, num_draft_tokens: int, max_kv_size: Optional[int] = None) -> None:
+    if max_kv_size is not None:
+        raise ValueError("speculative decoding: max_kv_size (a rotating cache) cannot be rewound; use a flat cache")
+    if isinstance(num_draft_tokens, bool) or not isinstance(num_draft_tokens, int) or not 1 <= num_draft_tokens <= 7:
+        raise ValueError(f"speculative decoding: num_draft_tokens must be an int in 1..7, got {num_draft_tokens!r}")
+    if model.args.vocab_size != draft_model.args.vocab_size:
+        raise ValueError(f"speculative decoding: the draft's vocabulary ({draft_model.args.vocab_size}) differs from the "
+                         f"target's ({model.args.vocab_size})")
+    if model.tp.world > 1 or draft_model.tp.world > 1:
+        raise ValueError("speculative decoding: tensor-parallel models are not supported")
+
+
+def _spec_cache(model, draft_model, run_len: int) -> list:
+    """The target's flat caches, then the draft's (the reference's prompt_cache layout)."""
+    return qllama.make_prompt_cache(model, 1, run_len) + qllama.make_prompt_cache(draft_model, 1, run_len)
+
+
+def _draft_and_verify(model, draft_model, tc: list, dc: list, prev: torch.Tensor, y: torch.Tensor, P: torch.Tensor,
+                      k: int, pick: Callable[[torch.Tensor], torch.Tensor], host_P: Optional[int] = None):
+    """Steps 1 and 2 of a round (DESIGN.md section 10).  prev / y [1]: the tokens at P - 1 and P (int64 [1] on the
+    device).  The draft takes one T = 2 step on [prev, y] at P - 1, P, then k - 1 single-token steps, each token picked
+    from the last logits (`pick`: logits [V] -> token [1]); the target verifies [y, d_1 .. d_k] at P .. P + k in one
+    step of k + 1 tokens.  Returns (d [k], the verify logits [k + 1, V]).  host_P: P as an int, to keep the caches'
+    offsets (the unfused glue writes a quantized cache at them); None inside a captured graph, which needs the fused
+    path."""
+    ar = torch.arange(k + 1, device=P.device)
+
+    def call(m, cache, toks, pos, end):
+        if host_P is not None:
+            for c in cache:
+                c.offset = host_P + end
+        return m(toks[None], cache, positions=pos)[0]
+
+    d = [pick(call(draft_model, dc, torch.cat([prev, y]), P - 1 + ar[:2], 1)[-1])]
+    for i in range(1, k):
+        d.append(pick(call(draft_model, dc, d[-1], P + i, i + 1)[-1]))
+    d = torch.cat(d)
+    return d, call(model, tc, torch.cat([y, d]), P + ar, k + 1)
+
+
+def speculative_generate_step(prompt: torch.Tensor, model: nn.Module, draft_model: nn.Module, *, num_draft_tokens: int = 2,
+                              max_tokens: int = 256, sampler: Optional[Callable[[torch.Tensor], torch.Tensor]] = None,
+                              prompt_cache: Optional[list] = None, prefill_step_size: int = 2048,
+                              kv_bits: Optional[int] = None, kv_group_size: int = 64, quantized_kv_start: int = 0
+                              ) -> Generator[Tuple[int, torch.Tensor, bool], None, None]:
+    """Mirror of gbx_lm/utils.py:341-522: `draft_model` proposes num_draft_tokens = k tokens a round and `model` checks
+    them in one step of k + 1 tokens; yields (token, logprobs, from_draft).  prompt_cache: the target's caches, then the
+    draft's (default: flat caches of prompt + max_tokens + k + 2 positions).  `sampler` picks every token from its
+    log-probabilities (default argmax).  kv_bits / kv_group_size / quantized_kv_start as in generate_step: both lists
+    are converted after the verify step that takes the target's offset past quantized_kv_start.
+
+    The round schedule (DESIGN.md section 10) keeps the block at k + 1 tokens in every round, the last one included, and
+    drops the tokens past max_tokens, so that at a fixed k the tokens do not depend on the draft."""
+    k = num_draft_tokens
+    _check_speculative(model, draft_model, k)
+    dev = next(model.parameters()).device
+    y0 = prompt.reshape(-1).to(dev)
+    sampler = sampler or (lambda lp: torch.argmax(lp, dim=-1))
+    cache = prompt_cache if prompt_cache is not None else _spec_cache(model, draft_model, y0.numel() + max_tokens + k + 2)
+    nt = len(model.layers)
+    kv = dict(kv_bits=kv_bits, kv_group_size=kv_group_size, quantized_kv_start=quantized_kv_start)
+    if max_tokens <= 0:
+        return
+    with torch.no_grad():
+        tc, dc = cache[:nt], cache[nt:]
+        lp = _logprobs(prefill(model, y0, tc, prefill_step_size, **kv))[0]
+        prefill(draft_model, y0, dc, prefill_step_size, **kv)
+        cache[:] = tc + dc
+        y = sampler(lp).reshape(1)
+        prev, P = y0[-1:], y0.numel()  # the target holds positions < P, y sits at P, the draft holds < P - 1 at least
+        yield int(y), lp, False
+        ntoks = 1
+        while ntoks < max_tokens:
+            tc, dc = cache[:nt], cache[nt:]
+            d, logits = _draft_and_verify(model, draft_model, tc, dc, prev, y, torch.tensor([P], device=dev), k,
+                                          lambda lg: sampler(_logprobs(lg)).reshape(1), host_P=P)
+            maybe_quantize_kv_cache(cache, quantized_kv_start, kv_group_size, kv_bits)  # by the target's offset
+            lps = _logprobs(logits)
+            a = sampler(lps).reshape(-1)
+            a_l, d_l = a.tolist(), d.tolist()
+            n = 0
+            while n < k and a_l[n] == d_l[n]:
+                n += 1
+            for i in range(n + 1):
+                yield a_l[i], lps[i], i < n
+                ntoks += 1
+                if ntoks == max_tokens:
+                    break
+            # rewind: the target keeps positions < P + n + 1, the draft < P + n (its next T = 2 step rewrites P + n)
+            block = torch.cat([y, d])
+            prev, y, P = block[n:n + 1], a[n:n + 1], P + n + 1
+            trim_prompt_cache(cache[:nt], k - n)
+            trim_prompt_cache(cache[nt:], k - n)
+
+
+def _check_fused(model, draft_model, cache: list) -> None:
+    """The device driver captures its rounds: every cache of the list (the target's, then the draft's) must be on the
+    fused decode path, whose positions live on the device."""
+    nt = len(model.layers)
+    for m, cs in ((model, cache[:nt]), (draft_model, cache[nt:])):
+        if not all(qllama.FUSED_DECODE and layer.self_attn.takes_fused_decode(c) for layer, c in zip(m.layers, cs)):
+            raise ValueError("speculative decoding on the device: a cache is off the fused decode path (raise "
+                             "GBXQ_FUSED_DECODE or use a quantized cache for contexts above 49152 keys)")
+
+
+class _SpecGraph:
+    """One round of speculative decoding captured in a CUDA graph: the draft's steps with their argmax fed back, the
+    verify step, the accept rule, the write of a_0 .. a_k into `out` at `idx`, and the advance of P / prev / y -- all
+    on device tensors, so rounds replay back to back without the host."""
+
+    def __init__(self, model, draft_model, cache: list, k: int, prev, y, P: int, out: torch.Tensor, idx: torch.Tensor,
+                 accepted: torch.Tensor):
+        nt = len(model.layers)
+        self.k, self.tc, self.dc = k, cache[:nt], cache[nt:]
+        _check_fused(model, draft_model, cache)
+        dev = out.device
+        self.prev, self.y = prev.clone(), y.clone()
+        self.P = torch.tensor([P], dtype=torch.long, device=dev)
+        self.out, self.idx, self.accepted = out, idx, accepted
+        self.model, self.draft_model = model, draft_model
+        state = (self.prev, self.y, self.P, self.out, self.idx, self.accepted)
+        snap = [t.clone() for t in state]
+        s = torch.cuda.Stream()
+        s.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(s), torch.no_grad():
+            for _ in range(2):  # warm-up (workspaces, libraries); it writes the rows the first replay writes anyway
+                self._round()
+                for t, v in zip(state, snap):
+                    t.copy_(v)
+        torch.cuda.current_stream().wait_stream(s)
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph), torch.no_grad():
+            self._round()
+
+    def _round(self):
+        k = self.k
+        d, logits = _draft_and_verify(self.model, self.draft_model, self.tc, self.dc, self.prev, self.y, self.P, k,
+                                      lambda lg: fast_argmax(lg).reshape(1))
+        a = fast_argmax(logits)  # [k + 1]
+        n = (a[:k] == d).long().cumprod(0).sum().reshape(1)  # leading matches
+        self.out.index_copy_(0, self.idx + torch.arange(k + 1, device=a.device), a)
+        self.prev.copy_(torch.cat([self.y, d]).index_select(0, n))
+        self.y.copy_(a.index_select(0, n))
+        self.P.add_(n + 1)
+        self.idx.add_(n + 1)
+        self.accepted.add_(n)
+
+
+def _speculative_device(model, draft_model, y0: torch.Tensor, max_tokens: int, k: int, prefill_step_size: int,
+                        kv: dict) -> Tuple[List[int], float, dict]:
+    """generate_tokens_device with a draft: rounds of _SpecGraph, r = ceil(remaining / (k + 1)) replays between host
+    synchronisations (each round emits 1 .. k + 1 tokens, so at most k past max_tokens, dropped).  Before the kv_bits
+    conversion the host synchronises every round, converts both lists after the round whose verify takes the target's
+    offset past quantized_kv_start, and captures the round again."""
+    dev = y0.device
+    cache = _spec_cache(model, draft_model, y0.numel() + max_tokens + k + 2)
+    # refused before the prefill when the rounds start on these bf16 caches; when the prefill converts them (kv_bits,
+    # a prompt longer than quantized_kv_start), the converted caches are checked right after it
+    if kv["kv_bits"] is None or y0.numel() <= kv["quantized_kv_start"]:
+        _check_fused(model, draft_model, cache)
+    nt = len(model.layers)
+    tc, dc = cache[:nt], cache[nt:]
+    tok = fast_argmax(prefill(model, y0, tc, prefill_step_size, **kv)[0]).reshape(1)
+    prefill(draft_model, y0, dc, prefill_step_size, **kv)
+    cache[:] = tc + dc
+    _check_fused(model, draft_model, cache)
+    out = torch.zeros((max_tokens + k + 1,), dtype=torch.long, device=dev)
+    out[:1] = tok
+    idx = torch.ones((1,), dtype=torch.long, device=dev)
+    accepted = torch.zeros((1,), dtype=torch.long, device=dev)
+    P, rounds = y0.numel(), 0
+    pending = kv["kv_bits"] is not None and isinstance(cache[0], StaticKVCache)  # a conversion still to come
+    sg = _SpecGraph(model, draft_model, cache, k, y0[-1:], tok, P, out, idx, accepted) if max_tokens > 1 else None
+    t_first = time.perf_counter()
+    emitted = 1
+    while emitted < max_tokens:
+        r = 1 if pending else -(-(max_tokens - emitted) // (k + 1))
+        for _ in range(r):
+            sg.graph.replay()
+        rounds += r
+        if pending:
+            P_start = int(sg.P) - (int(sg.idx) - emitted)
+            for i, c in enumerate(cache):  # the offsets after this round's verify (target) and last draft step
+                c.offset = P_start + k + (1 if i < nt else 0)
+            maybe_quantize_kv_cache(cache, kv["quantized_kv_start"], kv["kv_group_size"], kv["kv_bits"])
+            if not isinstance(cache[0], StaticKVCache):
+                pending = False
+                sg = _SpecGraph(model, draft_model, cache, k, sg.prev, sg.y, int(sg.P), out, idx, accepted)
+        emitted = int(idx)
+    if sg is not None:
+        P = int(sg.P)
+    for i, c in enumerate(cache):
+        c.offset = P if i < nt else P - 1
+    stats = {"draft_tokens": rounds * k, "accepted_tokens": int(accepted),
+             "acceptance_rate": int(accepted) / max(rounds * k, 1)}
+    return out[:max_tokens].tolist(), t_first, stats
+
+
 def generate_tokens_device(model, prompt: torch.Tensor, max_tokens: int = 128, prefill_step_size: int = 2048,
                            kv_bits: Optional[int] = None, kv_group_size: int = 64, quantized_kv_start: int = 0,
-                           max_kv_size: Optional[int] = None) -> Tuple[List[int], dict]:
+                           max_kv_size: Optional[int] = None, draft_model: Optional[nn.Module] = None,
+                           num_draft_tokens: int = 2) -> Tuple[List[int], dict]:
     """Greedy generation with the sampler inside the captured decode step (DecodeGraph device_loop): the same tokens as
     `generate_tokens` (argmax of the log-probabilities = argmax of the logits), but the host only enqueues replays and
     reads the tokens once at the end -- the per-token host round trip of utils.py:299-337 (~0.3-0.6 ms on a B200 box)
     is gone.  Same timing definitions as generate_tokens.  kv_bits / kv_group_size / quantized_kv_start as in
     generate_step: when the conversion falls inside the decode, the graph replays up to that step, the caches are
     converted, and a graph of the quantized step replays the rest.  max_kv_size as in generate_step: the captured step
-    writes the ring slot of its device-side position, so the replays wrap without the host."""
+    writes the ring slot of its device-side position, so the replays wrap without the host.
+    draft_model: speculative decoding with num_draft_tokens = k drafts a round (speculative_generate_step's schedule and
+    tokens), each round one captured graph (_SpecGraph); the stats add draft_tokens, accepted_tokens and
+    acceptance_rate."""
     y = prompt.reshape(-1).to(next(model.parameters()).device)
     n_prompt = y.numel()
+    if draft_model is not None:
+        _check_speculative(model, draft_model, num_draft_tokens, max_kv_size)
+        kv = dict(kv_bits=kv_bits, kv_group_size=kv_group_size, quantized_kv_start=quantized_kv_start)
+        t0 = time.perf_counter()
+        with torch.no_grad():
+            toks, t_first, spec = _speculative_device(model, draft_model, y, max_tokens, num_draft_tokens,
+                                                      prefill_step_size, kv)
+        t1 = time.perf_counter()
+        return toks, {"prompt_tokens": int(n_prompt), "prompt_tps": n_prompt / max(t_first - t0, 1e-9),
+                      "generation_tokens": len(toks), "generation_tps": max(len(toks) - 1, 1) / max(t1 - t_first, 1e-9),
+                      **spec}
     cache = _prompt_cache(model, n_prompt + max_tokens + 1, max_kv_size)
     kv = dict(kv_bits=kv_bits, kv_group_size=kv_group_size, quantized_kv_start=quantized_kv_start)
     t0 = time.perf_counter()
@@ -643,11 +860,19 @@ def batch_generate(model, prompts: List[torch.Tensor], max_tokens: int = 128, *,
 def generate_tokens(model, prompt: torch.Tensor, max_tokens: int = 128, **kw) -> Tuple[List[int], dict]:
     """Greedy generation + the reference's timing definitions (utils.py:590-607):
     prompt_tps = prompt_len / time_to_first_token, generation_tps = n / (t_now - t_first).  Keyword arguments
-    (use_cuda_graph, prefill_step_size, kv_bits, kv_group_size, quantized_kv_start, ...) go to generate_step."""
+    (use_cuda_graph, prefill_step_size, kv_bits, kv_group_size, quantized_kv_start, ...) go to generate_step; with
+    draft_model (and num_draft_tokens) to speculative_generate_step."""
     toks = []
     t0 = time.perf_counter()
     t_first = None
-    for tok, _ in generate_step(prompt, model, max_tokens=max_tokens, **kw):
+    draft_model = kw.pop("draft_model", None)
+    if draft_model is not None:
+        _check_speculative(model, draft_model, kw.get("num_draft_tokens", 2), kw.pop("max_kv_size", None))
+        kw.pop("use_cuda_graph", None)
+        steps = ((t, lp) for t, lp, _ in speculative_generate_step(prompt, model, draft_model, max_tokens=max_tokens, **kw))
+    else:
+        steps = generate_step(prompt, model, max_tokens=max_tokens, **kw)
+    for tok, _ in steps:
         if t_first is None:
             t_first = time.perf_counter()
         toks.append(tok)

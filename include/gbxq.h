@@ -279,6 +279,22 @@ int gbxq_rope_cache(void* q, const void* k, const void* v, const int64_t* pos_de
 int gbxq_decode_attention(const void* q, const void* k_cache, const void* v_cache, const int64_t* pos_dev,
                           int pos_stride, void* out, int B, int Hq, int Hkv, int D, int64_t max_len,
                           int64_t attend_len, float scale, void* stream);
+/*
+ * Verify blocks (speculative decoding): T consecutive tokens per batch row, 1 <= T <= 8, token t of row b at position
+ * p_b + t (p_b from pos_dev / pos_stride as above), on a flat cache (no keep argument).  q is [B,T,Hq,D], k / v
+ * [B,T,Hkv,D], out [B,T,Hq,D].  T outside 1..8 returns GBXQ_ESHAPE, before any CUDA call.
+ *   gbxq_rope_cache_multi       bitwise T calls of gbxq_rope_cache at p_b .. p_b + T - 1; positions >= max_len are not
+ *                               written (q is not rotated there either)
+ *   gbxq_decode_attention_multi query t of row b attends keys [0, min(p_b + t, attend_len-1)] of row b's cache, bitwise
+ *                               the gbxq_decode_attention call for that query at p_b + t.  The block's own keys are
+ *                               written before the call, so this is the causal mask inside the block.
+ */
+int gbxq_rope_cache_multi(void* q, const void* k, const void* v, const int64_t* pos_dev, int pos_stride,
+                          const float* inv_freq_dev, void* k_cache, void* v_cache, int B, int T, int Hq, int Hkv, int D,
+                          int64_t max_len, void* stream);
+int gbxq_decode_attention_multi(const void* q, const void* k_cache, const void* v_cache, const int64_t* pos_dev,
+                                int pos_stride, void* out, int B, int T, int Hq, int Hkv, int D, int64_t max_len,
+                                int64_t attend_len, float scale, void* stream);
 int gbxq_add_rmsnorm(const void* x, const void* r, const void* w, float eps, void* h_out, void* y_out, int64_t rows,
                      int H, void* stream);
 int gbxq_silu_mul(const void* gate, const void* up, void* out, int64_t n, void* stream);
@@ -317,6 +333,23 @@ int gbxq_decode_attention_quantized(const void* q, const uint32_t* k_codes, cons
                                     const void* v_biases, const int64_t* pos_dev, int pos_stride, void* out, int B,
                                     int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len, float scale,
                                     int bits, int group_size, void* workspace, size_t workspace_bytes, void* stream);
+/*
+ * Their verify-block forms, as gbxq_rope_cache_multi / gbxq_decode_attention_multi (T consecutive tokens per row, flat
+ * cache): the write is bitwise T calls of gbxq_rope_cache_quantized; each query of the attention is bitwise the
+ * gbxq_decode_attention_quantized call at its position, while one CTA reads each chunk's codes once for the T queries
+ * of its row.  The workspace holds B*T rows of partials: gbxq_decode_attention_quantized_workspace_bytes(B*T, Hq, Hkv,
+ * D, attend_len) bytes.
+ */
+int gbxq_rope_cache_quantized_multi(void* q, const void* k, const void* v, const int64_t* pos_dev, int pos_stride,
+                                    const float* inv_freq_dev, uint32_t* k_codes, void* k_scales, void* k_biases,
+                                    uint32_t* v_codes, void* v_scales, void* v_biases, int B, int T, int Hq, int Hkv,
+                                    int D, int64_t max_len, int bits, int group_size, void* stream);
+int gbxq_decode_attention_quantized_multi(const void* q, const uint32_t* k_codes, const void* k_scales,
+                                          const void* k_biases, const uint32_t* v_codes, const void* v_scales,
+                                          const void* v_biases, const int64_t* pos_dev, int pos_stride, void* out, int B,
+                                          int T, int Hq, int Hkv, int D, int64_t max_len, int64_t attend_len,
+                                          float scale, int bits, int group_size, void* workspace,
+                                          size_t workspace_bytes, void* stream);
 
 /*
  * Vocabulary projection of the decode step (SURVEY.md 8f rank 1): y[M,V] = x[M,K] . weight[V,K]^T with UNQUANTIZED bf16
